@@ -41,7 +41,16 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=0, help="scenarios in the CPU baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--collision-poses", type=int, default=1 << 24)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed search step computed as DIR/<name>.npy (float64, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU search's outputs: it needs --impl ours")
+    return args
 
 
 class ClockSampler:
@@ -350,6 +359,9 @@ def main():
                "sample": f"first {m} scenarios of rank 0's shard, oracle port of the reference's Python path "
                          f"(shapely/heapdict unavailable), multiprocessing.Pool({used}), search time only"}
 
+    if rank == 0 and args.dump_outputs:                # with N > 1 GPUs: rank 0's shard
+        dump_outputs(args.dump_outputs, out, res, idx)
+
     if rank == 0:
         ms_per_launch = max_ms / args.steps
         achieved = flops / (kernel_ms / args.steps * 1e-3) * 1e-12
@@ -394,6 +406,43 @@ def main():
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BUDGET = (64 << 20) - (64 << 10)          # array bytes; the rest of 64 MB is room for the .npy headers
+# Fields of HlPlanResult that describe the plan.  Left out because they change from run to run: path_offset and
+# keys_offset (positions in the pools, handed out by atomics), cycles (a clock reading), n_pose_checks and n_exact
+# (checks executed after the early exits, which depend on the order warps finish in).
+DUMP_FIELDS = ("status", "counter", "n_expanded", "arrival", "path_len", "rs_word", "goal_cost", "n_pose_checks_ref")
+
+
+def _ragged(starts, lens):
+    """Row indices starts[i] .. starts[i] + lens[i] - 1 for every i, concatenated."""
+    ends = np.cumsum(lens)
+    return np.repeat(starts - (ends - lens), lens) + np.arange(int(ends[-1]) if len(ends) else 0)
+
+
+def dump_outputs(dirname, out, res, scenario_index):
+    """Write one hybrid_astar_batch output as float64 ``dirname/<name>.npy``, scenario by scenario: the result fields,
+    the expanded keys [rows, 3] and the path arrays, both pools regrouped in scenario order.  If everything would
+    exceed DUMP_BUDGET, scenarios are taken in a fixed seeded order until the budget is spent; ``scenario_index`` names
+    the scenarios written, in the order their rows appear."""
+    n_exp = res["n_expanded"].astype(np.int64)
+    n_path = res["path_len"].astype(np.int64)
+    nbytes = 8 * (len(DUMP_FIELDS) + 1 + 3 * n_exp + 5 * n_path)
+    sel = np.arange(len(res))
+    if nbytes.sum() > DUMP_BUDGET:
+        order = np.random.default_rng(0).permutation(len(res))
+        sel = np.sort(order[:int(np.searchsorted(np.cumsum(nbytes[order]), DUMP_BUDGET, side="right"))])
+    kused, used = (int(v) for v in np.concatenate([out["kcursor"].cpu().numpy(), out["cursor"].cpu().numpy()]))
+    arrays = {"scenario_index": np.asarray(scenario_index)[sel]}
+    arrays.update({"result_" + f: res[f][sel] for f in DUMP_FIELDS})
+    arrays["expanded_keys"] = out["expanded"][:kused].cpu().numpy()[_ragged(res["keys_offset"][sel], n_exp[sel])]
+    rows = _ragged(res["path_offset"][sel], n_path[sel])
+    for name in ("x", "y", "yaw", "k", "dir"):
+        arrays["path_" + name] = out[name][:used].cpu().numpy()[rows]
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def collision_microbench(args, dev, fp32_peak):
