@@ -27,12 +27,9 @@
 #ifndef AW_LOCKSTEP
 #define AW_LOCKSTEP 1      // 0 free-running, 1 two alignment barriers per expansion, 2 one, 3 one every other expansion
 #endif
-#define AW_ENV_FLOATS 512
 #ifndef AW_MAX_PLANS
 #define AW_MAX_PLANS 6
 #endif
-#define FULL 0xffffffffu
-enum { ST_IDLE = 0, ST_SEARCH = 1, ST_DONE = 2 };
 
 struct AwSmem {                          // one per warp
     double start[3], goal[3];
@@ -68,213 +65,35 @@ struct AwSmem {                          // one per warp
     // stats
     unsigned long long n_checks, n_exact, n_ref;
     long long t_last, t_phase[AS_N_PHASES];
-    // backtrack
-    int chain_len, path_len;
-    long long path_off;
-    __align__(16) float envf[AW_ENV_FLOATS];
+    __align__(16) float envf[AS_ENV_FLOATS];
 };
 
 static_assert(sizeof(AwSmem) * AW_WARPS <= 227 * 1024, "per-CTA shared memory exceeds 227 KB");
-#undef TICK
 #define TICK(ph) do { if (lane == 0) { long long _n = clock64(); S.t_phase[ph] += _n - S.t_last; S.t_last = _n; } } while (0)
 
-// float32 environment of this warp's scenario into its shared-memory slice (falls back to global pointers)
-__device__ __noinline__ void stage_env_warp(const EnvBatchDev& eb, const EnvDesc& D, float* sm, int cap_floats,
-                                            EnvSmem& E, int lane) {
-    const int n_o = D.n_obs * HL_OBS32_STRIDE, n_f = D.n_field * HL_FIELD32_STRIDE, n_s = D.n_seg * 4;
-    E.n_obs = D.n_obs; E.n_field = D.n_field; E.n_seg = D.n_seg; E.all_rect = D.all_rect;
-    E.eps = D.eps; E.reach = D.reach;
-    for (int k = 0; k < 4; ++k) E.ext[k] = (float)D.body_ext[k];
-    const float* g_obs = eb.obs32 + (size_t)HL_OBS32_STRIDE * D.obs_off;
-    const float* g_field = eb.field32 + HL_FIELD32_STRIDE * (size_t)D.field_off;
-    const float* g_seg = eb.seg32 + 4 * (size_t)D.seg_off;
-    if (n_o + n_f + n_s <= cap_floats) {
-        float* s_obs = sm;
-        float* s_field = s_obs + n_o;
-        float* s_seg = s_field + n_f;
-        for (int i = lane; i < n_o; i += 32) s_obs[i] = g_obs[i];
-        for (int i = lane; i < n_f; i += 32) s_field[i] = g_field[i];
-        for (int i = lane; i < n_s; i += 32) s_seg[i] = g_seg[i];
-        E.obs = s_obs; E.field = s_field; E.seg = s_seg;
-    } else {
-        E.obs = g_obs; E.field = g_field; E.seg = g_seg;
-    }
-    __syncwarp();
-}
-
-struct AwOut {
-    HlPlanResult* results;
-    int32_t* expanded_keys;
-    long long keys_capacity;
-    unsigned long long* keys_cursor;
-    double* path_x; double* path_y; double* path_yaw; double* path_k;
-    int8_t* path_dir;
-    long long path_capacity;
-    unsigned long long* path_cursor;
-    unsigned long long* phase_cycles;
-    // two-phase sweeps (k_hybrid_astar_s): `order` lists the scenarios to run (NULL = 0 .. n-1; `order_count` then holds
-    // their number on the device); with `first_only` a scenario whose FIRST analytic shot fails is not searched but
-    // appended to `defer_list` for the second launch
-    const int* order; const int* order_count;
-    int* defer_list; int* defer_count;
-    int first_only;
-};
-
-// Results of a finished scenario: expanded keys, path (get_path_from_expanded_nodes, :429-454), record.
-__device__ __noinline__ void finalize_scenario(AwSmem& S, const AsWs& W, const AsParams& P, const AwOut& O, int lane) {
-    const int sc = S.scen;
-    long long koff = 0;
-    if (lane == 0 && S.n_closed > 0) {
-        koff = (long long)atomicAdd(O.keys_cursor, (unsigned long long)S.n_closed);
-        if (koff + S.n_closed > O.keys_capacity) { koff = -1; }
-    }
-    koff = __shfl_sync(FULL, koff, 0);
-    if (koff < 0) { if (lane == 0) { S.status = HL_STATUS_CAPACITY; S.n_closed = 0; } koff = 0; __syncwarp(); }
-    {
-        int32_t* ek = O.expanded_keys + (size_t)koff * 3;
-        for (int i = lane; i < S.n_closed; i += 32) {
-            int ix, iy, iw;
-            unpack_key(W.nkey[W.corder[i]], ix, iy, iw);
-            ek[3 * i] = ix; ek[3 * i + 1] = iy; ek[3 * i + 2] = iw;
-        }
-    }
-    if (lane == 0 && S.status == HL_STATUS_OK) {
-        // Walk cur -> parent -> ... -> start (slot 0 is the only node with the start key).  The chain is
-        // kept in hslot[] (the heap is dead once the search is over), goal side first.  closed_set[goal_key]
-        // is the goal node, so a goal in the start's own cell makes the reference's
-        // `while current_node_index != start_node_index` loop a no-op: empty path.
-        int len = 0, poses = 0, rs_pts = 0;
-        bool ok = true;
-        if (S.goal_key != S.start_key) {
-            for (int node = S.cur; node != 0; node = W.nparent[node]) {
-                if (len >= P.cap_nodes) { ok = false; break; }
-                W.hslot[len++] = node;
-                poses += W.nsteps[node] + 1;
-            }
-            if (S.arrival == 1) rs_pts = P.pawn ? S.dub_rows : (S.rs_pick < AW_MAX_PLANS ? S.plans[S.rs_pick] : S.plan_tmp).npts;
-        }
-        S.chain_len = len;
-        S.path_len = poses + rs_pts;
-        if (!ok || S.path_len > P.max_path_poses) { S.status = HL_STATUS_CAPACITY; S.path_len = 0; }
-        else if (S.path_len > 0) {
-            unsigned long long off = atomicAdd(O.path_cursor, (unsigned long long)S.path_len);
-            if ((long long)(off + S.path_len) > O.path_capacity) { S.status = HL_STATUS_CAPACITY; S.path_len = 0; }
-            S.path_off = (long long)off;
-        }
-    }
-    __syncwarp();
-    if (S.status == HL_STATUS_OK && S.path_len > 0) {
-        const int len = S.chain_len;
-        for (int c = lane; c < len; c += 32) {
-            const int node = W.hslot[len - 1 - c];          // c-th node from the start side
-            long long off = S.path_off;
-            for (int q = 0; q < c; ++q) off += W.nsteps[W.hslot[len - 1 - q]] + 1;
-            const int par = W.nparent[node];
-            const int p = W.nprim[node], n = W.nsteps[node];
-            const double ys = P.yaw_step[p];
-            const double init_yaw = angle_wrap(xadd(W.nyaw[par], ys));
-            const double stop = xadd(init_yaw, xmul(ys, (double)(n + 1)));
-            const double delta = xsub(stop, init_yaw);
-            const double step = xdiv(delta, (double)(n + 1));
-            double ax = 0.0, ay = 0.0;
-            for (int i = 0; i <= n; ++i) {
-                const double yw = rollout_yaw(init_yaw, stop, step, delta, n + 1, i);
-                const double txv = xmul(xmul(P.res, m_cos(yw)), P.dir[p]);
-                const double tyv = xmul(xmul(P.res, m_sin(yw)), P.dir[p]);
-                ax = (i == 0) ? txv : xadd(ax, txv);
-                ay = (i == 0) ? tyv : xadd(ay, tyv);
-                O.path_x[off + i] = xadd(W.nx[par], ax);
-                O.path_y[off + i] = xadd(W.ny[par], ay);
-                O.path_yaw[off + i] = rollout_yaw(init_yaw, stop, step, delta, n + 1, i + 1);
-                O.path_k[off + i] = P.curv[p];
-                O.path_dir[off + i] = (int8_t)P.dir[p];
-            }
-        }
-        if (S.arrival == 1 && P.pawn) {                 // the Dubins course of the goal extension: rows kept in the scratch
-            const int cnt = S.dub_rows;
-            const double* rx = W.dub + 9 * (size_t)P.dub_cap;
-            const double* ry = rx + P.dub_cap; const double* ryaw = ry + P.dub_cap; const double* rk = ryaw + P.dub_cap;
-            const long long off = S.path_off + (S.path_len - cnt);
-            for (int j = lane; j < cnt; j += 32) {
-                O.path_x[off + j] = rx[j]; O.path_y[off + j] = ry[j]; O.path_yaw[off + j] = ryaw[j];
-                O.path_k[off + j] = rk[j]; O.path_dir[off + j] = (int8_t)1;
-            }
-        } else if (S.arrival == 1) {
-            const RsPlan& plan = (S.rs_pick < AW_MAX_PLANS) ? S.plans[S.rs_pick] : S.plan_tmp;
-            const double q0[3] = {S.cx, S.cy, S.cyaw};
-            const double cq = m_cos(-q0[2]), sq = m_sin(-q0[2]);
-            const long long off = S.path_off + (S.path_len - plan.npts);
-            for (int j = lane; j < plan.npts; j += 32) {
-                double lx, ly, lyaw, wx, wy, wyaw;
-                int cs, dir;
-                rs_sample_local(plan, j, P.maxc, lx, ly, lyaw, cs, dir);
-                rs_to_world(q0, cq, sq, lx, ly, lyaw, wx, wy, wyaw);
-                O.path_x[off + j] = wx; O.path_y[off + j] = wy; O.path_yaw[off + j] = wyaw;
-                O.path_k[off + j] = cs == 0 ? 0.0 : (cs > 0 ? P.maxc : -P.maxc);
-                O.path_dir[off + j] = (int8_t)dir;
-            }
-        }
-    }
-    __syncwarp();
+// Results of a finished scenario: expanded keys, path, record; then the used hash positions are reset for the next
+// scenario of this warp.  Inlined: as a call of its own around the write-out call, the kernel spills more.
+__device__ __forceinline__ void finalize_scenario(AwSmem& S, const AsWs& W, const AsParams& P, const AsOut& O, int lane) {
+    const RsPlan* plan = P.pawn ? nullptr : (S.rs_pick >= 0 && S.rs_pick < AW_MAX_PLANS ? &S.plans[S.rs_pick] : &S.plan_tmp);
+    const AsWritten w = write_outputs(W, P, O, S.status, S.n_closed, S.cur, S.arrival, S.start_key, S.goal_key, plan,
+                                      S.dub_rows, lane);
     if (lane == 0) {
-        HlPlanResult r;
-        r.status = S.status;
-        r.counter = (S.status == HL_STATUS_START_GOAL_BLOCKED) ? 0 : S.counter;
-        r.n_expanded = S.n_closed;
-        r.arrival = S.arrival;
-        r.path_len = S.path_len;
-        r.rs_word = S.rs_word;
-        r.path_offset = S.path_off;
-        r.keys_offset = koff;
-        r.goal_cost = S.goal_cost;
-        r.n_pose_checks = (long long)S.n_checks;
-        r.n_pose_checks_ref = (S.status == HL_STATUS_START_GOAL_BLOCKED) ? 0 : (long long)S.n_ref;
-        r.n_exact = (long long)S.n_exact;
-        long long _n = clock64();
-        S.t_phase[PH_OUTPUT] += _n - S.t_last;
+        S.t_phase[PH_OUTPUT] += clock64() - S.t_last;
         long long tot = 0;
         for (int k = 0; k < AS_N_PHASES; ++k) tot += S.t_phase[k];
-        r.cycles = tot;
-        O.results[sc] = r;
+        write_record(O, S.scen, w, S.arrival, S.rs_word, S.goal_cost, S.counter, S.n_checks, S.n_exact, S.n_ref, tot);
         for (int k = 0; k < AS_N_PHASES; ++k) atomicAdd(O.phase_cycles + k, (unsigned long long)S.t_phase[k]);
     }
-    // reset the used hash positions for the next scenario of this warp
     for (int i = lane; i < S.n_nodes; i += 32) W.hkey[W.nhpos[i]] = KEY_EMPTY;
     __syncwarp();
 }
 
-// Start / goal feasibility (:76-80, :516-519), start node and its priority (:500-510).
 __device__ __noinline__ void setup_scenario(AwSmem& S, const AsWs& W, const AsParams& P, const EnvBatchDev& eb,
-                                            const EnvDesc& D, const EnvSmem& E, int hmask, unsigned FLAGS, int lane) {
-    int bad = 0;
-    if (lane < 2) {
-        const double* q = lane == 0 ? S.start : S.goal;
-        unsigned amb = FLAGS;
-        int r = pose_filter(D, E, q[0], q[1], q[2], FLAGS, &amb);
-        bad = (r == HL_HIT) || (r == HL_AMBIG && pose_exact(eb, D, q[0], q[1], q[2], amb));
-    }
-    bad = __any_sync(FULL, bad);
-    double h = warp_state_cost(eb, D, S.start[0], S.start[1], S.start[2], lane);
+                                            const EnvDesc& D, const EnvSmem& E, unsigned FLAGS, int lane) {
+    const AsStart st = start_node(W, P, eb, D, E, S.start, S.goal, FLAGS, lane);
     if (lane == 0) {
-        int ix, iy, iw;
-        long long sk = 0, gk = 0;
-        bool ok = make_key(S.start[0], S.start[1], S.start[2], P.res, P.yaw_res, ix, iy, iw, sk);
-        ok = make_key(S.goal[0], S.goal[1], S.goal[2], P.res, P.yaw_res, ix, iy, iw, gk) && ok;
-        S.start_key = sk; S.goal_key = gk;
-        if (!ok) S.status = HL_STATUS_CAPACITY;
-        else if (bad) S.status = HL_STATUS_START_GOAL_BLOCKED;
-        else {
-            W.nx[0] = S.start[0]; W.ny[0] = S.start[1]; W.nyaw[0] = S.start[2]; W.ng[0] = 0.0;
-            W.nkey[0] = sk; W.nparent[0] = 0; W.nprim[0] = -1; W.nsteps[0] = 0; W.nstate[0] = 0;
-            W.nheap[0] = -1;
-            int pos;
-            hash_find(W, hmask, sk, &pos);
-            W.hkey[pos] = sk; W.hval[pos] = 0; W.nhpos[0] = pos;
-            S.n_nodes = 1;
-            double prio = xmul(P.hybrid_cost, h);
-            prio = (prio > 0.0) ? prio : 0.0;           // max(start.cost = 0, 50*h)
-            heap_set(W, S.heap_n, 0, prio);
-        }
+        S.start_key = st.start_key; S.goal_key = st.goal_key; S.status = st.status;
+        if (st.status < 0) { S.n_nodes = 1; heap_set(W, S.heap_n, 0, st.prio); }
     }
     __syncwarp();
 }
@@ -349,7 +168,7 @@ __device__ __noinline__ void pawn_shot(AwSmem& S, const AsWs& W, const AsParams&
 
 __global__ void __launch_bounds__(AW_WARPS * 32, AW_MIN_CTAS)
 k_hybrid_astar_w(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen, AsParams P, char* ws_base,
-                 size_t ws_stride, unsigned int* work_counter, AwOut O) {
+                 size_t ws_stride, unsigned int* work_counter, AsOut O) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     AwSmem& S = reinterpret_cast<AwSmem*>(smem_raw)[wid];
@@ -382,14 +201,14 @@ k_hybrid_astar_w(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                 for (int k = 0; k < 3; ++k) { S.start[k] = s.start[k]; S.goal[k] = s.goal[k]; }
                 S.n_nodes = 0; S.heap_n = 0; S.counter = 0; S.n_closed = 0;
                 S.status = -1; S.arrival = 0; S.rs_word = -1; S.goal_cost = 0.0; S.rs_pick = -1;
-                S.n_checks = 0; S.n_exact = 0; S.n_ref = 0; S.path_len = 0; S.path_off = 0; S.chain_len = 0;
+                S.n_checks = 0; S.n_exact = 0; S.n_ref = 0;
                 for (int k = 0; k < AS_N_PHASES; ++k) S.t_phase[k] = 0;
                 S.t_last = clock64();
             }
             __syncwarp();
             Dp = eb.desc + S.env;
-            stage_env_warp(eb, *Dp, S.envf, AW_ENV_FLOATS, E, lane);
-            setup_scenario(S, W, P, eb, *Dp, E, hmask, FLAGS, lane);
+            stage_env_warp(eb, *Dp, S.envf, AS_ENV_FLOATS, E, lane);
+            setup_scenario(S, W, P, eb, *Dp, E, FLAGS, lane);
             TICK(PH_SETUP);
             if (S.status >= 0) finalize_scenario(S, W, P, O, lane);        // blocked / capacity: done already
             else if (lane == 0) S.state = ST_SEARCH;
@@ -801,7 +620,7 @@ static int ls_state_get(hl_ctx* ctx, LsState** out) {
 }
 
 static int ls_run(hl_ctx* ctx, const hl_env_batch* envs, const HlScenario* d_scen, int n_scen, const AsParams& P,
-                  const AwOut& O, cudaStream_t st) {
+                  const AsOut& O, cudaStream_t st) {
     LsState* L = nullptr;
     if (ls_state_get(ctx, &L)) return 1;
     const size_t stride = as_ws_bytes(P.cap_nodes, P.hash_size, P.max_nodes, P.dub_cap);
@@ -940,7 +759,7 @@ extern "C" int hl_hybrid_astar_batch(hl_ctx* ctx, const hl_env_batch* envs, cons
     const bool spec = !P.pawn && ctx->astar_variant != HL_ASTAR_WARP;
     cudaStream_t st = (cudaStream_t)stream;
     HL_CUDA_OK(cudaStreamWaitEvent(st, (cudaEvent_t)ctx->astar_done, 0));      // no-op until the first record
-    AwOut O;
+    AsOut O;
     O.results = d_results; O.expanded_keys = d_expanded_keys;
     O.keys_capacity = (long long)keys_capacity; O.keys_cursor = d_keys_cursor;
     O.path_x = d_path_x; O.path_y = d_path_y; O.path_yaw = d_path_yaw; O.path_k = d_path_k; O.path_dir = d_path_dir;
@@ -1000,12 +819,12 @@ extern "C" int hl_hybrid_astar_batch(hl_ctx* ctx, const hl_env_batch* envs, cons
         int* defer_count = (int*)(ctx->d_counters + 4);
         HL_CUDA_OK(cudaMemsetAsync(ctx->d_counters + 4, 0, sizeof(unsigned int), st));
         HL_CUDA_OK(cudaMemsetAsync(ctx->d_counters + 8, 0, sizeof(unsigned int), st));
-        AwOut O1 = O;
+        AsOut O1 = O;
         O1.first_only = 1; O1.defer_list = ctx->astar_defer; O1.defer_count = defer_count;
         k_hybrid_astar_s<<<grid, threads, smem, st>>>(envs->dev, d_scen, n_scen, P, (char*)ctx->astar_ws, stride,
                                                       ctx->d_counters, O1);
         HL_CUDA_OK(cudaGetLastError());
-        AwOut O2 = O;
+        AsOut O2 = O;
         O2.order = ctx->astar_defer; O2.order_count = defer_count;
         k_hybrid_astar_s<<<grid, threads, smem, st>>>(envs->dev, d_scen, n_scen, P, (char*)ctx->astar_ws, stride,
                                                       ctx->d_counters + 8, O2);

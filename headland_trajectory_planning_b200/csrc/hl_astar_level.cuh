@@ -69,7 +69,7 @@ struct LsCall {                             // per-call block in device memory, 
     int* n_act;                             // [2]
     int2* words;                            // (scenario, rank) of every word to sample this iteration
     int* n_words;
-    AwOut O;
+    AsOut O;
 };
 
 #define LS_FLAGS (HL_CHECK_OBSTACLES | HL_CHECK_BOUNDARY | HL_CHECK_LANE)
@@ -85,12 +85,11 @@ __global__ void __launch_bounds__(LS_THREADS) ls_setup(const LsCall* __restrict_
     const int lane = threadIdx.x & 31;
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     const AsParams& P = C.P;
-    const int hmask = P.hash_size - 1;
     for (int sc = warp; sc < C.n_scen; sc += n_warps) {
         LsScn& S = C.scn[sc];
         const AsWs W = ls_ws(C, sc);
         for (int i = lane; i < P.hash_size; i += 32) W.hkey[i] = KEY_EMPTY;
-        const HlScenario s = C.scen[sc];
+        const HlScenario& s = C.scen[sc];
         if (lane == 0) {
             S.env = s.env_id;
             for (int k = 0; k < 3; ++k) { S.start[k] = s.start[k]; S.goal[k] = s.goal[k]; }
@@ -104,35 +103,13 @@ __global__ void __launch_bounds__(LS_THREADS) ls_setup(const LsCall* __restrict_
         const EnvDesc& D = C.eb.desc[s.env_id];
         EnvSmem E;
         global_env(C.eb, D, E);
-        int bad = 0;
-        if (lane < 2) {
-            const double* q = lane == 0 ? s.start : s.goal;
-            unsigned amb = LS_FLAGS;
-            int r = pose_filter(D, E, q[0], q[1], q[2], LS_FLAGS, &amb);
-            bad = (r == HL_HIT) || (r == HL_AMBIG && pose_exact(C.eb, D, q[0], q[1], q[2], amb));
-        }
-        bad = __any_sync(FULL, bad);
-        const double h = warp_state_cost(C.eb, D, s.start[0], s.start[1], s.start[2], lane);
+        const AsStart st = start_node(W, P, C.eb, D, E, s.start, s.goal, LS_FLAGS, lane);
         if (lane == 0) {
-            int ix, iy, iw;
-            long long sk = 0, gk = 0;
-            bool ok = make_key(s.start[0], s.start[1], s.start[2], P.res, P.yaw_res, ix, iy, iw, sk);
-            ok = make_key(s.goal[0], s.goal[1], s.goal[2], P.res, P.yaw_res, ix, iy, iw, gk) && ok;
-            S.start_key = sk; S.goal_key = gk;
-            if (!ok) S.status = HL_STATUS_CAPACITY;
-            else if (bad) S.status = HL_STATUS_START_GOAL_BLOCKED;
-            else {
-                W.nx[0] = s.start[0]; W.ny[0] = s.start[1]; W.nyaw[0] = s.start[2]; W.ng[0] = 0.0;
-                W.nkey[0] = sk; W.nparent[0] = 0; W.nprim[0] = -1; W.nsteps[0] = 0; W.nstate[0] = 0;
-                W.nheap[0] = -1;
-                int pos;
-                hash_find(W, hmask, sk, &pos);
-                W.hkey[pos] = sk; W.hval[pos] = 0; W.nhpos[0] = pos;
+            S.start_key = st.start_key; S.goal_key = st.goal_key; S.status = st.status;
+            if (st.status < 0) {
                 S.n_nodes = 1;
-                double prio = xmul(P.hybrid_cost, h);
-                prio = (prio > 0.0) ? prio : 0.0;           // max(start.cost = 0, 50*h)
                 int hn = 0;
-                heap_set(W, hn, 0, prio);
+                heap_set(W, hn, 0, st.prio);
                 S.heap_n = hn;
                 C.act[0][atomicAdd(&C.n_act[0], 1)] = sc;
             }
@@ -533,129 +510,23 @@ __global__ void __launch_bounds__(LS_THREADS) ls_cost(const LsCall* __restrict__
 // Warp per scenario: expanded keys, path (get_path_from_expanded_nodes, :429-454), result record.
 __global__ void __launch_bounds__(LS_THREADS) ls_finalize(const LsCall* __restrict__ Cp) {
     __shared__ RsPlan s_plan[LS_THREADS / 32];
-    __shared__ int s_len[LS_THREADS / 32], s_plen[LS_THREADS / 32], s_status[LS_THREADS / 32];
-    __shared__ long long s_off[LS_THREADS / 32];
     const LsCall& C = *Cp;
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     const AsParams& P = C.P;
-    const AwOut& O = C.O;
     RsPlan& plan = s_plan[wib];
     for (int sc = warp; sc < C.n_scen; sc += n_warps) {
-        LsScn& S = C.scn[sc];
+        const LsScn& S = C.scn[sc];
         const AsWs W = ls_ws(C, sc);
-        const LsShot& T = C.shot[sc];
-        int status = S.status;
-        if (status < 0) status = HL_STATUS_CAPACITY;             // iteration budget exhausted (cannot happen)
-        const int n_closed = S.n_closed;
-        long long koff = 0;
-        if (lane == 0 && n_closed > 0) {
-            koff = (long long)atomicAdd(O.keys_cursor, (unsigned long long)n_closed);
-            if (koff + n_closed > O.keys_capacity) koff = -1;
-        }
-        koff = __shfl_sync(FULL, koff, 0);
-        int nk = n_closed;
-        if (koff < 0) { status = HL_STATUS_CAPACITY; nk = 0; koff = 0; }
-        {
-            int32_t* ek = O.expanded_keys + (size_t)koff * 3;
-            for (int i = lane; i < nk; i += 32) {
-                int ix, iy, iw;
-                unpack_key(W.nkey[W.corder[i]], ix, iy, iw);
-                ek[3 * i] = ix; ek[3 * i + 1] = iy; ek[3 * i + 2] = iw;
-            }
-        }
-        const int cur = (n_closed > 0) ? W.corder[n_closed - 1] : 0;       // the node the search ended on
-        const double q0[3] = {W.nx[cur], W.ny[cur], W.nyaw[cur]};
-        const double cq = m_cos(-q0[2]), sq = m_sin(-q0[2]);
+        const int status = S.status < 0 ? HL_STATUS_CAPACITY : S.status;   // iteration budget exhausted (cannot happen)
+        if (lane == 0 && S.arrival == 1)                                   // the goal extension: the winning word
+            rs_make_plan(S.rs_word, C.shot[sc].rs_lens[S.rs_word], P.maxc, xmul(P.res, P.maxc), plan);
         __syncwarp();
-        if (lane == 0) {
-            int len = 0, poses = 0, rs_pts = 0, path_len = 0;
-            long long path_off = 0;
-            if (status == HL_STATUS_OK) {
-                bool ok = true;
-                if (S.goal_key != S.start_key) {
-                    for (int node = cur; node != 0; node = W.nparent[node]) {
-                        if (len >= P.cap_nodes) { ok = false; break; }
-                        W.hslot[len++] = node;                                   // the heap is dead by now
-                        poses += W.nsteps[node] + 1;
-                    }
-                    if (S.arrival == 1) {
-                        rs_make_plan(S.rs_word, T.rs_lens[S.rs_word], P.maxc, xmul(P.res, P.maxc), plan);
-                        rs_pts = plan.npts;
-                    }
-                }
-                path_len = poses + rs_pts;
-                if (!ok || path_len > P.max_path_poses) { status = HL_STATUS_CAPACITY; path_len = 0; }
-                else if (path_len > 0) {
-                    unsigned long long off = atomicAdd(O.path_cursor, (unsigned long long)path_len);
-                    if ((long long)(off + path_len) > O.path_capacity) { status = HL_STATUS_CAPACITY; path_len = 0; }
-                    path_off = (long long)off;
-                }
-            }
-            s_len[wib] = len; s_plen[wib] = path_len; s_status[wib] = status; s_off[wib] = path_off;
-        }
-        __syncwarp();
-        status = s_status[wib];
-        const int path_len = s_plen[wib];
-        const long long path_off = s_off[wib];
-        if (status == HL_STATUS_OK && path_len > 0) {
-            const int len = s_len[wib];
-            for (int c = lane; c < len; c += 32) {
-                const int node = W.hslot[len - 1 - c];
-                long long off = path_off;
-                for (int q = 0; q < c; ++q) off += W.nsteps[W.hslot[len - 1 - q]] + 1;
-                const int par = W.nparent[node];
-                const int p = W.nprim[node], n = W.nsteps[node];
-                const double ys = P.yaw_step[p];
-                const double init_yaw = angle_wrap(xadd(W.nyaw[par], ys));
-                const double stop = xadd(init_yaw, xmul(ys, (double)(n + 1)));
-                const double delta = xsub(stop, init_yaw);
-                const double step = xdiv(delta, (double)(n + 1));
-                double ax = 0.0, ay = 0.0;
-                for (int i = 0; i <= n; ++i) {
-                    const double yw = rollout_yaw(init_yaw, stop, step, delta, n + 1, i);
-                    const double txv = xmul(xmul(P.res, m_cos(yw)), P.dir[p]);
-                    const double tyv = xmul(xmul(P.res, m_sin(yw)), P.dir[p]);
-                    ax = (i == 0) ? txv : xadd(ax, txv);
-                    ay = (i == 0) ? tyv : xadd(ay, tyv);
-                    O.path_x[off + i] = xadd(W.nx[par], ax);
-                    O.path_y[off + i] = xadd(W.ny[par], ay);
-                    O.path_yaw[off + i] = rollout_yaw(init_yaw, stop, step, delta, n + 1, i + 1);
-                    O.path_k[off + i] = P.curv[p];
-                    O.path_dir[off + i] = (int8_t)P.dir[p];
-                }
-            }
-            if (S.arrival == 1) {
-                const long long off = path_off + (path_len - plan.npts);
-                for (int j = lane; j < plan.npts; j += 32) {
-                    double lx, ly, lyaw, wx, wy, wyaw;
-                    int cs, dir;
-                    rs_sample_local(plan, j, P.maxc, lx, ly, lyaw, cs, dir);
-                    rs_to_world(q0, cq, sq, lx, ly, lyaw, wx, wy, wyaw);
-                    O.path_x[off + j] = wx; O.path_y[off + j] = wy; O.path_yaw[off + j] = wyaw;
-                    O.path_k[off + j] = cs == 0 ? 0.0 : (cs > 0 ? P.maxc : -P.maxc);
-                    O.path_dir[off + j] = (int8_t)dir;
-                }
-            }
-        }
-        __syncwarp();
-        if (lane == 0) {
-            HlPlanResult r;
-            r.status = status;
-            r.counter = (status == HL_STATUS_START_GOAL_BLOCKED) ? 0 : S.counter;
-            r.n_expanded = nk;
-            r.arrival = S.arrival;
-            r.path_len = path_len;
-            r.rs_word = (S.arrival == 1) ? S.rs_word : -1;
-            r.path_offset = path_off;
-            r.goal_cost = S.goal_cost;
-            r.n_pose_checks = (long long)S.checks;
-            r.n_pose_checks_ref = (status == HL_STATUS_START_GOAL_BLOCKED) ? 0 : (long long)S.ref;
-            r.n_exact = (long long)S.exact;
-            r.keys_offset = koff;
-            r.cycles = 0;
-            O.results[sc] = r;
-        }
+        const int end = (S.n_closed > 0) ? W.corder[S.n_closed - 1] : 0;   // the node the search ended on
+        const AsWritten w = write_outputs(W, P, C.O, status, S.n_closed, end, S.arrival, S.start_key, S.goal_key, &plan,
+                                          0, lane);
+        if (lane == 0)
+            write_record(C.O, sc, w, S.arrival, S.rs_word, S.goal_cost, S.counter, S.checks, S.exact, S.ref, 0);
         __syncwarp();
     }
 }

@@ -66,10 +66,10 @@ struct AqShot {                          // scratch of one shooter warp
     unsigned char rs_valid[HL_RS_CANDIDATES + 2], rs_accept[HL_RS_CANDIDATES + 2];
     RsProblem rs_prob;
     int rs_npts[HL_RS_CANDIDATES];       // sample count of every word planned so far (evaluation order)
-    int rs_n, rs_pick, rs_word, rs_assert;
+    int rs_n, rs_word, rs_assert;
     double rs_goal_cost;
     RsPlan plans[AQ_MAX_PLANS];
-    RsPlan plan_tmp;
+    RsPlan plan_tmp;                     // single words; at a successful shot the winning word (the goal extension)
     unsigned long long s_checks, s_exact, s_ref;
     volatile int done_epoch;             // this shooter finished the epoch
 };
@@ -103,10 +103,9 @@ struct AqSmem {                          // one per scenario slot, shared by its
     long long te_last, te[AS_N_PHASES];      // expander phase timers (lane 0 cycles)
     long long ts_last, ts[AS_N_PHASES];      // shooter phase timers
     // result assembly
-    int status, arrival, fin_closed, fin_counter, chain_len, path_len, win;
+    int status, arrival, fin_closed, fin_counter, win;
     double goal_cost;
-    long long path_off;
-    __align__(16) float envf[AW_ENV_FLOATS];
+    __align__(16) float envf[AS_ENV_FLOATS];
     double gx[AQ_GUIDE_CAP], gy[AQ_GUIDE_CAP];       // guide polyline of the scenario (calculate_state_cost's argmin)
     double gyaw[AQ_GUIDE_CAP], gs[AQ_GUIDE_CAP];     // ... its headings and arc lengths
     double pds[HL_MAX_PRIMS][AS_ROLL];               // step lengths of the rolled-out primitives (g-cost)
@@ -307,120 +306,22 @@ __device__ __noinline__ bool aq_word_collides(const EnvSmem& Ers, const EnvBatch
     return infeasible != 0;
 }
 
-// Result record + path of a finished scenario (expander warp, after the shooter reported).
-__device__ __noinline__ void finalize_spec(AqSmem& S, const AsWs& W, const AsParams& P, const AwOut& O, int lane) {
-    const int sc = S.scen;
+// Result record + path of a finished scenario (expander warp, after the shooter reported).  Inlined: as a call of its
+// own around the write-out call, the kernel spills more.
+__device__ __forceinline__ void finalize_spec(AqSmem& S, const AsWs& W, const AsParams& P, const AsOut& O, int lane) {
     const int n_closed = S.fin_closed;
-    long long koff = 0;
-    if (lane == 0 && n_closed > 0) {
-        koff = (long long)atomicAdd(O.keys_cursor, (unsigned long long)n_closed);
-        if (koff + n_closed > O.keys_capacity) koff = -1;
-    }
-    koff = __shfl_sync(FULL, koff, 0);
-    int nk = n_closed;
-    if (koff < 0) { if (lane == 0) S.status = HL_STATUS_CAPACITY; nk = 0; koff = 0; }
-    __syncwarp();
-    {
-        int32_t* ek = O.expanded_keys + (size_t)koff * 3;
-        for (int i = lane; i < nk; i += 32) {
-            int ix, iy, iw;
-            unpack_key(W.nkey[W.corder[i]], ix, iy, iw);
-            ek[3 * i] = ix; ek[3 * i + 1] = iy; ek[3 * i + 2] = iw;
-        }
-    }
-    const int cur = (n_closed > 0) ? W.corder[n_closed - 1] : 0;       // the node the search ended on
-    if (lane == 0 && S.status == HL_STATUS_OK) {
-        int len = 0, poses = 0, rs_pts = 0;
-        bool ok = true;
-        if (S.goal_key != S.start_key) {
-            for (int node = cur; node != 0; node = W.nparent[node]) {
-                if (len >= P.cap_nodes) { ok = false; break; }
-                W.hslot[len++] = node;                                   // the heap is dead by now
-                poses += W.nsteps[node] + 1;
-            }
-            if (S.arrival == 1) { const AqShot& T = S.sh[S.win]; rs_pts = (T.rs_pick < AQ_MAX_PLANS ? T.plans[T.rs_pick] : T.plan_tmp).npts; }
-        }
-        S.chain_len = len;
-        S.path_len = poses + rs_pts;
-        if (!ok || S.path_len > P.max_path_poses) { S.status = HL_STATUS_CAPACITY; S.path_len = 0; }
-        else if (S.path_len > 0) {
-            unsigned long long off = atomicAdd(O.path_cursor, (unsigned long long)S.path_len);
-            if ((long long)(off + S.path_len) > O.path_capacity) { S.status = HL_STATUS_CAPACITY; S.path_len = 0; }
-            S.path_off = (long long)off;
-        }
-    }
-    __syncwarp();
-    if (S.status == HL_STATUS_OK && S.path_len > 0) {
-        const int len = S.chain_len;
-        for (int c = lane; c < len; c += 32) {
-            const int node = W.hslot[len - 1 - c];
-            long long off = S.path_off;
-            for (int q = 0; q < c; ++q) off += W.nsteps[W.hslot[len - 1 - q]] + 1;
-            const int par = W.nparent[node];
-            const int p = W.nprim[node], n = W.nsteps[node];
-            const double ys = P.yaw_step[p];
-            const double init_yaw = angle_wrap(xadd(W.nyaw[par], ys));
-            const double stop = xadd(init_yaw, xmul(ys, (double)(n + 1)));
-            const double delta = xsub(stop, init_yaw);
-            const double step = xdiv(delta, (double)(n + 1));
-            double ax = 0.0, ay = 0.0;
-            for (int i = 0; i <= n; ++i) {
-                const double yw = rollout_yaw(init_yaw, stop, step, delta, n + 1, i);
-                const double txv = xmul(xmul(P.res, m_cos(yw)), P.dir[p]);
-                const double tyv = xmul(xmul(P.res, m_sin(yw)), P.dir[p]);
-                ax = (i == 0) ? txv : xadd(ax, txv);
-                ay = (i == 0) ? tyv : xadd(ay, tyv);
-                O.path_x[off + i] = xadd(W.nx[par], ax);
-                O.path_y[off + i] = xadd(W.ny[par], ay);
-                O.path_yaw[off + i] = rollout_yaw(init_yaw, stop, step, delta, n + 1, i + 1);
-                O.path_k[off + i] = P.curv[p];
-                O.path_dir[off + i] = (int8_t)P.dir[p];
-            }
-        }
-        if (S.arrival == 1) {
-            const AqShot& T = S.sh[S.win];
-            const RsPlan& plan = (T.rs_pick < AQ_MAX_PLANS) ? T.plans[T.rs_pick] : T.plan_tmp;
-            const double q0[3] = {W.nx[cur], W.ny[cur], W.nyaw[cur]};
-            const double cq = m_cos(-q0[2]), sq = m_sin(-q0[2]);
-            const long long off = S.path_off + (S.path_len - plan.npts);
-            for (int j = lane; j < plan.npts; j += 32) {
-                double lx, ly, lyaw, wx, wy, wyaw;
-                int cs, dir;
-                rs_sample_local(plan, j, P.maxc, lx, ly, lyaw, cs, dir);
-                rs_to_world(q0, cq, sq, lx, ly, lyaw, wx, wy, wyaw);
-                O.path_x[off + j] = wx; O.path_y[off + j] = wy; O.path_yaw[off + j] = wyaw;
-                O.path_k[off + j] = cs == 0 ? 0.0 : (cs > 0 ? P.maxc : -P.maxc);
-                O.path_dir[off + j] = (int8_t)dir;
-            }
-        }
-    }
-    __syncwarp();
+    const int end = (n_closed > 0) ? W.corder[n_closed - 1] : 0;       // the node the search ended on
+    const AqShot& T = S.sh[S.win];
+    const AsWritten w = write_outputs(W, P, O, S.status, n_closed, end, S.arrival, S.start_key, S.goal_key, &T.plan_tmp,
+                                      0, lane);
     if (lane == 0) {
-        HlPlanResult r;
-        r.status = S.status;
-        r.counter = (S.status == HL_STATUS_START_GOAL_BLOCKED) ? 0 : S.fin_counter;
-        r.n_expanded = nk;
-        r.arrival = S.arrival;
-        r.path_len = S.path_len;
-        r.rs_word = (S.arrival == 1) ? S.sh[S.win].rs_word : -1;
-        r.path_offset = S.path_off;
-        r.goal_cost = S.goal_cost;
-        unsigned long long sc_ = S.e_checks, se_ = S.e_exact;
-        for (int k = 0; k < AQ_SHOOTERS; ++k) { sc_ += S.sh[k].s_checks; se_ += S.sh[k].s_exact; }
-        r.n_pose_checks = (long long)sc_;
-        r.n_exact = (long long)se_;
-        {
-            // algorithmic count: shots of pops <= the final one (the shooter stops there) + the expansions of the
-            // pops BEFORE a successful shot (the expander may have run ahead; that work is not the reference's)
-            unsigned long long ref = 0;
-            for (int k = 0; k < AQ_SHOOTERS; ++k) ref += S.sh[k].s_ref;
-            const bool shot_won = (S.arrival == 1) || (S.status == HL_STATUS_RS_ASSERT);
-            ref += (shot_won && n_closed > 0) ? (unsigned long long)W.cref[n_closed - 1] : S.e_ref;
-            r.n_pose_checks_ref = (S.status == HL_STATUS_START_GOAL_BLOCKED) ? 0 : (long long)ref;
-        }
-        r.keys_offset = koff;
-        r.cycles = clock64() - S.t0;
-        O.results[sc] = r;
+        unsigned long long checks = S.e_checks, exact = S.e_exact, ref = 0;
+        for (int k = 0; k < AQ_SHOOTERS; ++k) { checks += S.sh[k].s_checks; exact += S.sh[k].s_exact; ref += S.sh[k].s_ref; }
+        // algorithmic count: shots of pops <= the final one (the shooter stops there) + the expansions of the
+        // pops BEFORE a successful shot (the expander may have run ahead; that work is not the reference's)
+        const bool shot_won = (S.arrival == 1) || (w.status == HL_STATUS_RS_ASSERT);
+        ref += (shot_won && n_closed > 0) ? (unsigned long long)W.cref[n_closed - 1] : S.e_ref;
+        write_record(O, S.scen, w, S.arrival, T.rs_word, S.goal_cost, S.fin_counter, checks, exact, ref, clock64() - S.t0);
         for (int k = 0; k < AS_N_PHASES; ++k) {
             const long long v = S.te[k] + S.ts[k];
             if (v) atomicAdd(O.phase_cycles + k, (unsigned long long)v);
@@ -432,7 +333,7 @@ __device__ __noinline__ void finalize_spec(AqSmem& S, const AsWs& W, const AsPar
 
 __global__ void __launch_bounds__(AQ_SLOTS * AQ_WARPS_PER_SLOT * 32, 1)
 k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen, AsParams P, char* ws_base,
-                 size_t ws_stride, unsigned int* work_counter, AwOut O) {
+                 size_t ws_stride, unsigned int* work_counter, AsOut O) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 #if AQ_WARP_MAP == 1 && AQ_SLOTS == 5 && AQ_WARPS_PER_SLOT == 3
@@ -501,7 +402,7 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                     E.n_obs = D0.n_obs; E.n_field = D0.n_field; E.n_seg = D0.n_seg; E.all_rect = D0.all_rect;
                     E.eps = D0.eps; E.reach = D0.reach;
                     for (int k = 0; k < 4; ++k) E.ext[k] = (float)D0.body_ext[k];
-                    if (n_o + n_f + n_s <= AW_ENV_FLOATS) { E.obs = S.envf; E.field = S.envf + n_o; E.seg = S.envf + n_o + n_f; }
+                    if (n_o + n_f + n_s <= AS_ENV_FLOATS) { E.obs = S.envf; E.field = S.envf + n_o; E.seg = S.envf + n_o + n_f; }
                     else {
                         E.obs = eb.obs32 + (size_t)HL_OBS32_STRIDE * D0.obs_off;
                         E.field = eb.field32 + HL_FIELD32_STRIDE * (size_t)D0.field_off;
@@ -537,7 +438,6 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                 if (lane == 0) {
                     const int cur = W.corder[i];
                     T.s_cur = cur; T.sx = W.nx[cur]; T.sy = W.ny[cur]; T.syaw = W.nyaw[cur]; T.sg = W.ng[cur];
-                    T.rs_pick = -1;
                 }
                 __syncwarp();
                 q0[0] = T.sx; q0[1] = T.sy; q0[2] = T.syaw;
@@ -675,7 +575,6 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                     rs_make_plans_warp(T.rs_acc, T.rs_lens, T.rs_npts, winner, 1, &T.plan_tmp, q0, cq, sq, D.origin, P.maxc, stepn, lane);   // the result path's plan
                     if (lane == 0) {
                         T.s_ref += tally;
-                        T.rs_pick = AQ_MAX_PLANS;                // = plan_tmp (finalize_spec)
                         T.rs_word = T.rs_acc[winner]; T.rs_goal_cost = T.rs_prio[winner];
                     }
                     success = true;
@@ -726,7 +625,7 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
             S.status = -1; S.arrival = 0; S.goal_cost = 0.0; S.ew_status = -1; S.ew_arrival2 = 0;
             S.e_checks = 0; S.e_exact = 0; S.e_ref = 0; S.win = 0;
             for (int k = 0; k < AQ_SHOOTERS; ++k) { S.sh[k].s_checks = 0; S.sh[k].s_exact = 0; S.sh[k].s_ref = 0; S.sh[k].rs_assert = 0; }
-            S.path_len = 0; S.path_off = 0; S.chain_len = 0; S.fin_closed = 0; S.fin_counter = 0;
+            S.fin_closed = 0; S.fin_counter = 0;
             S.popped = 0; S.ew_done = 0; S.shot_limit = 0; S.shot_best = AQ_NO_HIT;
             S.t0 = clock64();
             for (int k = 0; k < AS_N_PHASES; ++k) { S.te[k] = 0; S.ts[k] = 0; }
@@ -735,7 +634,7 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
         __syncwarp();
         Dp = eb.desc + S.env;
         const EnvDesc& D = *Dp;
-        stage_env_warp(eb, D, S.envf, AW_ENV_FLOATS, E, lane);
+        stage_env_warp(eb, D, S.envf, AS_ENV_FLOATS, E, lane);
         if (D.n_guide <= AQ_GUIDE_CAP) {
             for (int i = lane; i < D.n_guide; i += 32) {
                 S.gx[i] = eb.guide_x[D.guide_off + i]; S.gy[i] = eb.guide_y[D.guide_off + i];
@@ -743,37 +642,11 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
             }
         }
         if (lane == 0) S.guide_staged = D.n_guide <= AQ_GUIDE_CAP ? 1 : 0;
-        // start / goal feasibility and start node (shared helper works on an AwSmem-like view)
         {
-            int bad = 0;
-            if (lane < 2) {
-                const double* q = lane == 0 ? S.start : S.goal;
-                unsigned amb = FLAGS;
-                int r = pose_filter(D, E, q[0], q[1], q[2], FLAGS, &amb);
-                bad = (r == HL_HIT) || (r == HL_AMBIG && pose_exact(eb, D, q[0], q[1], q[2], amb));
-            }
-            bad = __any_sync(FULL, bad);
-            double h = warp_state_cost(eb, D, S.start[0], S.start[1], S.start[2], lane);
+            const AsStart st = start_node(W, P, eb, D, E, S.start, S.goal, FLAGS, lane);
             if (lane == 0) {
-                int ix, iy, iw;
-                long long sk = 0, gk = 0;
-                bool ok = make_key(S.start[0], S.start[1], S.start[2], P.res, P.yaw_res, ix, iy, iw, sk);
-                ok = make_key(S.goal[0], S.goal[1], S.goal[2], P.res, P.yaw_res, ix, iy, iw, gk) && ok;
-                S.start_key = sk; S.goal_key = gk;
-                if (!ok) S.ew_status = HL_STATUS_CAPACITY;
-                else if (bad) S.ew_status = HL_STATUS_START_GOAL_BLOCKED;
-                else {
-                    W.nx[0] = S.start[0]; W.ny[0] = S.start[1]; W.nyaw[0] = S.start[2]; W.ng[0] = 0.0;
-                    W.nkey[0] = sk; W.nparent[0] = 0; W.nprim[0] = -1; W.nsteps[0] = 0; W.nstate[0] = 0;
-                    W.nheap[0] = -1;
-                    int pos;
-                    hash_find(W, hmask, sk, &pos);
-                    W.hkey[pos] = sk; W.hval[pos] = 0; W.nhpos[0] = pos;
-                    S.n_nodes = 1;
-                    double prio = xmul(P.hybrid_cost, h);
-                    prio = (prio > 0.0) ? prio : 0.0;
-                    aq_heap_set(S, W, S.heap_n, 0, prio);
-                }
+                S.start_key = st.start_key; S.goal_key = st.goal_key; S.ew_status = st.status;
+                if (st.status < 0) { S.n_nodes = 1; aq_heap_set(S, W, S.heap_n, 0, st.prio); }
             }
             __syncwarp();
         }
@@ -860,7 +733,7 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                 E.n_obs = D0.n_obs; E.n_field = D0.n_field; E.n_seg = D0.n_seg; E.all_rect = D0.all_rect;
                 E.eps = D0.eps; E.reach = D0.reach;
                 for (int k = 0; k < 4; ++k) E.ext[k] = (float)D0.body_ext[k];
-                if (n_o + n_f + n_s <= AW_ENV_FLOATS) { E.obs = S.envf; E.field = S.envf + n_o; E.seg = S.envf + n_o + n_f; }
+                if (n_o + n_f + n_s <= AS_ENV_FLOATS) { E.obs = S.envf; E.field = S.envf + n_o; E.seg = S.envf + n_o + n_f; }
                 else {
                     E.obs = eb.obs32 + (size_t)HL_OBS32_STRIDE * D0.obs_off;
                     E.field = eb.field32 + HL_FIELD32_STRIDE * (size_t)D0.field_off;

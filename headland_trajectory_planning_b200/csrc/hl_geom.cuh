@@ -728,29 +728,6 @@ static __device__ bool pose_infeasible(const EnvBatchDev& eb, const EnvDesc& D, 
     return false;
 }
 
-__device__ __forceinline__ void stage_env(const EnvBatchDev& eb, const EnvDesc& D, float* sm, int cap_floats,
-                                          EnvSmem& E, bool& staged) {
-    int need = D.n_obs * HL_OBS32_STRIDE + D.n_field * HL_FIELD32_STRIDE + D.n_seg * 4;
-    E.n_obs = D.n_obs; E.n_field = D.n_field; E.n_seg = D.n_seg; E.all_rect = D.all_rect;
-    E.eps = D.eps; E.reach = D.reach;
-    for (int k = 0; k < 4; ++k) E.ext[k] = (float)D.body_ext[k];
-    const float* g_obs = eb.obs32 + (size_t)HL_OBS32_STRIDE * D.obs_off;
-    const float* g_field = eb.field32 + HL_FIELD32_STRIDE * (size_t)D.field_off;
-    const float* g_seg = eb.seg32 + 4 * (size_t)D.seg_off;
-    staged = need <= cap_floats;
-    if (staged) {
-        float* s_obs = sm;
-        float* s_field = s_obs + D.n_obs * HL_OBS32_STRIDE;
-        float* s_seg = s_field + D.n_field * HL_FIELD32_STRIDE;
-        for (int i = threadIdx.x; i < D.n_obs * HL_OBS32_STRIDE; i += blockDim.x) s_obs[i] = g_obs[i];
-        for (int i = threadIdx.x; i < D.n_field * HL_FIELD32_STRIDE; i += blockDim.x) s_field[i] = g_field[i];
-        for (int i = threadIdx.x; i < D.n_seg * 4; i += blockDim.x) s_seg[i] = g_seg[i];
-        E.obs = s_obs; E.field = s_field; E.seg = s_seg;
-    } else {
-        E.obs = g_obs; E.field = g_field; E.seg = g_seg;
-    }
-}
-
 __device__ __forceinline__ void global_env(const EnvBatchDev& eb, const EnvDesc& D, EnvSmem& E) {
     E.n_obs = D.n_obs; E.n_field = D.n_field; E.n_seg = D.n_seg; E.all_rect = D.all_rect;
     E.eps = D.eps; E.reach = D.reach;
