@@ -12,7 +12,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_NAME = "libheadland_b200.so"
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 HL_MAX_PRIMS = 16
 HL_CAPSULE_VERTS = 66
 HL_RS_CANDIDATES = 46
@@ -62,6 +62,13 @@ class HlSearchParams(C.Structure):
     ]
 
 
+class HlGridField(C.Structure):
+    _fields_ = [
+        ("occ_offset", C.c_int64), ("out_offset", C.c_int64),
+        ("w", C.c_int32), ("h", C.c_int32), ("gi", C.c_int32), ("gj", C.c_int32),
+    ]
+
+
 SCENARIO_DTYPE = np.dtype([("env_id", "<i4"), ("reserved", "<i4"),
                            ("start", "<f8", (3,)), ("goal", "<f8", (3,))])
 RESULT_DTYPE = np.dtype([("status", "<i4"), ("counter", "<i4"), ("n_expanded", "<i4"),
@@ -78,7 +85,7 @@ EXPORTS = [
     "hl_last_error", "hl_abi_version", "hl_ctx_create", "hl_ctx_destroy", "hl_ctx_sm_count", "hl_ctx_device",
     "hl_ctx_set_astar_variant", "hl_env_upload", "hl_env_free", "hl_env_count", "hl_env_device", "hl_collision_check", "hl_path_reduce",
     "hl_rs_all_paths", "hl_rs_sample", "hl_hybrid_astar_batch", "hl_hybrid_astar_workspace_bytes", "hl_astar_phase_cycles",
-    "hl_distance_field", "hl_grid_pack", "hl_grid_footprint_check", "hl_measure_fp32_peak", "hl_ypark_paths", "hl_arc_paths", "hl_ref_path_count", "hl_ref_path_fill",
+    "hl_distance_field", "hl_distance_field_batch", "hl_grid_pack", "hl_grid_footprint_check", "hl_measure_fp32_peak", "hl_ypark_paths", "hl_arc_paths", "hl_ref_path_count", "hl_ref_path_fill",
     "hl_dubins_count", "hl_dubins_knots", "hl_dubins_fill", "hl_min_boundary_distance", "hl_corridor_hits",
 ]
 
@@ -155,6 +162,7 @@ def load_library():
         lib.hl_hybrid_astar_workspace_bytes.restype = i64
         lib.hl_astar_phase_cycles.argtypes = [vp, C.POINTER(C.c_uint64), i32, i32]
         lib.hl_distance_field.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, C.POINTER(i32), vp]
+        lib.hl_distance_field_batch.argtypes = [vp, vp, i64, C.POINTER(HlGridField), i32, i32, vp, i64, C.POINTER(i32), vp]
         lib.hl_grid_pack.argtypes = [vp, vp, i32, i32, vp, vp]
         lib.hl_grid_footprint_check.argtypes = [vp, vp, i32, i32, dbl, vp, i64, C.POINTER(dbl), vp, vp]
         lib.hl_measure_fp32_peak.argtypes = [vp, C.POINTER(dbl)]

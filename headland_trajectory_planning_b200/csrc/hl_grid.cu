@@ -14,7 +14,10 @@
 // K7 is the grid-based footprint check the reference left commented out
 // (orchard_geometry_environment.py:8,35-43,460-461) on the grid layout of
 // occupancy_grid_utils.py:70-101; parity unpinned (no reference implementation).
+#include <algorithm>
+#include <climits>
 #include <cstring>
+#include <vector>
 #include "hl_common.cuh"
 
 #ifndef DF_TILE
@@ -24,21 +27,60 @@
 
 struct DfMoves { int n; int di[8]; int dj[8]; double w[8]; };
 
-__global__ void k_df_init(const uint8_t* __restrict__ occ, int W, int H, int gi, int gj, double* __restrict__ out,
-                          int* __restrict__ list, int* __restrict__ count, int tiles_i, int tiles_j, int* __restrict__ bad) {
-    long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (idx >= (long long)W * H) return;
-    int i = (int)(idx / H), j = (int)(idx % H);
-    out[idx] = (i == gi && j == gj) ? 0.0 : INFINITY;
-    if ((i == 0 || j == 0 || i == W - 1 || j == H - 1) && !occ[idx]) atomicOr(bad, 1);   // open border: aliases reachable
-    if (i == gi && j == gj) {
-        int ti = i / DF_TILE, tj = j / DF_TILE;
-        for (int a = -1; a <= 1; ++a)
-            for (int b = -1; b <= 1; ++b) {
-                int x = ti + a, y = tj + b;
-                if (x >= 0 && y >= 0 && x < tiles_i && y < tiles_j) list[atomicAdd(count, 1)] = x * tiles_j + y;
-            }
+// One grid of a batch: a map, or the (2W-1) x (2H-1) extended grid of an open-border map (see k_df_ext_init).  Every K6
+// kernel walks a table of these; the first 32 bytes are what a relaxation CTA reads for a tile.
+struct __align__(16) DfField {
+    const uint8_t* occ;           // [w][h], non-zero = occupied
+    double* D;                    // [w][h] costs
+    int w, h;
+    int tiles_j, tile_base;       // tiles per row; first tile of this grid in the wavefront's global tile numbering
+    long long cell_base;          // first cell of this grid in its table's global cell numbering (elementwise kernels)
+    int gi, gj;                   // goal cell
+};
+
+// entry of global cell c in a table whose cell_base increase (every grid has at least one cell)
+__device__ __forceinline__ int df_field_of(const DfField* __restrict__ fs, int n, long long c) {
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (fs[mid].cell_base <= c) lo = mid; else hi = mid - 1;
     }
+    return lo;
+}
+
+// a map whose goal lies strictly inside a grid of at least 3 x 3 is relaxed in place unless a border cell is free
+__host__ __device__ inline bool df_goal_inside(const DfField& f) {
+    return f.w >= 3 && f.h >= 3 && f.gi > 0 && f.gj > 0 && f.gi < f.w - 1 && f.gj < f.h - 1;
+}
+
+// the goal's 3 x 3 tile neighbourhood of grid fi joins the first frontier.  List entries are (grid, tile of that grid).
+__device__ void df_seed(const DfField& f, int fi, int2* __restrict__ list, int* __restrict__ count) {
+    const int tiles_i = (f.w + DF_TILE - 1) / DF_TILE, ti = f.gi / DF_TILE, tj = f.gj / DF_TILE;
+    for (int a = -1; a <= 1; ++a)
+        for (int b = -1; b <= 1; ++b) {
+            const int x = ti + a, y = tj + b;
+            if (x >= 0 && y >= 0 && x < tiles_i && y < f.tiles_j) list[atomicAdd(count, 1)] = make_int2(fi, x * f.tiles_j + y);
+        }
+}
+
+// +inf everywhere and 0 at the goal of every map; open[f] = 1 when a border cell of map f is free (aliases reachable).
+// Maps with their goal inside are seeded on the table's own tiling, which is the wavefront's when no border is open.
+__global__ void k_df_init(const DfField* __restrict__ fs, int n, long long cells, int* __restrict__ open,
+                          int2* __restrict__ list, int* __restrict__ count) {
+    const long long c = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (c >= cells) return;
+    const int fi = df_field_of(fs, n, c);
+    const DfField f = fs[fi];
+    const long long idx = c - f.cell_base;
+    const int i = (int)(idx / f.h), j = (int)(idx % f.h);
+    f.D[idx] = (i == f.gi && j == f.gj) ? 0.0 : INFINITY;
+    if ((i == 0 || j == 0 || i == f.w - 1 || j == f.h - 1) && !f.occ[idx]) open[fi] = 1;
+    if (i == f.gi && j == f.gj && df_goal_inside(f)) df_seed(f, fi, list, count);
+}
+
+__global__ void k_df_seed(const DfField* __restrict__ fs, int n, int2* __restrict__ list, int* __restrict__ count) {
+    const int fi = blockIdx.x * blockDim.x + threadIdx.x;
+    if (fi < n) df_seed(fs[fi], fi, list, count);
 }
 
 // DF_CPT cells per thread of a DF_TILE x DF_TILE tile (DF_TILE^2 / DF_CPT threads), the move set a template parameter: the 8 (King) or 5
@@ -102,15 +144,18 @@ __device__ __forceinline__ bool df_less(double a, double b) { return __double_as
 #ifndef DF_ROWSKIP
 #define DF_ROWSKIP 1                    // a warp sits an iteration out when no row its cells can see changed in the previous one
 #endif
-template <bool KING>
+// ONE: the wavefront has a single grid, passed by value (`one`) instead of read from the table per tile: its fields are
+// then kernel constants, as in the single-map kernel before batching, and take no registers across the relaxation loop
+// (measured on the 4096 x 4096 King field: reading the table per tile costs 1.7 %)
+template <bool KING, bool ONE>
 __global__ void __launch_bounds__(DF_RELAX_THREADS, DF_MIN_CTAS)
-k_df_relax(const uint8_t* __restrict__ occ, int W, int H, int gi, int gj, double* __restrict__ D,
-           const int* __restrict__ list_cur, const int* __restrict__ count_cur, int* __restrict__ list_next,
-           int* __restrict__ count_next, int* __restrict__ mark_next, int* __restrict__ mark_cur, int* __restrict__ count_clear,
-           int tiles_i, int tiles_j, int* __restrict__ any_next) {
+k_df_relax(const DfField* __restrict__ fields, const DfField one, const int2* __restrict__ list_cur, const int* __restrict__ count_cur,
+           int2* __restrict__ list_next, int* __restrict__ count_next, int* __restrict__ mark_next, int* __restrict__ mark_cur,
+           int* __restrict__ count_clear, int* __restrict__ any_next) {
     // the frontier is a LIST of tiles walked by a small grid with a stride (instead of one CTA per tile of the map, 16 k
     // CTAs of which a few hundred have work).  No memset between launches: a tile clears its own mark when it is
-    // processed, and the counter the launch after next appends to is zeroed here (three counters rotate).
+    // processed, and the counter the launch after next appends to is zeroed here (three counters rotate).  The tiles of
+    // all grids of a batch share the list; marks are indexed by the global tile id (tile_base + tile).
 #if DF_PDL
     // programmatic dependent launch: this grid was scheduled while the previous relaxation launch was still running;
     // nothing that launch wrote is read before it has completed, and the NEXT launch may be scheduled from here on
@@ -130,10 +175,19 @@ k_df_relax(const uint8_t* __restrict__ occ, int W, int H, int gi, int gj, double
     const int tid = threadIdx.x;
     const int a0 = DF_ROW0(tid), b = 1 + (tid % DF_TILE);      // cell q of this thread: row DF_ROW(a0, q), column b
     for (int li = blockIdx.x; li < n_cur; li += gridDim.x) {
-        const int tile = list_cur[li];
+        const int2 entry = list_cur[li];
+        const DfField f = ONE ? one : fields[entry.x];
+        // the grid pointers come from memory, so without this they are generic: LD / ST instead of LDG / STG, occupancy
+        // without the read-only path, and every access ordered against the shared tile (measured: +10 % per launch)
+        __builtin_assume(__isGlobal(f.occ));
+        __builtin_assume(__isGlobal(f.D));
+        const uint8_t* __restrict__ occ = f.occ;
+        double* __restrict__ D = f.D;
+        const int W = f.w, H = f.h, tiles_j = f.tiles_j, tile_base = f.tile_base;
+        const int tile = entry.y;
         const int ti = tile / tiles_j, tj = tile % tiles_j;
         const int i0 = ti * DF_TILE - 1, j0 = tj * DF_TILE - 1;
-        if (tid == 0) { s_border_changed = 0; mark_cur[tile] = 0; }
+        if (tid == 0) { s_border_changed = 0; mark_cur[tile_base + tile] = 0; }
 #if DF_ROWSKIP
         if (tid < DF_TILE + 2) { s_rowchg[0][tid] = 1; s_rowchg[1][tid] = 0; }      // first iteration: every row counts as changed
         int it = 0;
@@ -143,7 +197,7 @@ k_df_relax(const uint8_t* __restrict__ occ, int W, int H, int gi, int gj, double
             const int i = i0 + x, j = j0 + y;
             const bool in = i >= 0 && j >= 0 && i < W && j < H;
             sd[x][y] = in ? D[(long long)i * H + j] : INFINITY;
-            so[x][y] = in ? occ[(long long)i * H + j] : 1;
+            so[x][y] = in ? __ldg(occ + (long long)i * H + j) : 1;
         }
         __syncthreads();
         double init[DF_CPT], cur[DF_CPT];
@@ -281,9 +335,10 @@ k_df_relax(const uint8_t* __restrict__ occ, int W, int H, int gi, int gj, double
         }
         __syncthreads();
         if (tid < 9 && tid != 4 && (s_border_changed >> tid) & 1) {
-            const int tx = ti + tid / 3 - 1, ty = tj + tid % 3 - 1;
-            if (tx >= 0 && ty >= 0 && tx < tiles_i && ty < tiles_j && atomicExch(&mark_next[tx * tiles_j + ty], 1) == 0)
-                list_next[atomicAdd(count_next, 1)] = tx * tiles_j + ty;
+            const int tx = ti + tid / 3 - 1, ty = tj + tid % 3 - 1;     // flags stay inside the tile's own grid
+            const int tiles_i = (W + DF_TILE - 1) / DF_TILE;
+            if (tx >= 0 && ty >= 0 && tx < tiles_i && ty < tiles_j && atomicExch(&mark_next[tile_base + tx * tiles_j + ty], 1) == 0)
+                list_next[atomicAdd(count_next, 1)] = make_int2(entry.x, tx * tiles_j + ty);
             *any_next = 1;
         }
         __syncthreads();                                   // the shared tile is reused by the next list entry
@@ -302,19 +357,32 @@ k_df_relax(const uint8_t* __restrict__ occ, int W, int H, int gi, int gj, double
 //   out[cell] = C(alias of the cell with the largest (P, i, j))                                   (k_df_fold)
 // oracle/distance_field.py (pinned bit-for-bit on the reference) agrees on every tested grid
 // (tests/test_grid_gpu.py::test_wrap_around_quirk_matches_reference).
-__global__ void k_df_ext_occ(const uint8_t* __restrict__ occ, int W, int H, uint8_t* __restrict__ eocc) {
-    const int EW = 2 * W - 1, EH = 2 * H - 1;
-    long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (idx >= (long long)EW * EH) return;
-    const int a = (int)(idx / EH), b = (int)(idx % EH);
+// The extended grids of a batch are packed in one workspace: entry k of `ex` (grid of map `mx[k]`) owns cells
+// ex[k].cell_base .. + EW * EH of eocc, C (= ex[k].D) and the two priority buffers.  This pass builds the extended
+// occupancy and initialises C (+inf, 0 at the goal).
+__global__ void k_df_ext_init(const DfField* __restrict__ mx, const DfField* __restrict__ ex, int n, long long cells,
+                              uint8_t* __restrict__ eocc) {
+    const long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (g >= cells) return;
+    const int k = df_field_of(ex, n, g);
+    const DfField e = ex[k];
+    const int W = mx[k].w, H = mx[k].h;
+    const long long idx = g - e.cell_base;
+    const int a = (int)(idx / e.h), b = (int)(idx % e.h);
     const int i = a - (W - 1), j = b - (H - 1);
-    eocc[idx] = occ[(long long)(i < 0 ? i + W : i) * H + (j < 0 ? j + H : j)];
+    eocc[g] = mx[k].occ[(long long)(i < 0 ? i + W : i) * H + (j < 0 ? j + H : j)];
+    e.D[idx] = (a == e.gi && b == e.gj) ? 0.0 : INFINITY;
 }
 
-__global__ void k_df_prio(const double* __restrict__ C, const double* __restrict__ Pin, double* __restrict__ Pout,
-                          int EW, int EH, DfMoves mv, int ga, int gb, int* __restrict__ changed) {
-    long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (idx >= (long long)EW * EH) return;
+__global__ void k_df_prio(const DfField* __restrict__ ex, int n, long long cells, const double* __restrict__ Pin_all,
+                          double* __restrict__ Pout_all, DfMoves mv, int* __restrict__ changed) {
+    const long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (g >= cells) return;
+    const DfField e = ex[df_field_of(ex, n, g)];
+    const double* __restrict__ C = e.D;
+    const double* __restrict__ Pin = Pin_all + e.cell_base;
+    const int EW = e.w, EH = e.h, ga = e.gi, gb = e.gj;
+    const long long idx = g - e.cell_base;
     const int a = (int)(idx / EH), b = (int)(idx % EH);
     double np_ = INFINITY;
     if (a == ga && b == gb) np_ = 0.0;
@@ -331,12 +399,20 @@ __global__ void k_df_prio(const double* __restrict__ C, const double* __restrict
         }
     }
     if (np_ != Pin[idx]) *changed = 1;
-    Pout[idx] = np_;
+    Pout_all[g] = np_;
 }
 
-__global__ void k_df_fold(const double* __restrict__ C, const double* __restrict__ P, int W, int H, double* __restrict__ out) {
-    long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (idx >= (long long)W * H) return;
+// each cell of map mx[k] takes the cost of its alias with the largest (P, i, j) on the extended grid ex[k]
+__global__ void k_df_fold(const DfField* __restrict__ mx, const DfField* __restrict__ ex, int n, long long cells,
+                          const double* __restrict__ P_all) {
+    const long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (g >= cells) return;
+    const int k = df_field_of(mx, n, g);
+    const DfField m = mx[k];
+    const double* __restrict__ C = ex[k].D;
+    const double* __restrict__ P = P_all + ex[k].cell_base;
+    const int W = m.w, H = m.h;
+    const long long idx = g - m.cell_base;
     const int ci = (int)(idx / H), cj = (int)(idx % H);
     const int EH = 2 * H - 1;
     double best_c = INFINITY, best_p = -INFINITY;
@@ -354,31 +430,31 @@ __global__ void k_df_fold(const double* __restrict__ C, const double* __restrict
             if (p > best_p || (p == best_p && (i > best_i || (i == best_i && j > best_j)))) { best_p = p; best_i = i; best_j = j; best_c = c; }
         }
     }
-    out[idx] = best_c;
+    m.D[idx] = best_c;
 }
 
-// Tiled wavefront to the fixed point on a w x h grid (cells outside count as occupied).  *open_border is set when
-// a border cell is free (only when `open_border` is given; nothing is relaxed then).
-static int df_solve(const uint8_t* d_occ, int w, int h, int gi, int gj, const DfMoves& mv, double* d_out,
-                    cudaStream_t st, int* open_border, int* sweeps_out) {
-    const int tiles_i = (w + DF_TILE - 1) / DF_TILE, tiles_j = (h + DF_TILE - 1) / DF_TILE;
-    const int n_tiles = tiles_i * tiles_j;
-    int* ws = nullptr;                       // list[2][n_tiles] | mark[2][n_tiles] | count[2] | flags[1 + DF_BATCH]
-    // The wavefront needs one launch per tile it crosses (~150 for a 4096 x 4096 map), so the launches are queued
-    // DF_BATCH at a time and the host looks at the "frontier not empty" flags once per batch (one stream
-    // synchronisation per launch before); a launch with an empty frontier list costs a few microseconds.
-    // Launches are queued DF_BATCH at a time with one host look per batch (launches behind the first empty frontier do
-    // nothing and cost ~2 us each).  The wavefront needs about one launch per tile it crosses, so the first look comes
-    // after (tiles_i + tiles_j) / 2 launches, the later ones every 32: 2 host looks for the 4096 x 4096 field (157
-    // launches) instead of 10 -- every look is a stream synchronisation, i.e. an idle GPU for as long as the host
-    // thread takes to come back.
-    enum { DF_BATCH_MAX = 128, DF_BATCH_NEXT = 32 };
-    int DF_BATCH = (tiles_i + tiles_j) / 2 < 16 ? 16 : ((tiles_i + tiles_j) / 2 > DF_BATCH_MAX ? DF_BATCH_MAX : (tiles_i + tiles_j) / 2);
-    const size_t ws_ints = 4 * (size_t)n_tiles + 4 + 1 + DF_BATCH_MAX;
-    HL_CUDA_OK(cudaMalloc(&ws, ws_ints * sizeof(int)));
-    int* list[2] = {ws, ws + n_tiles};
-    int* mark[2] = {ws + 2 * (size_t)n_tiles, ws + 3 * (size_t)n_tiles};
-    int* count = ws + 4 * (size_t)n_tiles;
+// Launches are queued DF_BATCH at a time with one host look per batch (launches behind the first empty frontier do
+// nothing and cost ~2 us each).  The wavefront needs about one launch per tile it crosses, so the first look comes
+// after (tiles_i + tiles_j) / 2 launches of the deepest grid, the later ones every 32: 2 host looks for the
+// 4096 x 4096 field (157 launches) instead of 10 -- every look is a stream synchronisation, i.e. an idle GPU for as
+// long as the host thread takes to come back.
+enum { DF_BATCH_MAX = 128, DF_BATCH_NEXT = 32 };
+
+// ints of a wavefront workspace: list[2][n_tiles] (int2) | mark[2][n_tiles] | count[4] | flags[1 + DF_BATCH_MAX]
+static size_t df_ws_ints(long long n_tiles) { return 6 * (size_t)n_tiles + 4 + 1 + DF_BATCH_MAX; }
+
+// Tiled wavefront to the fixed point of every grid of the table `rel` (device copy d_rel; cells outside a grid count as
+// occupied).  The grids' tiles share one global numbering (tile_base), so a relaxation launch walks the frontier of all
+// of them and a batch costs about the depth of its deepest grid.  The caller initialises the costs and hands over the
+// workspace `ws` zeroed, with the first frontier in list[0] / count[0].
+static int df_wavefront(const char* what, const std::vector<DfField>& rel, const DfField* d_rel, int* ws, int n_tiles,
+                        const DfMoves& mv, cudaStream_t st, int* sweeps_out) {
+    int depth = 0;                           // the largest tiles_i + tiles_j of the batch
+    for (const DfField& f : rel) depth = std::max(depth, (f.w + DF_TILE - 1) / DF_TILE + f.tiles_j);
+    int DF_BATCH = depth / 2 < 16 ? 16 : (depth / 2 > DF_BATCH_MAX ? DF_BATCH_MAX : depth / 2);
+    int2* list[2] = {(int2*)ws, (int2*)ws + n_tiles};
+    int* mark[2] = {ws + 4 * (size_t)n_tiles, ws + 5 * (size_t)n_tiles};
+    int* count = ws + 6 * (size_t)n_tiles;
     int* flags = count + 4;                  // count[0..2]: three rotating frontier counters
     int rc = 0, sweeps = 0;
     int sm = 148;
@@ -393,15 +469,13 @@ static int df_solve(const uint8_t* d_occ, int w, int h, int gi, int gj, const Df
 #endif
     const int per_sm = DF_GRID_PER_SM;
     const int grid = n_tiles < sm * per_sm ? n_tiles : sm * per_sm;
+    const bool one = rel.size() == 1;
+    auto relax = mv.n == 8 ? (one ? k_df_relax<true, true> : k_df_relax<true, false>)
+                           : (one ? k_df_relax<false, true> : k_df_relax<false, false>);
     do {
-        if (cudaMemsetAsync(ws, 0, ws_ints * sizeof(int), st) != cudaSuccess) { rc = 1; break; }
-        long long cells = (long long)w * h;
-        k_df_init<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(d_occ, w, h, gi, gj, d_out, list[0], count, tiles_i, tiles_j, flags);
         int host_flags[1 + DF_BATCH_MAX] = {0};
-        if (cudaMemcpyAsync(host_flags, flags, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) { rc = 1; break; }
-        if (open_border) { *open_border = host_flags[0]; if (host_flags[0]) break; }
         int cur = 0;                            // launch number: lists / marks alternate (cur & 1), counters rotate (cur % 3)
-        const int max_sweeps = 8 * (tiles_i + tiles_j) * DF_TILE + 64;
+        const int max_sweeps = 8 * depth * DF_TILE + 64;
         bool converged = false;
         while (!converged && sweeps < max_sweeps) {
             cudaMemsetAsync(flags + 1, 0, DF_BATCH * sizeof(int), st);
@@ -419,24 +493,13 @@ static int df_solve(const uint8_t* d_occ, int w, int h, int gi, int gj, const Df
                 attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
                 attr[0].val.programmaticStreamSerializationAllowed = 1;
                 cfg.attrs = attr; cfg.numAttrs = 1;
-                const uint8_t* a_occ = d_occ; double* a_out = d_out;
-                const int* a_lc = list[lc]; const int* a_cc = c_cur;
+                const int2* a_lc = list[lc]; const int* a_cc = c_cur;
                 int* a_fl = flags + 1 + k;
-                cudaError_t le;
-                if (mv.n == 8)
-                    le = cudaLaunchKernelEx(&cfg, k_df_relax<true>, a_occ, w, h, gi, gj, a_out, a_lc, a_cc, list[ln], c_nxt, mark[ln],
-                                            mark[lc], c_clr, tiles_i, tiles_j, a_fl);
-                else
-                    le = cudaLaunchKernelEx(&cfg, k_df_relax<false>, a_occ, w, h, gi, gj, a_out, a_lc, a_cc, list[ln], c_nxt, mark[ln],
-                                            mark[lc], c_clr, tiles_i, tiles_j, a_fl);
-                if (le != cudaSuccess) { rc = 1; break; }       // a launch that did not happen would read as "frontier empty"
+                if (cudaLaunchKernelEx(&cfg, relax, d_rel, rel[0], a_lc, a_cc, list[ln], c_nxt, mark[ln], mark[lc], c_clr, a_fl) != cudaSuccess) {
+                    rc = 1; break;                              // a launch that did not happen would read as "frontier empty"
+                }
 #else
-                if (mv.n == 8)
-                    k_df_relax<true><<<grid, DF_RELAX_THREADS, 0, st>>>(d_occ, w, h, gi, gj, d_out, list[lc], c_cur, list[ln], c_nxt,
-                                                                        mark[ln], mark[lc], c_clr, tiles_i, tiles_j, flags + 1 + k);
-                else
-                    k_df_relax<false><<<grid, DF_RELAX_THREADS, 0, st>>>(d_occ, w, h, gi, gj, d_out, list[lc], c_cur, list[ln], c_nxt,
-                                                                         mark[ln], mark[lc], c_clr, tiles_i, tiles_j, flags + 1 + k);
+                relax<<<grid, DF_RELAX_THREADS, 0, st>>>(d_rel, rel[0], list[lc], c_cur, list[ln], c_nxt, mark[ln], mark[lc], c_clr, flags + 1 + k);
                 if (cudaGetLastError() != cudaSuccess) { rc = 1; break; }
 #endif
                 ++cur;
@@ -449,12 +512,139 @@ static int df_solve(const uint8_t* d_occ, int w, int h, int gi, int gj, const Df
             }
             DF_BATCH = DF_BATCH_NEXT;
         }
-        if (rc == 0 && !converged) { hl_set_error("hl_distance_field: no convergence after %d launches", sweeps); rc = 2; }
+        if (rc == 0 && !converged) { hl_set_error("%s: no convergence after %d launches", what, sweeps); rc = 2; }
     } while (0);
-    if (rc == 1) hl_set_error("hl_distance_field: CUDA error: %s", cudaGetErrorString(cudaGetLastError()));
-    cudaFree(ws);
+    if (rc == 1) hl_set_error("%s: CUDA error: %s", what, cudaGetErrorString(cudaGetLastError()));
     if (sweeps_out) *sweeps_out += sweeps;
     return rc;
+}
+
+// move set of a_star_utils.py:8-21 (motion_type 0, King) or :24-34 (1, Pawn); false for any other motion_type
+static bool df_moves(int motion_type, DfMoves* mv) {
+    static const int king[8][2] = {{-1, 0}, {-1, 1}, {0, 1}, {1, 1}, {1, 0}, {1, -1}, {0, -1}, {-1, -1}};
+    static const int pawn[5][2] = {{-1, 0}, {0, 1}, {-1, 1}, {1, 1}, {1, 0}};
+    memset(mv, 0, sizeof(*mv));
+    if (motion_type != 0 && motion_type != 1) return false;
+    const int (*k)[2] = motion_type == 0 ? king : pawn;
+    mv->n = motion_type == 0 ? 8 : 5;
+    for (int m = 0; m < mv->n; ++m) { mv->di[m] = k[m][0]; mv->dj[m] = k[m][1]; mv->w[m] = hypot((double)k[m][0], (double)k[m][1]); }
+    return true;
+}
+
+// Distance fields of n validated maps in one wavefront.  A map whose border is occupied and whose goal lies strictly
+// inside is the whole search space and is relaxed in place; any other map takes part as its extended grid (the
+// reference's index wrap-around) and is folded into its output slice afterwards.  When every map is of the first kind
+// (the common case) the call is one allocation, the init pass that also seeds the frontier, one synchronisation to read
+// the open-border flags, and the wavefront.
+static int df_run(const char* what, const uint8_t* d_occ, const HlGridField* hf, int n, const DfMoves& mv, double* d_out,
+                  int32_t* h_sweeps, cudaStream_t st) {
+    std::vector<DfField> map(n);
+    long long cells = 0, n_tiles = 0;
+    for (int k = 0; k < n; ++k) {
+        DfField& f = map[k];
+        memset(&f, 0, sizeof(f));
+        f.occ = d_occ + hf[k].occ_offset; f.D = d_out + hf[k].out_offset;
+        f.w = hf[k].w; f.h = hf[k].h; f.gi = hf[k].gi; f.gj = hf[k].gj;
+        f.tiles_j = (f.h + DF_TILE - 1) / DF_TILE;
+        f.tile_base = (int)std::min(n_tiles, (long long)INT_MAX);
+        n_tiles += (long long)((f.w + DF_TILE - 1) / DF_TILE) * f.tiles_j;
+        f.cell_base = cells; cells += (long long)f.w * f.h;
+    }
+    const long long max_tiles = INT_MAX / 6;
+    if (n_tiles > max_tiles) { hl_set_error("%s: %lld tiles exceed the %lld of one wavefront", what, n_tiles, max_tiles); return 1; }
+    // map[n] | mx[n] | wavefront workspace for the maps' own tiling | open[n] | changed
+    char* d_tab = nullptr;
+    const size_t tab_bytes = 2 * (size_t)n * sizeof(DfField) + (df_ws_ints(n_tiles) + n + 1) * sizeof(int);
+    if (cudaMalloc(&d_tab, tab_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        hl_set_error("%s: cudaMalloc of %zu bytes for the field tables and the wavefront failed", what, tab_bytes);
+        return 1;
+    }
+    DfField* d_map = (DfField*)d_tab; DfField* d_mx = d_map + n;
+    int* ws = (int*)(d_mx + n);
+    int* d_open = ws + df_ws_ints(n_tiles);
+    int* d_changed = d_open + n;
+    char* d_ext = nullptr;                   // rel[n] | C | P0 | P1 of all extended grids | their wavefront workspace | eocc
+    int rc = 0, sweeps = 0;
+    do {
+        std::vector<int> open(n, 0);
+        if (cudaMemsetAsync(d_tab, 0, tab_bytes, st) != cudaSuccess ||
+            cudaMemcpyAsync(d_map, map.data(), n * sizeof(DfField), cudaMemcpyHostToDevice, st) != cudaSuccess) { rc = 2; break; }
+        k_df_init<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(d_map, n, cells, d_open, (int2*)ws, ws + 6 * n_tiles);
+        if (cudaMemcpyAsync(open.data(), d_open, n * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess) { rc = 2; break; }
+        std::vector<DfField> rel, ext, mx;
+        long long ecells = 0, mcells = 0;
+        for (int k = 0; k < n; ++k) {
+            const DfField& f = map[k];
+            if (df_goal_inside(f) && !open[k]) { rel.push_back(f); continue; }
+            DfField m = f;
+            m.cell_base = mcells; mcells += (long long)f.w * f.h;
+            mx.push_back(m);
+            DfField e;
+            memset(&e, 0, sizeof(e));
+            e.w = 2 * f.w - 1; e.h = 2 * f.h - 1; e.gi = f.gi + f.w - 1; e.gj = f.gj + f.h - 1;
+            e.tiles_j = (e.h + DF_TILE - 1) / DF_TILE;
+            e.cell_base = ecells; ecells += (long long)e.w * e.h;
+            ext.push_back(e);
+        }
+        const int n_ext = (int)ext.size();
+        const DfField* d_rel = d_map;        // no extended grid: the wavefront runs on the map table as seeded
+        const DfField* d_ex = nullptr;
+        if (n_ext) {
+            // the closed maps and the extended grids get a tiling of their own, a workspace for it and a new first frontier
+            n_tiles = 0;
+            rel.insert(rel.end(), ext.begin(), ext.end());
+            for (DfField& f : rel) { f.tile_base = (int)std::min(n_tiles, (long long)INT_MAX); n_tiles += (long long)((f.w + DF_TILE - 1) / DF_TILE) * f.tiles_j; }
+            if (n_tiles > max_tiles) { hl_set_error("%s: %lld tiles exceed the %lld of one wavefront", what, n_tiles, max_tiles); rc = 1; break; }
+            const size_t ext_bytes = (size_t)n * sizeof(DfField) + 3 * sizeof(double) * (size_t)ecells + df_ws_ints(n_tiles) * sizeof(int) + (size_t)ecells;
+            if (cudaMalloc(&d_ext, ext_bytes) != cudaSuccess) {
+                cudaGetLastError();
+                hl_set_error("%s: the extended grids of %d maps with a free border cell or a border goal need %zu bytes, "
+                             "cudaMalloc failed", what, n_ext, ext_bytes);
+                rc = 1; break;
+            }
+            DfField* d_rel2 = (DfField*)d_ext;
+            double* C = (double*)(d_rel2 + n);
+            ws = (int*)(C + 3 * ecells);
+            uint8_t* eocc = (uint8_t*)(ws + df_ws_ints(n_tiles));
+            const int n_rel = (int)rel.size();
+            for (int k = n_rel - n_ext; k < n_rel; ++k) { rel[k].occ = eocc + rel[k].cell_base; rel[k].D = C + rel[k].cell_base; }
+            d_rel = d_rel2;
+            d_ex = d_rel2 + (n_rel - n_ext);
+            if (cudaMemsetAsync(ws, 0, df_ws_ints(n_tiles) * sizeof(int), st) != cudaSuccess ||
+                cudaMemcpyAsync(d_rel2, rel.data(), n_rel * sizeof(DfField), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+                cudaMemcpyAsync(d_mx, mx.data(), n_ext * sizeof(DfField), cudaMemcpyHostToDevice, st) != cudaSuccess) { rc = 2; break; }
+            k_df_ext_init<<<(unsigned)((ecells + 255) / 256), 256, 0, st>>>(d_mx, d_ex, n_ext, ecells, eocc);
+            k_df_seed<<<(unsigned)((n_rel + 127) / 128), 128, 0, st>>>(d_rel2, n_rel, (int2*)ws, ws + 6 * n_tiles);
+        }
+        if (df_wavefront(what, n_ext ? rel : map, d_rel, ws, (int)n_tiles, mv, st, &sweeps)) { rc = 1; break; }
+        if (!n_ext) break;
+        // closing-order priorities of all extended grids to their fixed point, then the fold into the maps
+        double* C = (double*)((DfField*)d_ext + n);
+        double* P0 = C + ecells; double* P1 = C + 2 * ecells;
+        if (cudaMemcpyAsync(P0, C, sizeof(double) * (size_t)ecells, cudaMemcpyDeviceToDevice, st) != cudaSuccess) { rc = 2; break; }
+        const unsigned eblocks = (unsigned)((ecells + 255) / 256);
+        int max_it = 0;
+        for (const DfField& e : ext) max_it = std::max(max_it, 4 * (e.w + e.h));
+        int it = 0, h_changed = 1;
+        while (h_changed && it < max_it) {
+            cudaMemsetAsync(d_changed, 0, sizeof(int), st);
+            k_df_prio<<<eblocks, 256, 0, st>>>(d_ex, n_ext, ecells, P0, P1, mv, d_changed);
+            if (cudaMemcpyAsync(&h_changed, d_changed, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) { rc = 2; break; }
+            double* t = P0; P0 = P1; P1 = t;
+            ++it; ++sweeps;
+        }
+        if (rc) break;
+        if (h_changed) { hl_set_error("%s: closing-order priorities did not converge", what); rc = 1; break; }
+        k_df_fold<<<(unsigned)((mcells + 255) / 256), 256, 0, st>>>(d_mx, d_ex, n_ext, mcells, P0);
+        if (cudaStreamSynchronize(st) != cudaSuccess) { rc = 2; break; }
+    } while (0);
+    if (rc == 2) hl_set_error("%s: CUDA error: %s", what, cudaGetErrorString(cudaGetLastError()));
+    cudaFree(d_tab);
+    if (d_ext) cudaFree(d_ext);
+    if (h_sweeps) *h_sweeps = sweeps;
+    return rc ? 1 : 0;
 }
 
 extern "C" int hl_distance_field(hl_ctx* ctx, const uint8_t* d_occ, int32_t w, int32_t h, int32_t gi,
@@ -463,64 +653,55 @@ extern "C" int hl_distance_field(hl_ctx* ctx, const uint8_t* d_occ, int32_t w, i
     if (!ctx || !d_occ || !d_out || w < 1 || h < 1) { hl_set_error("hl_distance_field: bad arguments"); return 1; }
     if (gi < 0 || gj < 0 || gi >= w || gj >= h) { hl_set_error("hl_distance_field: goal (%d,%d) outside the %dx%d grid", gi, gj, w, h); return 1; }
     if (hl_enter(ctx, nullptr, d_out, "hl_distance_field")) return 1;
-    cudaStream_t st = (cudaStream_t)stream;
     DfMoves mv;
-    memset(&mv, 0, sizeof(mv));
-    if (motion_type == 0) {                 // a_star_utils.py:8-21
-        const int k[8][2] = {{-1, 0}, {-1, 1}, {0, 1}, {1, 1}, {1, 0}, {1, -1}, {0, -1}, {-1, -1}};
-        mv.n = 8;
-        for (int m = 0; m < 8; ++m) { mv.di[m] = k[m][0]; mv.dj[m] = k[m][1]; mv.w[m] = hypot((double)k[m][0], (double)k[m][1]); }
-    } else if (motion_type == 1) {          // :24-34
-        const int k[5][2] = {{-1, 0}, {0, 1}, {-1, 1}, {1, 1}, {1, 0}};
-        mv.n = 5;
-        for (int m = 0; m < 5; ++m) { mv.di[m] = k[m][0]; mv.dj[m] = k[m][1]; mv.w[m] = hypot((double)k[m][0], (double)k[m][1]); }
-    } else { hl_set_error("hl_distance_field: motion_type must be 0 (King) or 1 (Pawn)"); return 1; }
-    int sweeps = 0;
-    // fast path: every border cell occupied and the goal strictly inside -> no alias is reachable, the map itself is
-    // the whole search space
-    if (w >= 3 && h >= 3 && gi > 0 && gj > 0 && gi < w - 1 && gj < h - 1) {
-        int open_border = 0;
-        const int rc = df_solve(d_occ, w, h, gi, gj, mv, d_out, st, &open_border, &sweeps);
-        if (rc) return 1;
-        if (!open_border) { if (h_sweeps) *h_sweeps = sweeps; return 0; }
+    if (!df_moves(motion_type, &mv)) { hl_set_error("hl_distance_field: motion_type must be 0 (King) or 1 (Pawn)"); return 1; }
+    const HlGridField f = {0, 0, w, h, gi, gj};
+    return df_run("hl_distance_field", d_occ, &f, 1, mv, d_out, h_sweeps, (cudaStream_t)stream);
+}
+
+extern "C" int hl_distance_field_batch(hl_ctx* ctx, const uint8_t* d_occ, int64_t occ_bytes, const HlGridField* h_fields,
+                                       int32_t n_fields, int32_t motion_type, double* d_out, int64_t out_elems,
+                                       int32_t* h_sweeps, void* stream) {
+    const char* what = "hl_distance_field_batch";
+    if (h_sweeps) *h_sweeps = 0;
+    if (!ctx || n_fields < 0 || occ_bytes < 0 || out_elems < 0 || (n_fields > 0 && (!h_fields || !d_occ || !d_out))) {
+        hl_set_error("%s: bad arguments", what); return 1;
     }
-    // general path: the extended grid of the reference's index wrap-around
-    const int EW = 2 * w - 1, EH = 2 * h - 1;
-    const long long ecells = (long long)EW * EH;
-    uint8_t* eocc = nullptr;
-    double* buf = nullptr;                   // C | P0 | P1
-    int* changed = nullptr;
-    if (cudaMalloc(&eocc, (size_t)ecells) != cudaSuccess || cudaMalloc(&buf, 3 * sizeof(double) * (size_t)ecells) != cudaSuccess ||
-        cudaMalloc(&changed, sizeof(int)) != cudaSuccess) {
-        if (eocc) cudaFree(eocc);
-        if (buf) cudaFree(buf);
-        hl_set_error("hl_distance_field: cudaMalloc failed for the %dx%d extended grid", EW, EH);
-        return 1;
-    }
-    double* C = buf; double* P0 = buf + ecells; double* P1 = buf + 2 * ecells;
-    const unsigned eblocks = (unsigned)((ecells + 255) / 256);
-    int rc = 0;
-    do {
-        k_df_ext_occ<<<eblocks, 256, 0, st>>>(d_occ, w, h, eocc);
-        if (df_solve(eocc, EW, EH, gi + w - 1, gj + h - 1, mv, C, st, nullptr, &sweeps)) { rc = 1; break; }
-        if (cudaMemcpyAsync(P0, C, sizeof(double) * (size_t)ecells, cudaMemcpyDeviceToDevice, st) != cudaSuccess) { rc = 2; break; }
-        int it = 0, h_changed = 1;
-        while (h_changed && it < 4 * (EW + EH)) {
-            cudaMemsetAsync(changed, 0, sizeof(int), st);
-            k_df_prio<<<eblocks, 256, 0, st>>>(C, P0, P1, EW, EH, mv, gi + w - 1, gj + h - 1, changed);
-            if (cudaMemcpyAsync(&h_changed, changed, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) { rc = 2; break; }
-            double* t = P0; P0 = P1; P1 = t;
-            ++it; ++sweeps;
+    DfMoves mv;
+    if (!df_moves(motion_type, &mv)) { hl_set_error("%s: motion_type must be 0 (King) or 1 (Pawn), got %d", what, motion_type); return 1; }
+    for (int k = 0; k < n_fields; ++k) {
+        const HlGridField& f = h_fields[k];
+        if (f.w < 1 || f.h < 1) { hl_set_error("%s: field %d: a %dx%d grid (w and h must be at least 1)", what, k, f.w, f.h); return 1; }
+        if (f.gi < 0 || f.gj < 0 || f.gi >= f.w || f.gj >= f.h) {
+            hl_set_error("%s: field %d: goal (%d,%d) outside the %dx%d grid", what, k, f.gi, f.gj, f.w, f.h); return 1;
         }
-        if (rc) break;
-        if (h_changed) { hl_set_error("hl_distance_field: closing-order priorities did not converge"); rc = 1; break; }
-        k_df_fold<<<(unsigned)(((long long)w * h + 255) / 256), 256, 0, st>>>(C, P0, w, h, d_out);
-        if (cudaStreamSynchronize(st) != cudaSuccess) { rc = 2; break; }
-    } while (0);
-    if (rc == 2) hl_set_error("hl_distance_field: CUDA error: %s", cudaGetErrorString(cudaGetLastError()));
-    cudaFree(eocc); cudaFree(buf); cudaFree(changed);
-    if (h_sweeps) *h_sweeps = sweeps;
-    return rc ? 1 : 0;
+        const long long cells = (long long)f.w * f.h;
+        if (f.occ_offset < 0 || f.occ_offset > occ_bytes - cells) {
+            hl_set_error("%s: field %d: grid bytes [%lld, %lld) outside the %lld bytes of d_occ", what, k,
+                         (long long)f.occ_offset, (long long)f.occ_offset + cells, (long long)occ_bytes); return 1;
+        }
+        if (f.out_offset < 0 || f.out_offset > out_elems - cells) {
+            hl_set_error("%s: field %d: output slice [%lld, %lld) outside the %lld elements of d_out", what, k,
+                         (long long)f.out_offset, (long long)f.out_offset + cells, (long long)out_elems); return 1;
+        }
+    }
+    // sorted by start, two slices overlap only if some pair of neighbours does
+    std::vector<int> order(n_fields);
+    for (int k = 0; k < n_fields; ++k) order[k] = k;
+    std::sort(order.begin(), order.end(), [&](int a, int b) {
+        return h_fields[a].out_offset != h_fields[b].out_offset ? h_fields[a].out_offset < h_fields[b].out_offset : a < b;
+    });
+    for (int k = 1; k < n_fields; ++k) {
+        const HlGridField& a = h_fields[order[k - 1]];
+        if (h_fields[order[k]].out_offset < a.out_offset + (long long)a.w * a.h) {
+            hl_set_error("%s: fields %d and %d: output slices overlap", what, std::min(order[k - 1], order[k]),
+                         std::max(order[k - 1], order[k]));
+            return 1;
+        }
+    }
+    if (n_fields == 0) return 0;
+    if (hl_enter(ctx, nullptr, d_occ, what) || hl_enter(ctx, nullptr, d_out, what)) return 1;
+    return df_run(what, d_occ, h_fields, n_fields, mv, d_out, h_sweeps, (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------------- K7

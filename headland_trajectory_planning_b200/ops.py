@@ -384,6 +384,49 @@ def distance_field(occ, goal, motion_type="King"):
     return out, sweeps.value
 
 
+def distance_field_batch(occs, goals, motion_type="King"):
+    """Distance fields of many (grid, goal) pairs in one wavefront (hl_distance_field_batch).  ``occs``: one [W,H]
+    bool/uint8 grid shared by every goal (uploaded once), or a sequence of B grids, one per goal, of any shapes (host
+    arrays or CUDA tensors).  ``goals``: B pairs (i, j).  Returns (list of B float64 CUDA tensors [W_b, H_b], views of
+    one pooled buffer, relaxation launches); each field equals ``distance_field`` of its grid and goal bit for bit."""
+    torch = _torch()
+    lib = _lib.load_library()
+    if motion_type not in ("King", "Pawn"):
+        raise _lib.HeadlandError(f"unknown motion type {motion_type!r} (King or Pawn)")
+    goals = [(int(g[0]), int(g[1])) for g in goals]
+    shared = (torch.is_tensor(occs) or isinstance(occs, np.ndarray)) and occs.ndim == 2
+    grids = [g if torch.is_tensor(g) else np.asarray(g) for g in ([occs] if shared else occs)]
+    if not shared and len(grids) != len(goals):
+        raise _lib.HeadlandError(f"distance_field_batch: {len(grids)} grids for {len(goals)} goals")
+    dev = _device(None, *grids)
+    if not goals:
+        return [], 0
+    if any(g.ndim != 2 for g in grids):
+        raise _lib.HeadlandError("distance_field_batch: every grid must be 2-D [W, H]")
+    shapes = [tuple(int(v) for v in g.shape) for g in grids]
+    if any(torch.is_tensor(g) for g in grids):
+        occ = torch.cat([(g if torch.is_tensor(g) else torch.from_numpy(g.astype(np.uint8))).to(dev, torch.uint8).reshape(-1)
+                         for g in grids])
+    else:                                  # host grids: one upload
+        occ = torch.from_numpy(np.concatenate([g.astype(np.uint8).reshape(-1) for g in grids])).to(dev)
+    occ_base = np.concatenate([[0], np.cumsum([w * h for w, h in shapes])])
+    fields = (_lib.HlGridField * len(goals))()
+    out_base = 0
+    for k, (gi, gj) in enumerate(goals):
+        s = 0 if shared else k
+        w, h = shapes[s]
+        fields[k] = _lib.HlGridField(int(occ_base[s]), out_base, w, h, gi, gj)
+        out_base += w * h
+    out = torch.empty(out_base, dtype=torch.float64, device=dev)
+    sweeps = C.c_int32(0)
+    mt = {"King": 0, "Pawn": 1}[motion_type]
+    _lib.check(lib.hl_distance_field_batch(_lib.get_ctx(), _lib.ptr(occ), occ.numel(), fields, len(goals), mt,
+                                           _lib.ptr(out), out.numel(), C.byref(sweeps), _lib.stream_ptr()),
+               "hl_distance_field_batch")
+    views = [out[f.out_offset:f.out_offset + f.w * f.h].view(f.w, f.h) for f in fields]
+    return views, sweeps.value
+
+
 def grid_pack(occ):
     torch = _torch()
     lib = _lib.load_library()

@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define HL_ABI_VERSION 3
+#define HL_ABI_VERSION 4
 
 /* ---- limits (compile-time capacities of the kernels) ---------------------- */
 #define HL_MAX_PRIMS        16   /* motion primitives per expansion (King: 14, Pawn: 8) */
@@ -340,6 +340,25 @@ int hl_astar_phase_cycles(hl_ctx* ctx, uint64_t* h_out, int32_t n, int32_t reset
 int hl_distance_field(hl_ctx* ctx, const uint8_t* d_occ, int32_t w, int32_t h, int32_t gi,
                       int32_t gj, int32_t motion_type, double* d_out, int32_t* h_sweeps,
                       void* stream);
+
+/* One field of a batch: a [w][h] occupancy grid (row-major, non-zero = occupied, like hl_distance_field) and a goal cell. */
+typedef struct {
+    int64_t occ_offset;   /* first byte of this field's grid in d_occ; several fields may share one grid        */
+    int64_t out_offset;   /* first element of this field's [w][h] float64 result in d_out; slices must not overlap */
+    int32_t w, h;
+    int32_t gi, gj;       /* goal cell, 0 <= gi < w, 0 <= gj < h                                                  */
+} HlGridField;
+
+/* Distance fields of n_fields (grid, goal) pairs in one tiled wavefront: every relaxation launch serves all fields, so
+ * a batch costs about the depth of its deepest field rather than the sum.  Each output slice is bit-identical to what
+ * hl_distance_field returns for that grid and goal (wrap-around included).  motion_type is shared by the batch.
+ *   h_fields  [n_fields] HOST array; checked before anything launches (bounds against occ_bytes / out_elems,
+ *             overlapping output slices, goals, sizes): a failure names the field index in hl_last_error
+ *   h_sweeps  optional host int: relaxation launches used (shared by the batch).  n_fields == 0 launches nothing.
+ *   Synchronises the stream.                                                                              */
+int hl_distance_field_batch(hl_ctx* ctx, const uint8_t* d_occ, int64_t occ_bytes,
+                            const HlGridField* h_fields, int32_t n_fields, int32_t motion_type,
+                            double* d_out, int64_t out_elems, int32_t* h_sweeps, void* stream);
 
 /* ---- K7 occupancy-grid footprint ---------------------------------------------
  * The grid-based footprint check the reference intended
