@@ -739,12 +739,29 @@ __device__ __forceinline__ bool row_any(const uint32_t* __restrict__ bits, long 
     return false;
 }
 
+// Cells [lo, hi] (clamped to [0, n-1]) whose closed interval [fl(i*res), fl((i+1)*res)] meets [vmin, vmax].
+// fl(i*res) is monotone in i, so the candidates are contiguous: start from the floor() estimate (clamped to [-1, n]
+// before the conversion, so huge coordinates cannot overflow the int) and step it by the edge comparisons themselves.
+// floor(v/res) alone is off by one where fl(i*res)/res rounds below i (an edge touching from below) or an edge one
+// ulp below fl(i*res) still divides to i (an overlap of one ulp).
+__device__ __forceinline__ void cell_range(double vmin, double vmax, double res, int n, int& lo, int& hi) {
+    lo = (int)fmin(fmax(floor(vmin / res), -1.0), (double)n);
+    while (lo > -1 && (double)lo * res >= vmin) --lo;           // cell lo-1 ends at fl(lo*res) >= vmin
+    while (lo < n && (double)(lo + 1) * res < vmin) ++lo;       // cell lo ends before vmin
+    hi = (int)fmin(fmax(floor(vmax / res), -1.0), (double)n);
+    while (hi < n && (double)(hi + 1) * res <= vmax) ++hi;      // cell hi+1 starts at or before vmax
+    while (hi > -1 && (double)hi * res > vmax) --hi;            // cell hi starts after vmax
+    lo = max(lo, 0); hi = min(hi, n - 1);
+}
+
 __global__ void __launch_bounds__(256)
 k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, double res, const double* __restrict__ poses,
                  long long n, double x0, double x1, double y0, double y1, uint8_t* __restrict__ out) {
     long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (idx >= n) return;
     const double px = poses[3 * idx], py = poses[3 * idx + 1], yaw = poses[3 * idx + 2];
+    // a pose that is not finite can never be certified free (fmin / fmax below would drop NaN corners)
+    if (!isfinite(px) || !isfinite(py) || !isfinite(yaw)) { out[idx] = 1; return; }
     const double c = cos(yaw), s = sin(yaw);
     const double lx[4] = {x0, x0, x1, x1}, ly[4] = {y1, y0, y0, y1};
     double cx[4], cy[4];
@@ -755,10 +772,9 @@ k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, double res, co
         cy[k] = xadd(xadd(xmul(s, lx[k]), xmul(c, ly[k])), py);
         xmin = fmin(xmin, cx[k]); xmax = fmax(xmax, cx[k]);
     }
-    int ia = (int)floor(xmin / res), ib = (int)floor(xmax / res);
-    // a rectangle that touches x = i*res from above also meets cell i-1 (closed sets)
-    if ((double)ia * res == xmin) ia -= 1;
-    ia = max(ia, 0); ib = min(ib, W - 1);
+    // closed sets: a rectangle touching a cell edge meets the cells on both sides of it
+    int ia, ib;
+    cell_range(xmin, xmax, res, W, ia, ib);
     bool hit = false;
     for (int i = ia; i <= ib && !hit; ++i) {
         const double a = (double)i * res, b = (double)(i + 1) * res;
@@ -780,9 +796,8 @@ k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, double res, co
             }
         }
         if (ymin > ymax) continue;
-        int ja = (int)floor(ymin / res), jb = (int)floor(ymax / res);
-        if ((double)ja * res == ymin) ja -= 1;
-        ja = max(ja, 0); jb = min(jb, H - 1);
+        int ja, jb;
+        cell_range(ymin, ymax, res, H, ja, jb);
         if (ja <= jb) hit = row_any(bits, (long long)i * H, ja, jb);
     }
     out[idx] = hit ? 1 : 0;

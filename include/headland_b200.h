@@ -364,8 +364,11 @@ int hl_distance_field_batch(hl_ctx* ctx, const uint8_t* d_occ, int64_t occ_bytes
  * The grid-based footprint check the reference intended
  * (orchard_geometry_environment.py:8,35-43,460-461; grid layout of
  * occupancy_grid_utils.py:70-101: cell (i,j) covers [i*res,(i+1)*res) x [j*res,(j+1)*res)).
- * No reference implementation exists (parity unpinned): a pose is infeasible iff any
- * occupied cell's square meets the closed body rectangle.
+ * No reference implementation exists (parity unpinned): a pose is infeasible iff the
+ * closed body rectangle (float64 corners (c*lx - s*ly) + x, (s*lx + c*ly) + y, no fused
+ * multiply-add) meets the closed square [fl(i*res), fl((i+1)*res)] x [fl(j*res), fl((j+1)*res)]
+ * of some occupied cell (i, j); touching counts.  A pose with a NaN or infinite x, y or yaw
+ * is infeasible (out = 1) whatever the grid holds.
  *   d_occ_bits  bit-packed grid, bit (i*H + j); res metres per cell                   */
 int hl_grid_pack(hl_ctx* ctx, const uint8_t* d_occ, int32_t w, int32_t h, uint32_t* d_bits,
                  void* stream);

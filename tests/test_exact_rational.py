@@ -16,157 +16,13 @@ This file checks them against brute-force set-theoretic definitions evaluated in
 Poses are placed so that a footprint corner (or edge) sits within 1e-9 .. 1e-6 m of an obstacle edge, a field edge
 or a lane-capsule boundary -- where a wrong strict/non-strict comparison or a missed case would show."""
 import math
-from fractions import Fraction as Fr
 
 import numpy as np
-import pytest
 
 import hl_helpers as H
+from exact_geom import EXT, F, _edge_samples, _poses_near, x_rect_hits_convex, x_rect_in_polygon, x_rect_in_union
 from oracle import geometry as geo
 from oracle import planner as OP
-
-
-# ------------------------------------------------------------------ exact primitives
-def F(a):
-    return [(Fr(float(x)), Fr(float(y))) for x, y in np.asarray(a, dtype=np.float64).reshape(-1, 2)]
-
-
-def orient(a, b, c):
-    return (b[0] - a[0]) * (c[1] - a[1]) - (b[1] - a[1]) * (c[0] - a[0])
-
-
-def on_segment(a, b, p):
-    return orient(a, b, p) == 0 and min(a[0], b[0]) <= p[0] <= max(a[0], b[0]) and min(a[1], b[1]) <= p[1] <= max(a[1], b[1])
-
-
-def in_closed_polygon(p, poly):
-    """winding number by exact crossing count; boundary counts as inside"""
-    inside = False
-    n = len(poly)
-    for i in range(n):
-        a, b = poly[i], poly[(i + 1) % n]
-        if on_segment(a, b, p):
-            return True
-        if (a[1] > p[1]) != (b[1] > p[1]):
-            xint = a[0] + (b[0] - a[0]) * (p[1] - a[1]) / (b[1] - a[1])
-            if p[0] < xint:
-                inside = not inside
-    return inside
-
-
-def in_open_convex(p, poly_ccw):
-    return all(orient(poly_ccw[i], poly_ccw[(i + 1) % len(poly_ccw)], p) > 0 for i in range(len(poly_ccw)))
-
-
-def in_closed_convex(p, poly_ccw):
-    return all(orient(poly_ccw[i], poly_ccw[(i + 1) % len(poly_ccw)], p) >= 0 for i in range(len(poly_ccw)))
-
-
-def segs_meet(a, b, c, d):
-    """closed segments share a point"""
-    o1, o2, o3, o4 = orient(a, b, c), orient(a, b, d), orient(c, d, a), orient(c, d, b)
-    if ((o1 > 0) != (o2 > 0)) and o1 != 0 and o2 != 0 and ((o3 > 0) != (o4 > 0)) and o3 != 0 and o4 != 0:
-        return True
-    return on_segment(a, b, c) or on_segment(a, b, d) or on_segment(c, d, a) or on_segment(c, d, b)
-
-
-def seg_params_with(a, b, c, d):
-    """parameters t in [0, 1] on a->b where the closed segment c->d touches it (finite list)"""
-    r = (b[0] - a[0], b[1] - a[1])
-    s = (d[0] - c[0], d[1] - c[1])
-    den = r[0] * s[1] - r[1] * s[0]
-    qp = (c[0] - a[0], c[1] - a[1])
-    out = []
-    if den != 0:
-        t = (qp[0] * s[1] - qp[1] * s[0]) / den
-        u = (qp[0] * r[1] - qp[1] * r[0]) / den
-        if 0 <= t <= 1 and 0 <= u <= 1:
-            out.append(t)
-    else:                                             # parallel: endpoints of c-d that lie on a-b
-        rr = r[0] * r[0] + r[1] * r[1]
-        for p in (c, d):
-            if orient(a, b, p) == 0:
-                t = ((p[0] - a[0]) * r[0] + (p[1] - a[1]) * r[1]) / rr
-                if 0 <= t <= 1:
-                    out.append(t)
-    return out
-
-
-def pieces_midpoints(a, b, edges):
-    ts = {Fr(0), Fr(1)}
-    for c, d in edges:
-        ts.update(seg_params_with(a, b, c, d))
-    ts = sorted(ts)
-    return [(a[0] + (b[0] - a[0]) * (t0 + t1) / 2, a[1] + (b[1] - a[1]) * (t0 + t1) / 2) for t0, t1 in zip(ts[:-1], ts[1:])]
-
-
-def ring_edges(poly):
-    return [(poly[i], poly[(i + 1) % len(poly)]) for i in range(len(poly))]
-
-
-# ------------------------------------------------------------------ exact definitions
-def x_rect_hits_convex(rect, poly_ccw):
-    if any(in_closed_convex(p, poly_ccw) for p in rect) or any(in_closed_convex(p, rect) for p in poly_ccw):
-        return True
-    return any(segs_meet(a, b, c, d) for a, b in ring_edges(rect) for c, d in ring_edges(poly_ccw))
-
-
-def x_rect_in_polygon(rect, poly):
-    pe = ring_edges(poly)
-    for a, b in ring_edges(rect):
-        if not all(in_closed_polygon(m, poly) for m in pieces_midpoints(a, b, pe)):
-            return False
-    return True                                       # simple polygon: boundary inside => region inside
-
-
-def x_rect_in_union(rect, polys_ccw):
-    all_edges = [e for P in polys_ccw for e in ring_edges(P)]
-    for a, b in ring_edges(rect):                     # the rectangle's boundary is covered
-        for m in pieces_midpoints(a, b, all_edges):
-            if not any(in_closed_convex(m, P) for P in polys_ccw):
-                return False
-    redges = ring_edges(rect)                         # no hole of the union inside the rectangle
-    for i, P in enumerate(polys_ccw):
-        others = [e for j, Q in enumerate(polys_ccw) if j != i for e in ring_edges(Q)]
-        for a, b in ring_edges(P):
-            for m in pieces_midpoints(a, b, redges + others):
-                if in_open_convex(m, rect) and not any(in_open_convex(m, Q) or
-                                                       any(on_segment(c, d, m) for c, d in ring_edges(Q))
-                                                       for j, Q in enumerate(polys_ccw) if j != i):
-                    return False
-    return True
-
-
-# ------------------------------------------------------------------ pose generators
-EXT = geo.body_extent(0.55, 3.0, 1.48)
-DELTAS = (1e-9, -1e-9, 1e-7, -1e-7, 1e-6, -1e-6, 3e-4, -3e-4)
-
-
-def _poses_near(rng, boundary_pts, normals, n):
-    """poses whose k-th footprint corner lies at boundary point + delta * normal"""
-    lx = np.array([EXT[0], EXT[0], EXT[1], EXT[1]])
-    ly = np.array([EXT[3], EXT[2], EXT[2], EXT[3]])
-    out = []
-    for _ in range(n):
-        j = rng.integers(len(boundary_pts))
-        k = rng.integers(4)
-        yaw = rng.uniform(-math.pi, math.pi)
-        d = DELTAS[rng.integers(len(DELTAS))]
-        q = boundary_pts[j] + d * normals[j]
-        c, s = math.cos(yaw), math.sin(yaw)
-        out.append([q[0] - (c * lx[k] - s * ly[k]), q[1] - (s * lx[k] + c * ly[k]), yaw])
-    return np.array(out)
-
-
-def _edge_samples(rng, poly, per_edge=3):
-    pts, nrm = [], []
-    for a, b in zip(poly, np.roll(poly, -1, axis=0)):
-        e = b - a
-        n = np.array([e[1], -e[0]]) / np.hypot(*e)
-        for t in list(rng.uniform(0.02, 0.98, per_edge)) + [0.0]:
-            pts.append(a + t * e)
-            nrm.append(n)
-    return np.array(pts), np.array(nrm)
 
 
 def test_rect_vs_convex_obstacles_exact():
