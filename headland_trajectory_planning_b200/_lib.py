@@ -12,7 +12,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_NAME = "libheadland_b200.so"
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 HL_MAX_PRIMS = 16
 HL_CAPSULE_VERTS = 66
 HL_RS_CANDIDATES = 46
@@ -69,6 +69,13 @@ class HlGridField(C.Structure):
     ]
 
 
+class HlRasterGrid(C.Structure):
+    _fields_ = [
+        ("out_offset", C.c_int64), ("env_id", C.c_int32),
+        ("w", C.c_int32), ("h", C.c_int32), ("i0", C.c_int32), ("j0", C.c_int32),
+    ]
+
+
 SCENARIO_DTYPE = np.dtype([("env_id", "<i4"), ("reserved", "<i4"),
                            ("start", "<f8", (3,)), ("goal", "<f8", (3,))])
 RESULT_DTYPE = np.dtype([("status", "<i4"), ("counter", "<i4"), ("n_expanded", "<i4"),
@@ -85,7 +92,8 @@ EXPORTS = [
     "hl_last_error", "hl_abi_version", "hl_ctx_create", "hl_ctx_destroy", "hl_ctx_sm_count", "hl_ctx_device",
     "hl_ctx_set_astar_variant", "hl_env_upload", "hl_env_free", "hl_env_count", "hl_env_device", "hl_collision_check", "hl_path_reduce",
     "hl_rs_all_paths", "hl_rs_sample", "hl_hybrid_astar_batch", "hl_hybrid_astar_workspace_bytes", "hl_astar_phase_cycles",
-    "hl_distance_field", "hl_distance_field_batch", "hl_grid_pack", "hl_grid_footprint_check", "hl_measure_fp32_peak", "hl_ypark_paths", "hl_arc_paths", "hl_ref_path_count", "hl_ref_path_fill",
+    "hl_distance_field", "hl_distance_field_batch", "hl_grid_pack", "hl_grid_footprint_check", "hl_grid_footprint_check_at", "hl_env_rasterize",
+    "hl_measure_fp32_peak", "hl_ypark_paths", "hl_arc_paths", "hl_ref_path_count", "hl_ref_path_fill",
     "hl_dubins_count", "hl_dubins_knots", "hl_dubins_fill", "hl_min_boundary_distance", "hl_corridor_hits",
 ]
 
@@ -165,6 +173,8 @@ def load_library():
         lib.hl_distance_field_batch.argtypes = [vp, vp, i64, C.POINTER(HlGridField), i32, i32, vp, i64, C.POINTER(i32), vp]
         lib.hl_grid_pack.argtypes = [vp, vp, i32, i32, vp, vp]
         lib.hl_grid_footprint_check.argtypes = [vp, vp, i32, i32, dbl, vp, i64, C.POINTER(dbl), vp, vp]
+        lib.hl_grid_footprint_check_at.argtypes = [vp, vp, i32, i32, i32, i32, dbl, vp, i64, C.POINTER(dbl), vp, vp]
+        lib.hl_env_rasterize.argtypes = [vp, vp, C.POINTER(HlRasterGrid), i32, dbl, u32, vp, i64, vp, vp]
         lib.hl_measure_fp32_peak.argtypes = [vp, C.POINTER(dbl)]
         lib.hl_ypark_paths.argtypes = [vp, vp, vp, i64, dbl, vp, vp]
         lib.hl_arc_paths.argtypes = [vp, vp, vp, i64, dbl, vp, vp]

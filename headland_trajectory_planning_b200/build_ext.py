@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libheadland_b200.so")
-SOURCES = ["hl_ctx.cu", "hl_collision.cu", "hl_rs.cu", "hl_astar.cu", "hl_grid.cu", "hl_bench.cu", "hl_ypark.cu", "hl_refpath.cu", "hl_dubins.cu"]
+SOURCES = ["hl_ctx.cu", "hl_collision.cu", "hl_rs.cu", "hl_astar.cu", "hl_grid.cu", "hl_raster.cu", "hl_bench.cu", "hl_ypark.cu", "hl_refpath.cu", "hl_dubins.cu"]
 
 
 def nvcc_path():

@@ -739,23 +739,26 @@ __device__ __forceinline__ bool row_any(const uint32_t* __restrict__ bits, long 
     return false;
 }
 
-// Cells [lo, hi] (clamped to [0, n-1]) whose closed interval [fl(i*res), fl((i+1)*res)] meets [vmin, vmax].
-// fl(i*res) is monotone in i, so the candidates are contiguous: start from the floor() estimate (clamped to [-1, n]
-// before the conversion, so huge coordinates cannot overflow the int) and step it by the edge comparisons themselves.
-// floor(v/res) alone is off by one where fl(i*res)/res rounds below i (an edge touching from below) or an edge one
-// ulp below fl(i*res) still divides to i (an overlap of one ulp).
-__device__ __forceinline__ void cell_range(double vmin, double vmax, double res, int n, int& lo, int& hi) {
-    lo = (int)fmin(fmax(floor(vmin / res), -1.0), (double)n);
-    while (lo > -1 && (double)lo * res >= vmin) --lo;           // cell lo-1 ends at fl(lo*res) >= vmin
-    while (lo < n && (double)(lo + 1) * res < vmin) ++lo;       // cell lo ends before vmin
-    hi = (int)fmin(fmax(floor(vmax / res), -1.0), (double)n);
-    while (hi < n && (double)(hi + 1) * res <= vmax) ++hi;      // cell hi+1 starts at or before vmax
-    while (hi > -1 && (double)hi * res > vmax) --hi;            // cell hi starts after vmax
-    lo = max(lo, 0); hi = min(hi, n - 1);
+// Cells [lo, hi] (global indices, clamped to [g0, g0+n-1]) whose closed interval [fl(i*res), fl((i+1)*res)] meets
+// [vmin, vmax].  fl(i*res) is monotone in i, so the candidates are contiguous: start from the floor() estimate (clamped
+// to [g0-1, g0+n] before the conversion, so huge coordinates cannot overflow) and step it by the edge comparisons
+// themselves.  floor(v/res) alone is off by one where fl(i*res)/res rounds below i (an edge touching from below) or an
+// edge one ulp below fl(i*res) still divides to i (an overlap of one ulp).  Indices are 64-bit here so that g0 - 1 and
+// g0 + n + 1 stay representable; (double)i + 1.0 is exactly (double)(i + 1) for every int32 i.
+__device__ __forceinline__ void cell_range(double vmin, double vmax, double res, int g0, int n, long long& lo, long long& hi) {
+    const long long a = (long long)g0 - 1, b = (long long)g0 + n;
+    lo = (long long)fmin(fmax(floor(vmin / res), (double)a), (double)b);
+    while (lo > a && (double)lo * res >= vmin) --lo;             // cell lo-1 ends at fl(lo*res) >= vmin
+    while (lo < b && ((double)lo + 1.0) * res < vmin) ++lo;      // cell lo ends before vmin
+    hi = (long long)fmin(fmax(floor(vmax / res), (double)a), (double)b);
+    while (hi < b && ((double)hi + 1.0) * res <= vmax) ++hi;     // cell hi+1 starts at or before vmax
+    while (hi > a && (double)hi * res > vmax) --hi;              // cell hi starts after vmax
+    lo = max(lo, (long long)g0); hi = min(hi, b - 1);
 }
 
+// (gi0, gj0): global index of the grid's cell (0, 0); bits are indexed by the local cell (i - gi0) * H + (j - gj0)
 __global__ void __launch_bounds__(256)
-k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, double res, const double* __restrict__ poses,
+k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, int gi0, int gj0, double res, const double* __restrict__ poses,
                  long long n, double x0, double x1, double y0, double y1, uint8_t* __restrict__ out) {
     long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (idx >= n) return;
@@ -773,11 +776,11 @@ k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, double res, co
         xmin = fmin(xmin, cx[k]); xmax = fmax(xmax, cx[k]);
     }
     // closed sets: a rectangle touching a cell edge meets the cells on both sides of it
-    int ia, ib;
-    cell_range(xmin, xmax, res, W, ia, ib);
+    long long ia, ib;
+    cell_range(xmin, xmax, res, gi0, W, ia, ib);
     bool hit = false;
-    for (int i = ia; i <= ib && !hit; ++i) {
-        const double a = (double)i * res, b = (double)(i + 1) * res;
+    for (long long i = ia; i <= ib && !hit; ++i) {
+        const double a = (double)i * res, b = ((double)i + 1.0) * res;
         double ymin = INFINITY, ymax = -INFINITY;
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -796,11 +799,22 @@ k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, double res, co
             }
         }
         if (ymin > ymax) continue;
-        int ja, jb;
-        cell_range(ymin, ymax, res, H, ja, jb);
-        if (ja <= jb) hit = row_any(bits, (long long)i * H, ja, jb);
+        long long ja, jb;
+        cell_range(ymin, ymax, res, gj0, H, ja, jb);
+        if (ja <= jb) hit = row_any(bits, (i - gi0) * H, (int)(ja - gj0), (int)(jb - gj0));
     }
     out[idx] = hit ? 1 : 0;
+}
+
+static int grid_footprint_launch(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_t w, int32_t h, int32_t i0, int32_t j0,
+                                 double res, const double* d_poses, int64_t n, const double body_ext[4], uint8_t* d_out,
+                                 void* stream, const char* what) {
+    if (n == 0) return 0;
+    if (hl_enter(ctx, nullptr, d_out, what)) return 1;
+    k_grid_footprint<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        d_occ_bits, w, h, i0, j0, res, d_poses, (long long)n, body_ext[0], body_ext[1], body_ext[2], body_ext[3], d_out);
+    HL_CUDA_OK(cudaGetLastError());
+    return 0;
 }
 
 extern "C" int hl_grid_footprint_check(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_t w, int32_t h,
@@ -809,10 +823,22 @@ extern "C" int hl_grid_footprint_check(hl_ctx* ctx, const uint32_t* d_occ_bits, 
     if (!ctx || !d_occ_bits || !d_poses || !d_out || !body_ext || n < 0 || w <= 0 || h <= 0 || !(res > 0)) {
         hl_set_error("hl_grid_footprint_check: bad arguments"); return 1;
     }
-    if (n == 0) return 0;
-    if (hl_enter(ctx, nullptr, d_out, "hl_grid_footprint_check")) return 1;
-    k_grid_footprint<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        d_occ_bits, w, h, res, d_poses, (long long)n, body_ext[0], body_ext[1], body_ext[2], body_ext[3], d_out);
-    HL_CUDA_OK(cudaGetLastError());
-    return 0;
+    return grid_footprint_launch(ctx, d_occ_bits, w, h, 0, 0, res, d_poses, n, body_ext, d_out, stream, "hl_grid_footprint_check");
+}
+
+extern "C" int hl_grid_footprint_check_at(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_t w, int32_t h, int32_t i0,
+                                          int32_t j0, double res, const double* d_poses, int64_t n,
+                                          const double body_ext[4], uint8_t* d_out, void* stream) {
+    const char* what = "hl_grid_footprint_check_at";
+    if (!ctx || !d_occ_bits || !d_poses || !d_out || !body_ext || n < 0 || w <= 0 || h <= 0 || !(res > 0) || !isfinite(res)) {
+        hl_set_error("%s: bad arguments", what); return 1;
+    }
+    if ((long long)i0 + w > INT_MAX || (long long)j0 + h > INT_MAX) {
+        hl_set_error("%s: a %dx%d grid at (%d, %d) overflows the int32 cell index", what, w, h, i0, j0); return 1;
+    }
+    if (!isfinite((double)i0 * res) || !isfinite((double)(i0 + w) * res) || !isfinite((double)j0 * res) ||
+        !isfinite((double)(j0 + h) * res)) {
+        hl_set_error("%s: the grid's cell edges are not finite at res = %g", what, res); return 1;
+    }
+    return grid_footprint_launch(ctx, d_occ_bits, w, h, i0, j0, res, d_poses, n, body_ext, d_out, stream, what);
 }

@@ -1,5 +1,6 @@
 """Thin Python wrappers over the C ABI (device tensors in, device tensors out)."""
 import ctypes as C
+import math
 
 import numpy as np
 
@@ -440,7 +441,21 @@ def grid_pack(occ):
     return bits
 
 
-def grid_footprint_check(bits, shape, res, poses, body_ext):
+def _int32(v, what):
+    """``v`` as a Python int that fits an int32 ABI slot; ctypes would wrap a larger value silently, so the C side's
+    range checks would see a different number."""
+    v = int(v)
+    if not -2**31 <= v < 2**31:
+        raise _lib.HeadlandError(f"{what} = {v} does not fit int32")
+    return v
+
+
+def grid_footprint_check(bits, shape, res, poses, body_ext, origin=(0, 0)):
+    """K7: 1 where the body rectangle at a pose meets an occupied cell of the bit-packed grid (``grid_pack``).  The
+    grid's cell (0, 0) has the global index ``origin`` = (i0, j0): cell (i, j) covers [fl((i0+i)*res),
+    fl((i0+i+1)*res)] x [fl((j0+j)*res), fl((j0+j+1)*res)], as ``rasterize`` lays its grids out."""
+    w, h = _int32(shape[0], "grid_footprint_check: w"), _int32(shape[1], "grid_footprint_check: h")
+    i0, j0 = _int32(origin[0], "grid_footprint_check: origin i0"), _int32(origin[1], "grid_footprint_check: origin j0")
     torch = _torch()
     lib = _lib.load_library()
     dev = _device()
@@ -452,10 +467,72 @@ def grid_footprint_check(bits, shape, res, poses, body_ext):
     if n == 0:
         return out
     ext = (C.c_double * 4)(*[float(v) for v in body_ext])
-    _lib.check(lib.hl_grid_footprint_check(_lib.get_ctx(), _lib.ptr(bits), int(shape[0]), int(shape[1]), float(res),
-                                           _lib.ptr(poses), n, ext, _lib.ptr(out), _lib.stream_ptr()),
-               "hl_grid_footprint_check")
+    _lib.check(lib.hl_grid_footprint_check_at(_lib.get_ctx(), _lib.ptr(bits), w, h, i0, j0, float(res), _lib.ptr(poses), n, ext, _lib.ptr(out),
+                                              _lib.stream_ptr()), "hl_grid_footprint_check_at")
     return out
+
+
+def _cell_range(vmin, vmax, res):
+    """Cells lo..hi whose closed interval [fl(i*res), fl((i+1)*res)] meets [vmin, vmax] (K7's cell_range rule, not
+    clamped to a grid): the floor() estimate stepped by the float64 edge comparisons themselves."""
+    lo = int(math.floor(vmin / res))
+    while float(lo) * res >= vmin:
+        lo -= 1
+    while (float(lo) + 1.0) * res < vmin:
+        lo += 1
+    hi = int(math.floor(vmax / res))
+    while (float(hi) + 1.0) * res <= vmax:
+        hi += 1
+    while float(hi) * res > vmax:
+        hi -= 1
+    return lo, hi
+
+
+def raster_window(field_ring, res, margin):
+    """(i0, j0, w, h) of the cells whose closed intervals meet the float64 bounding box of ``field_ring`` grown by
+    ``margin`` metres on every side (computed on the host)."""
+    ring = np.asarray(field_ring, dtype=np.float64).reshape(-1, 2)
+    if len(ring) == 0:
+        raise _lib.HeadlandError("raster_window: the field ring has no vertices")
+    res, margin = float(res), float(margin)
+    if not (math.isfinite(res) and res > 0) or not (math.isfinite(margin) and margin >= 0):
+        raise _lib.HeadlandError(f"raster_window: res must be finite and positive and margin finite and >= 0 "
+                                 f"(res={res}, margin={margin})")
+    i0, i1 = _cell_range(float(ring[:, 0].min()) - margin, float(ring[:, 0].max()) + margin, res)
+    j0, j1 = _cell_range(float(ring[:, 1].min()) - margin, float(ring[:, 1].max()) + margin, res)
+    return i0, j0, i1 - i0 + 1, j1 - j0 + 1
+
+
+def rasterize(envs, grids, res, flags=CHECK_OBSTACLES | CHECK_BOUNDARY, count_exact=False):
+    """K12 (``hl_env_rasterize``): occupancy grids of environments of ``envs``, all in one launch.  ``grids`` is a
+    sequence of (env_id, i0, j0, w, h); cell (i, j) of a grid is the closed square [fl((i0+i)*res), fl((i0+i+1)*res)]
+    x [fl((j0+j)*res), fl((j0+j+1)*res)], occupied (1) when it meets an obstacle quad (CHECK_OBSTACLES) or is not
+    contained in the field polygon (CHECK_BOUNDARY).  Returns a list of uint8 CUDA tensors [w, h], views of one pooled
+    buffer, in ``distance_field``'s layout; with ``count_exact`` also the int64 CUDA counter of cells the float64
+    predicates decided."""
+    grids = [tuple(g) for g in grids]
+    if any(len(g) != 5 for g in grids):
+        raise _lib.HeadlandError("rasterize: every grid is (env_id, i0, j0, w, h)")
+    names = ("env_id", "i0", "j0", "w", "h")
+    grids = [tuple(_int32(v, f"rasterize: grid {k}: {nm}") for v, nm in zip(g, names)) for k, g in enumerate(grids)]
+    if not 0 <= int(flags) < 2**32:
+        raise _lib.HeadlandError(f"rasterize: flags = {int(flags)} does not fit uint32")
+    torch = _torch()
+    lib = _lib.load_library()
+    dev = _device(envs)
+    table = (_lib.HlRasterGrid * max(len(grids), 1))()
+    base = 0
+    for k, (env_id, i0, j0, w, h) in enumerate(grids):
+        if w < 1 or h < 1:
+            raise _lib.HeadlandError(f"rasterize: grid {k}: a {w}x{h} grid (w and h must be at least 1)")
+        table[k] = _lib.HlRasterGrid(base, env_id, w, h, i0, j0)
+        base += w * h
+    out = torch.empty(max(base, 1), dtype=torch.uint8, device=dev)
+    n_exact = torch.zeros(1, dtype=torch.int64, device=dev)
+    _lib.check(lib.hl_env_rasterize(envs.ctx, envs.handle, table, len(grids), float(res), int(flags), _lib.ptr(out), base,
+                                    _lib.ptr(n_exact) if count_exact else None, _lib.stream_ptr()), "hl_env_rasterize")
+    views = [out[table[k].out_offset:table[k].out_offset + w * h].view(w, h) for k, (_, _, _, w, h) in enumerate(grids)]
+    return (views, n_exact) if count_exact else views
 
 
 PHASE_NAMES = ["pop", "rs_candidates", "rs_select", "rs_plan", "rs_sample", "arrival", "rollout", "filter", "exact",

@@ -7,7 +7,7 @@ import math
 import numpy as np
 
 from . import ops
-from .env_batch import EnvBatch, make_record
+from .env_batch import EnvBatch, EnvRecord, make_record
 from .geometry_host import flat_line_buffer, square_point_buffer, Poly
 
 
@@ -120,6 +120,18 @@ class OrchardGeometryEnvironment(object):
         d = ops.min_boundary_distance(self._env_batch(car_model), path[:, :3], np.array([0, len(path)], dtype=np.int64),
                                       with_aux=with_aux)
         return float(d[0].item())
+
+    # ---- occupancy grid (the grid path the reference left commented out, :8,35-43,460-461) -> GPU
+    def occupancy_grid(self, res, margin=2.0, flags=ops.CHECK_OBSTACLES | ops.CHECK_BOUNDARY):
+        """(uint8 CUDA tensor [w, h], (i0, j0)): K12 raster of the obstacle / tree-row quads and the field polygon on
+        the cells that meet the field ring's bounding box grown by ``margin``; cell (i, j) is the closed square
+        [fl((i0+i)*res), fl((i0+i+1)*res)] x [fl((j0+j)*res), fl((j0+j+1)*res)], 1 = occupied.  Pass (i0, j0) as the
+        ``origin`` of ``ops.grid_footprint_check``.  Needs no car model."""
+        if "raster" not in self._uploads:
+            self._uploads["raster"] = EnvBatch([EnvRecord(self.obstacle_quads(), self.field_ring(), (0.0, 0.0, 0.0, 0.0))])
+        i0, j0, w, h = ops.raster_window(self.field_ring(), res, margin)
+        grid = ops.rasterize(self._uploads["raster"], [(0, i0, j0, w, h)], res, flags)[0]
+        return grid, (i0, j0)
 
     # ---- host-side topology helpers used by the orchestration (:49-64, 93-127, 199-248)
     def check_side_of_a_point(self, point):

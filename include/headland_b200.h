@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define HL_ABI_VERSION 4
+#define HL_ABI_VERSION 5
 
 /* ---- limits (compile-time capacities of the kernels) ---------------------- */
 #define HL_MAX_PRIMS        16   /* motion primitives per expansion (King: 14, Pawn: 8) */
@@ -375,6 +375,46 @@ int hl_grid_pack(hl_ctx* ctx, const uint8_t* d_occ, int32_t w, int32_t h, uint32
 int hl_grid_footprint_check(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_t w, int32_t h,
                             double res, const double* d_poses, int64_t n,
                             const double body_ext[4], uint8_t* d_out, void* stream);
+/* The same check on a grid whose cell (0, 0) has the global index (i0, j0): cell (i, j) is the closed square
+ * [fl((i0+i)*res), fl((i0+i+1)*res)] x [fl((j0+j)*res), fl((j0+j+1)*res)], so a grid may cover negative coordinates
+ * (hl_env_rasterize's windows).  hl_grid_footprint_check is this call with i0 = j0 = 0.  Rejects w or h below 1,
+ * i0 + w or j0 + h beyond int32, res not finite or not positive, and grid edges that are not finite.             */
+int hl_grid_footprint_check_at(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_t w, int32_t h, int32_t i0, int32_t j0,
+                               double res, const double* d_poses, int64_t n, const double body_ext[4],
+                               uint8_t* d_out, void* stream);
+
+/* ---- K12 occupancy grids from environment geometry ------------------------------------------------
+ * Rasterises the obstacle / tree-row quads and the field polygon of an environment batch into [w][h] uint8 grids
+ * (byte i*h + j, 1 = occupied, 0 = free: hl_distance_field's layout; hl_grid_pack makes K7's bits), many grids of
+ * many environments in one launch.  No reference implementation exists (the reference's grid path is commented
+ * out, orchard_geometry_environment.py:8,35-43,460-461): the grids are defined by the closed-set rule below.
+ *
+ * Cell rule.  Let S be the closed square of cell (i, j) of a grid, with edges the float64 products
+ * fl((i0+i)*res), fl((i0+i+1)*res), fl((j0+j)*res), fl((j0+j+1)*res) (exactly K7's edges).
+ *   - HL_CHECK_OBSTACLES: occupied iff S meets some closed obstacle or tree-row quad;
+ *   - HL_CHECK_BOUNDARY:  occupied iff S is not contained in the closed field polygon (GEOS contains: touching the
+ *                         ring from inside is still contained; an environment without field vertices is all occupied);
+ *   - both flags: occupied if either test fires.
+ * Both tests are K1's float64 predicates applied to the identity pose (x, y, cos, sin) = (0, 0, 1, 0) with the
+ * cell's edges as the rectangle: under that pose the corners and pose-frame coordinates reproduce the edges bit
+ * for bit, so every byte is the boolean hl_collision_check's float64 path gives for that rectangle.  A float32
+ * filter with K1's band decides the cells clear of the band; the rest go to those predicates (d_n_exact counts them).
+ *   h_grids    [n_grids] HOST array; checked before anything launches (a failure names the grid index): env_id
+ *              outside the batch, w or h below 1, i0 + w or j0 + h beyond int32, grid edges that are not finite,
+ *              output slices outside out_elems or overlapping.  n_grids == 0 launches nothing.
+ *   res        metres per cell, finite and positive
+ *   flags      HL_CHECK_OBSTACLES and / or HL_CHECK_BOUNDARY, nothing else
+ *   d_n_exact  optional device counter (int64) of cells decided by the float64 predicates, or NULL           */
+typedef struct {
+    int64_t out_offset;   /* first byte of this grid's [w][h] uint8 slice in d_out; slices must not overlap */
+    int32_t env_id;       /* environment of the batch                                                      */
+    int32_t w, h;         /* cells                                                                        */
+    int32_t i0, j0;       /* global index of cell (0, 0)                                                  */
+} HlRasterGrid;
+
+int hl_env_rasterize(hl_ctx* ctx, const hl_env_batch* envs, const HlRasterGrid* h_grids, int32_t n_grids,
+                     double res, uint32_t flags, uint8_t* d_out, int64_t out_elems,
+                     unsigned long long* d_n_exact, void* stream);
 
 /* ---- micro-benchmarks used for roofline denominators ------------------------- */
 /* Measured FP32 FMA peak of this device in TFLOP/s (dependent-chain-free FFMA loop). */
