@@ -24,9 +24,6 @@
 #ifndef AW_MIN_CTAS
 #define AW_MIN_CTAS 1
 #endif
-#ifndef AW_LOCKSTEP
-#define AW_LOCKSTEP 1      // 0 free-running, 1 two alignment barriers per expansion, 2 one, 3 one every other expansion
-#endif
 #ifndef AW_MAX_PLANS
 #define AW_MAX_PLANS 6
 #endif
@@ -185,8 +182,6 @@ k_hybrid_astar_w(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
     EnvSmem E;
     E.n_obs = E.n_field = E.n_seg = E.all_rect = 0; E.eps = 0.f; E.reach = 0.f; E.obs = E.field = E.seg = nullptr;
     const EnvDesc* Dp = eb.desc;
-    int iter = 0;
-    (void)iter;
 
     while (true) {
         // ---- refill: a warp without a scenario takes the next one from the global queue
@@ -214,16 +209,7 @@ k_hybrid_astar_w(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
             else if (lane == 0) S.state = ST_SEARCH;
             __syncwarp();
         }
-#if AW_LOCKSTEP == 3
-        {   // alignment every other expansion only
-            if ((iter++ & 1) == 0) { if (__syncthreads_and(S.state == ST_DONE)) break; }
-            else if (S.state == ST_DONE) { /* keep pace: wait at the next aligned iteration */ }
-        }
-#elif AW_LOCKSTEP
         if (__syncthreads_and(S.state == ST_DONE)) break;                   // alignment point 1
-#else
-        if (S.state == ST_DONE) break;
-#endif
         const bool live = (S.state == ST_SEARCH);
         const EnvDesc& D = *Dp;
         if (live) {
@@ -379,9 +365,7 @@ k_hybrid_astar_w(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
             __syncwarp();
             TICK(PH_ARRIVE);
         }
-#if AW_LOCKSTEP == 1
         __syncthreads();                                                    // alignment point 2
-#endif
         if (live && S.status < 0) {
             // ---- primitive expansion (:558-596)
             const int n = S.nsteps, np1 = n + 1;
@@ -808,8 +792,7 @@ extern "C" int hl_hybrid_astar_batch(hl_ctx* ctx, const hl_env_batch* envs, cons
     // the rest; the second launch searches the listed ones, which then all start at once instead of waiting in the
     // work queue behind trivial scenarios (the sweep's tail is the start time of its longest searches).  Results are
     // identical: the second launch redoes a listed scenario from its first pop.
-    static const bool two_phase_on = getenv("HL_ASTAR_SINGLE_PHASE") == nullptr;
-    if (spec && two_phase_on && (long long)n_scen > 2LL * grid * slots) {
+    if (spec && (long long)n_scen > 2LL * grid * slots) {
         if ((size_t)n_scen > ctx->astar_defer_cap) {
             if (ctx->astar_defer) cudaFree(ctx->astar_defer);
             ctx->astar_defer = nullptr; ctx->astar_defer_cap = 0;

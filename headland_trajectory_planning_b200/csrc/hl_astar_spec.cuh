@@ -17,21 +17,18 @@
 #pragma once
 #include "hl_astar_common.cuh"
 
-#ifndef AQ_EXPANDERS
 #define AQ_EXPANDERS 2                 // expander warps per scenario: warp 0 + a helper that shares the rollout / filter / heuristic
-#endif
 #ifndef AQ_SLOTS
-#define AQ_SLOTS (AQ_EXPANDERS > 1 ? 5 : 6)   // scenarios per CTA: 5 x 3 warps (128 registers) or 6 x 2 warps (168)
+#define AQ_SLOTS 5                     // scenarios per CTA (5 x 3 warps at 128 registers)
 #endif
 #define AQ_MAX_PLANS 6
-#ifndef AQ_SHOOTERS
-#define AQ_SHOOTERS 1                  // shooter warps per scenario (shots of different pops are independent;
-                                       // 2-3 shooters measured slower: the expander is the critical path)
-#endif
-#define AQ_WARPS_PER_SLOT (AQ_EXPANDERS + AQ_SHOOTERS)
+// one shooter warp per scenario (shots of different pops are independent, but 2-3 shooters measured slower: the
+// expander is the critical path)
+#define AQ_WARPS_PER_SLOT (AQ_EXPANDERS + 1)
 #ifndef AQ_HEAP_SM
-#define AQ_HEAP_SM 1023                // open-list entries kept in shared memory (top 10 levels of the heap); 0 = all in the workspace
+#define AQ_HEAP_SM 1023                // open-list entries kept in shared memory (top 10 levels of the heap)
 #endif
+static_assert(AQ_HEAP_SM > 0, "the search keeps the top of its open list in shared memory");
 #ifndef AQ_GUIDE_CAP
 #define AQ_GUIDE_CAP 192               // guide polyline points staged in shared memory (longer polylines are read from HBM / L2)
 #endif
@@ -88,8 +85,9 @@ struct AqSmem {                          // one per scenario slot, shared by its
     // expander state
     int n_nodes, heap_n, counter, n_closed, ew_status, ew_arrival2;
     int cur; double cx, cy, cyaw, cg; int cprim; int nsteps;
-    // shooters (AQ_SHOOTERS warps; shooter k takes pops k, k + AQ_SHOOTERS, ...)
-    AqShot sh[AQ_SHOOTERS];
+    // the shooter warp's scratch: an array of one, read through `win` (always 0) where the result is assembled.
+    // Folding that index away changes the kernel's generated code, so it is left to a change measured on its own.
+    AqShot sh[1];
     // expander scratch
     double tx[HL_MAX_PRIMS][AS_ROLL], ty[HL_MAX_PRIMS][AS_ROLL], pyaw[HL_MAX_PRIMS][AS_ROLL];
     unsigned char pamb[HL_MAX_PRIMS][AS_ROLL];
@@ -110,57 +108,25 @@ struct AqSmem {                          // one per scenario slot, shared by its
     double gyaw[AQ_GUIDE_CAP], gs[AQ_GUIDE_CAP];     // ... its headings and arc lengths
     double pds[HL_MAX_PRIMS][AS_ROLL];               // step lengths of the rolled-out primitives (g-cost)
     int guide_staged, need_seg;
-#if AQ_HEAP_SM > 0
     double hp_prio[AQ_HEAP_SM];                     // top of the open-list heap (HeapRef)
     int hp_slot[AQ_HEAP_SM];
-#endif
 };
 static_assert(sizeof(AqSmem) * AQ_SLOTS <= 227 * 1024, "per-CTA shared memory exceeds 227 KB");
 
 // Alignment of the AQ_SLOTS warps of one role (named barrier `id`, all threads of those warps) with an AND
 // reduction: keeps the role's warps inside the same code region (instruction cache) and tells them when
-// every one of them is finished.
-#ifndef AQ_WARP_MAP
-#define AQ_WARP_MAP 0                  // 1: same-role warps share a scheduler (measured: see DESIGN.md)
-#endif
-#ifndef AQ_ALIGN
-#define AQ_ALIGN 1                     // 0: no role alignment (each warp leaves when its own queue is drained)
-#endif
+// every one of them is finished.  Every iteration of either role passes it (measured, DESIGN.md section 5: without it
+// the kernel is 2x slower, at every second iteration only 25.7 instead of 21.2 ms per sweep).
 __device__ __forceinline__ bool role_barrier_all(int id, int nthreads, bool pred) {
-#if !AQ_ALIGN
-    return pred;
-#endif
     int r;
     asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.s32 p, %1, 0;\n\tbarrier.red.and.pred q, %2, %3, p;\n\tselp.s32 %0, 1, 0, q;\n\t}"
                  : "=r"(r) : "r"((int)pred), "r"(id), "r"(nthreads) : "memory");
     return r != 0;
 }
 
-#ifndef AQ_COARSE
-#define AQ_COARSE 1                    // shooter: probe all words coarsely before the per-word passes
-#endif
-#ifndef AQ_EVERY_E
-#define AQ_EVERY_E 1                   // expanders align every AQ_EVERY_E-th iteration
-#endif
-#ifndef AQ_EVERY_S
-#define AQ_EVERY_S 1                   // shooters align every AQ_EVERY_S-th iteration
-#endif
-#ifndef AQ_MID
-#define AQ_MID 0                       // extra alignment points inside an iteration (0 none, 1 one per role, 2 two for the expander)
-#endif
-__device__ __forceinline__ void role_sync(int id, int nthreads) {
-#if AQ_ALIGN
-    asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(nthreads) : "memory");
-#endif
-}
-
 // the warps of one scenario's expander team (named barrier 3 + slot)
 __device__ __forceinline__ void team_sync(int slot) {
-#if AQ_EXPANDERS > 1
     asm volatile("bar.sync %0, %1;" :: "r"(3 + slot), "r"(AQ_TEAM) : "memory");
-#else
-    __syncwarp();
-#endif
 }
 
 __device__ __forceinline__ int warp_read(volatile int* p, int lane) {
@@ -170,19 +136,11 @@ __device__ __forceinline__ int warp_read(volatile int* p, int lane) {
 }
 
 __device__ __noinline__ int aq_heap_pop(AqSmem& S, const AsWs& w, int& n) {
-#if AQ_HEAP_SM > 0
     const HeapRef<AQ_HEAP_SM> H{w, S.hp_prio, S.hp_slot};
-#else
-    const HeapRef<0> H{w, nullptr, nullptr};
-#endif
     return heap_popitem_t<AQ_HEAP_SM>(H, n);
 }
 __device__ __noinline__ void aq_heap_set(AqSmem& S, const AsWs& w, int& n, int slot, double prio) {
-#if AQ_HEAP_SM > 0
     const HeapRef<AQ_HEAP_SM> H{w, S.hp_prio, S.hp_slot};
-#else
-    const HeapRef<0> H{w, nullptr, nullptr};
-#endif
     heap_set_t<AQ_HEAP_SM>(H, n, slot, prio);
 }
 
@@ -191,11 +149,7 @@ __device__ __noinline__ void aq_heap_set(AqSmem& S, const AsWs& w, int& n, int s
 // priority), the ancestors below it move down one level in parallel and the new entry takes the freed position --
 // the arrangement the sequential swaps produce, in one step instead of up to 13 dependent ones.
 __device__ __forceinline__ void aq_heap_push_warp(AqSmem& S, const AsWs& w, int slot, double prio, int lane) {
-#if AQ_HEAP_SM > 0
     const HeapRef<AQ_HEAP_SM> H{w, S.hp_prio, S.hp_slot};
-#else
-    const HeapRef<0> H{w, nullptr, nullptr};
-#endif
     const int i = S.heap_n;
     const int depth = 31 - __clz(i + 1);                 // the root is the depth-th ancestor
     const bool mine = lane >= 1 && lane <= depth;
@@ -315,8 +269,7 @@ __device__ __forceinline__ void finalize_spec(AqSmem& S, const AsWs& W, const As
     const AsWritten w = write_outputs(W, P, O, S.status, n_closed, end, S.arrival, S.start_key, S.goal_key, &T.plan_tmp,
                                       0, lane);
     if (lane == 0) {
-        unsigned long long checks = S.e_checks, exact = S.e_exact, ref = 0;
-        for (int k = 0; k < AQ_SHOOTERS; ++k) { checks += S.sh[k].s_checks; exact += S.sh[k].s_exact; ref += S.sh[k].s_ref; }
+        unsigned long long checks = S.e_checks + S.sh[0].s_checks, exact = S.e_exact + S.sh[0].s_exact, ref = S.sh[0].s_ref;
         // algorithmic count: shots of pops <= the final one (the shooter stops there) + the expansions of the
         // pops BEFORE a successful shot (the expander may have run ahead; that work is not the reference's)
         const bool shot_won = (S.arrival == 1) || (w.status == HL_STATUS_RS_ASSERT);
@@ -336,30 +289,23 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                  size_t ws_stride, unsigned int* work_counter, AsOut O) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#if AQ_WARP_MAP == 1 && AQ_SLOTS == 5 && AQ_WARPS_PER_SLOT == 3
-    // warps of the same role on the same scheduler (warp w issues on sub-partition w % 4): sub-partition 0 holds four
-    // shooters, 1 four lead expanders, 2 four helpers, 3 the three warps of slot 4
-    const int slot = (wid & 3) == 3 ? 4 : wid >> 2;
-    const int wrole = (wid & 3) == 3 ? (wid == 3 ? 2 : (wid == 7 ? 0 : 1)) : ((wid & 3) == 0 ? 2 : (wid & 3) - 1);
-#else
     const int slot = wid / AQ_WARPS_PER_SLOT;
-    const int wrole = wid % AQ_WARPS_PER_SLOT;          // 0 .. AQ_EXPANDERS-1 = expander team, then the shooters
-#endif
+    const int wrole = wid % AQ_WARPS_PER_SLOT;          // 0 .. AQ_EXPANDERS-1 = expander team, then the shooter
     const int ew = wrole;                               // index inside the expander team
-    const int role = wrole < AQ_EXPANDERS ? 0 : wrole - AQ_EXPANDERS + 1;   // 0 = expander, 1.. = shooters
+    const bool shooter = wrole >= AQ_EXPANDERS;
     const int tl = ew * 32 + lane;                      // lane inside the expander team
     AqSmem& S = reinterpret_cast<AqSmem*>(smem_raw)[slot];
     const AsWs W = as_carve(ws_base + ((size_t)blockIdx.x * AQ_SLOTS + slot) * ws_stride, P.cap_nodes, P.hash_size,
                             P.max_nodes);
     const int hmask = P.hash_size - 1;
     const unsigned FLAGS = HL_CHECK_OBSTACLES | HL_CHECK_BOUNDARY | HL_CHECK_LANE;
-    if (role == 0 && ew == 0) {
+    if (ew == 0) {
 #pragma unroll 1
         for (int i = lane; i < P.hash_size; i += 32) W.hkey[i] = KEY_EMPTY;
         if (lane == 0) {
             S.x_expanding = 0; S.x_finished = 0; S.need_seg = 0;
             S.state = ST_IDLE; S.epoch = 0; S.popped = 0; S.ew_done = 0; S.shot_best = AQ_NO_HIT;
-            for (int k = 0; k < AQ_SHOOTERS; ++k) S.sh[k].done_epoch = 0;
+            S.sh[0].done_epoch = 0;
         }
     }
     __syncthreads();
@@ -367,10 +313,9 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
     EnvSmem E;
     E.n_obs = E.n_field = E.n_seg = E.all_rect = 0; E.eps = 0.f; E.reach = 0.f; E.obs = E.field = E.seg = nullptr;
 
-    if (role >= 1) {
+    if (shooter) {
         // =========================================== SHOOTER ===========================================
-        const int shooter = role - 1;
-        AqShot& T = S.sh[shooter];
+        AqShot& T = S.sh[0];
         int my_epoch = 0;
         int i = 0;
         bool active = false;            // a scenario is attached and its shots are not finished
@@ -379,10 +324,8 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
         EnvSmem Ers = E;
         const float inv_maxc = (float)(1.0 / P.maxc);
         const double stepn = xmul(P.res, P.maxc);
-        unsigned s_iter = 0;
         while (true) {
-            if ((s_iter++ % AQ_EVERY_S) == 0 &&
-                role_barrier_all(1, AQ_SLOTS * AQ_SHOOTERS * 32, finished)) break;   // alignment point of the shooters
+            if (role_barrier_all(1, AQ_SLOTS * 32, finished)) break;   // alignment point of the shooters
             bool shooting = false, success = false;
             int m = 0;
             double q0[3] = {0.0, 0.0, 0.0}, cq = 1.0, sq = 0.0;
@@ -412,7 +355,7 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                     Ers.eps = E.eps + 6e-5f;
                     if (lane == 0) { T.s_checks = 0; T.s_exact = 0; T.s_ref = 0; T.rs_assert = 0; }
                     __syncwarp();
-                    i = shooter;                     // pops shooter, shooter + AQ_SHOOTERS, ...
+                    i = 0;
                     active = true;
                 } else if (st == ST_DONE) { finished = true; break; }
                 else { __nanosleep(200); break; }
@@ -491,10 +434,6 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                 shooting = true;
             }
             } while (0);
-#if AQ_MID >= 1
-            role_sync(1, AQ_SLOTS * AQ_SHOOTERS * 32);                  // shooters enter the sampling code together
-            if (shooting) STICK(PH_OUTPUT);
-#endif
             if (!shooting) continue;
             const EnvDesc& D = *Dp;
             {
@@ -509,7 +448,6 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                     rs_make_plans_warp(T.rs_acc, T.rs_lens, T.rs_npts, k0, nw, T.plans, q0, cq, sq, D.origin, P.maxc, stepn, lane);
                     STICK(PH_RS_PLAN);
                     unsigned dead = 0;
-#if AQ_COARSE
                     if (nw >= 2) {
                         const int per = 32 / nw;
                         const int r = lane / per, q = lane - r * per;
@@ -533,7 +471,6 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                             if (hitm & (((per >= 32) ? 0xffffffffu : ((1u << per) - 1u)) << (w * per))) dead |= 1u << w;
                         if (lane == 0) T.s_checks += (unsigned long long)__popc(livem);
                     }
-#endif
 #pragma unroll 1
                     for (int w = 0; w < nw; ++w) {
                         const RsPlan& plan = T.plans[w];
@@ -586,7 +523,7 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                 if (lane == 0) { __threadfence_block(); atomicMin(&S.shot_best, i); __threadfence_block(); T.done_epoch = my_epoch; }
                 __syncwarp();
                 active = false;
-            } else i += AQ_SHOOTERS;
+            } else ++i;
         }
         return;
     }
@@ -598,10 +535,9 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
     bool finished = false;
     int my_epoch = 0;
     const EnvDesc* Dp = eb.desc;
-    unsigned e_iter = 0;
     int helper_epoch = 0;
     while (true) {
-        if ((e_iter++ % AQ_EVERY_E) == 0 && role_barrier_all(2, AQ_SLOTS * AQ_TEAM, finished)) break;
+        if (role_barrier_all(2, AQ_SLOTS * AQ_TEAM, finished)) break;
         bool expanding = false;
         if (ew == 0) {
         do {
@@ -624,7 +560,7 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
             S.n_nodes = 0; S.heap_n = 0; S.counter = 0; S.n_closed = 0;
             S.status = -1; S.arrival = 0; S.goal_cost = 0.0; S.ew_status = -1; S.ew_arrival2 = 0;
             S.e_checks = 0; S.e_exact = 0; S.e_ref = 0; S.win = 0;
-            for (int k = 0; k < AQ_SHOOTERS; ++k) { S.sh[k].s_checks = 0; S.sh[k].s_exact = 0; S.sh[k].s_ref = 0; S.sh[k].rs_assert = 0; }
+            S.sh[0].s_checks = 0; S.sh[0].s_exact = 0; S.sh[0].s_ref = 0; S.sh[0].rs_assert = 0;
             S.fin_closed = 0; S.fin_counter = 0;
             S.popped = 0; S.ew_done = 0; S.shot_limit = 0; S.shot_best = AQ_NO_HIT;
             S.t0 = clock64();
@@ -719,7 +655,6 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
         }
         } while (0);
         }
-#if AQ_EXPANDERS > 1
         if (ew == 0 && lane == 0) { S.x_expanding = expanding ? 1 : 0; S.x_finished = finished ? 1 : 0; }
         team_sync(slot);
         if (ew != 0) {                                       // the helper follows warp 0's decisions
@@ -741,7 +676,6 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
                 }
             }
         }
-#endif
         const EnvDesc& D = *Dp;
         if (expanding) {
             {
@@ -982,17 +916,12 @@ k_hybrid_astar_s(EnvBatchDev eb, const HlScenario* __restrict__ scen, int n_scen
         __syncwarp();
         }
         if (mode == 2) {
-            {
-                bool all = true;
-#pragma unroll 1
-                for (int k = 0; k < AQ_SHOOTERS; ++k) all = all && (warp_read(&S.sh[k].done_epoch, lane) == my_epoch);
-                if (!all) { __nanosleep(100); continue; }
-            }
+            if (warp_read(&S.sh[0].done_epoch, lane) != my_epoch) { __nanosleep(100); continue; }
         __threadfence_block();
         if (lane == 0) {
             const int best = *(volatile int*)&S.shot_best;
             const int hit = (best == AQ_NO_HIT) ? -1 : best;
-            if (hit >= 0) S.win = hit % AQ_SHOOTERS;
+            if (hit >= 0) S.win = 0;
             if (hit >= 0 && S.sh[S.win].rs_assert && !(S.ew_arrival2 && hit >= S.n_closed - 1)) {
                 S.status = HL_STATUS_RS_ASSERT; S.fin_closed = hit + 1; S.fin_counter = hit + 1; S.arrival = 0;
             } else if (hit >= 0 && !(S.ew_arrival2 && hit >= S.n_closed - 1)) {     // first free word at pop `hit`

@@ -80,11 +80,8 @@ __device__ __forceinline__ float4 lds4(const float* p) { return *reinterpret_cas
 // instead; the float32 pipeline goes on as if the ambiguous test had passed (a later verdict can only add "hit"), and
 // when the CTA has no tile left its warps resolve the queue, one entry per warp at a time, all in parallel.
 #define K1_DEFER_CAP 48
-#ifndef K1_DRAIN_MID
-#define K1_DRAIN_MID 0                    // 1: drain the float64 queue between tiles as soon as every warp gets an entry.
-                                          // Measured SLOWER (16.86 vs 17.43 G checks/s, 16 Mi random poses): tiles are assigned
-                                          // by a fixed stride, so a CTA that stops to drain simply finishes that much later
-#endif
+// Draining between tiles measured slower (16.86 vs 17.43 G checks/s, 16 Mi random poses): tiles are assigned by a fixed
+// stride, so a CTA that stops to drain simply finishes that much later.
 struct K1Defer { long long i; int env; unsigned amb; int rect; int pad; };
 struct __align__(16) K1Cta {
     double raw[K1_TILE * 3];              // TMA landing zone: x, y, yaw of the tile                        24 KB
@@ -832,20 +829,6 @@ k_collision(EnvBatchDev eb, const int32_t* __restrict__ env_id, const double* __
             }
         }
         __syncthreads();                                   // S.st / lists are rewritten by the next tile
-#if K1_DRAIN_MID
-        // experiment (off): drain the queue BETWEEN tiles once every warp gets an entry, and whatever is pending before
-        // the CTA's last tile, so that the other CTAs of the SM keep the pipes busy meanwhile
-        {
-            const int nq = S.dq_cnt;                       // CTA-uniform: read behind the barrier
-            const bool last_next = tile + gridDim.x < n_tiles && tile + 2 * (long long)gridDim.x >= n_tiles;
-            if (nq >= K1_WARPS || (last_next && nq > 0)) {
-                drain_queue();
-                __syncthreads();
-                if (tid == 0) S.dq_cnt = 0;
-                __syncthreads();
-            }
-        }
-#endif
     }
     // ---- what is still queued: one entry per warp at a time, every warp busy
     drain_queue();

@@ -83,66 +83,22 @@ __global__ void k_df_seed(const DfField* __restrict__ fs, int n, int2* __restric
     if (fi < n) df_seed(fs[fi], fi, list, count);
 }
 
-// DF_CPT cells per thread of a DF_TILE x DF_TILE tile (DF_TILE^2 / DF_CPT threads), the move set a template parameter: the 8 (King) or 5
-// (Pawn) predecessors are compile-time offsets into the shared tile.  Only the neighbours that read an improved border
-// cell in their halo are flagged for the next launch.  History on the 4096 x 4096 King field:
-//   16.1 ms  one CTA per map tile, move table in a rolled loop, a host look per launch
-//   14.4     frontier list, launches queued 16 at a time          13.3  constant offsets
-//    9.2     directional flags                                      7.8  two cells per thread, no memset between launches
-//   (tools/variants_df.sh: 1 / 2 / 4 cells per thread 9.2 / 7.8 / 10.0 ms; tried and slower: one WARP per tile with
-//    Gauss-Seidel sweeps, 12.1 ms -- what a launch costs is the latency of the slowest tile visit)
-// ncu on that version (profiles/r2v_k6_*): a launch is ISSUE-bound, 74 % issue-active, FP64 pipe 26 %, and two thirds of
-// the instructions were fmin's NaN handling (DSETP.MIN + fix-up + moves, 7 per minimum).  Costs are never NaN, so:
-//    6.1 ms  minimum as compare + two selects                       5.7  a thread's two cells vertically ADJACENT (10 loads
-//                                                                        of the shared 3-column neighbourhood instead of 16)
-//    5.0     the compare on the FP64 pipe (DSETP.LT, 3 instructions) instead of a 64-bit integer compare (4)
-//    4.6     a warp skips an iteration when no row it can see changed (the wave crosses a tile as a band)
-//    4.26    minimum of the predecessors FIRST, one addition per weight (exact: fl(x + w) is monotone in x)
-// (3 CTAs per SM at 35 registers: 4.79; 4 cells per thread: 4.71; first host look after (tiles_i + tiles_j) / 2 launches.)
-//    4.03    16 x 16 tiles of 128 threads (310 launches of 13 us, four times the frontier list)
-//    3.47    launches chained by programmatic dependent launch (DF_PDL)
+// DF_CPT vertically adjacent cells per thread of a DF_TILE x DF_TILE tile (DF_TILE^2 / DF_CPT threads), the move set a
+// template parameter: the 8 (King) or 5 (Pawn) predecessors are compile-time offsets into the shared tile.  Only the
+// neighbours that read an improved border cell in their halo are flagged for the next launch.  How each step of this
+// design was measured on the 4096 x 4096 King field: DESIGN.md section 5, "K6 relaxation".
 #ifndef DF_CPT
 #define DF_CPT 2
 #endif
-#ifndef DF_ADJ
-#define DF_ADJ 1                       // 1: a thread's cells are vertically ADJACENT (rows a0 .. a0 + DF_CPT - 1): the three-column
-#endif                                 // neighbourhood of the cells overlaps, 5 + 5 (King) loads for 2 cells instead of 16;
-                                       // 0: rows DF_TILE / DF_CPT apart (round-2 first version)
 #define DF_RELAX_THREADS (DF_TILE * DF_TILE / DF_CPT)
-#if DF_ADJ
-#define DF_ROW0(tid) (1 + DF_CPT * ((tid) / DF_TILE))
-#define DF_ROW(a0, q) ((a0) + (q))
-#else
-#define DF_ROW0(tid) (1 + ((tid) / DF_TILE))
-#define DF_ROW(a0, q) ((a0) + (q) * (DF_TILE / DF_CPT))
-#endif
-// min of two costs.  Costs are +0, positive or +inf, never NaN: their bit patterns order like integers, so the minimum is
-// an integer compare + two selects (4 ALU instructions) instead of fmin's DSETP.MIN + NaN fix-up + moves (7, one of
-// them on the FP64 pipe).  The relaxation kernel is issue-bound (ncu: issue-active 74 %), instructions are time.
-#ifndef DF_MIN_MODE
-#define DF_MIN_MODE 1                  // 0: integer compare (4 ALU instructions); 1: DSETP.LT + two selects (3, one on the FP64 pipe);
-                                       // 2: half each.  Measured (4096 x 4096 King, row skip on): 4.93 / 4.57 / 4.81 ms
-#endif
-__device__ __forceinline__ double df_min_i(double a, double b) {
-    const long long x = __double_as_longlong(a), y = __double_as_longlong(b);
-    return __longlong_as_double(y < x ? y : x);
-}
-__device__ __forceinline__ double df_min_d(double a, double b) { return (b < a) ? b : a; }
-// df_min serves the straight moves, df_min2 the diagonal ones (mode 2: integer / FP64 compare, half each)
-__device__ __forceinline__ double df_min(double a, double b) { return DF_MIN_MODE == 1 ? df_min_d(a, b) : df_min_i(a, b); }
-__device__ __forceinline__ double df_min2(double a, double b) { return DF_MIN_MODE == 0 ? df_min_i(a, b) : df_min_d(a, b); }
+// min of two costs.  Costs are +0, positive or +inf, never NaN, so the minimum is a compare + two selects (DSETP.LT, 3
+// instructions, one on the FP64 pipe) instead of fmin's DSETP.MIN + NaN fix-up + moves (7).  The relaxation kernel is
+// issue-bound (ncu: issue-active 74 %), instructions are time.
+__device__ __forceinline__ double df_min(double a, double b) { return (b < a) ? b : a; }
+// non-negative doubles order like their bit patterns
 __device__ __forceinline__ bool df_less(double a, double b) { return __double_as_longlong(a) < __double_as_longlong(b); }
 #ifndef DF_MIN_CTAS
 #define DF_MIN_CTAS 2                    // launch bound (with 32 x 32 tiles: 64 registers = two 512-thread CTAs per SM, 66 would leave one)
-#endif
-#ifndef DF_PDL
-#define DF_PDL 1                        // relaxation launches with programmatic stream serialization (griddepcontrol)
-#endif
-#ifndef DF_MIN_TREE
-#define DF_MIN_TREE 1                   // one addition per weight: min of the predecessors first (exact, see the loop)
-#endif
-#ifndef DF_ROWSKIP
-#define DF_ROWSKIP 1                    // a warp sits an iteration out when no row its cells can see changed in the previous one
 #endif
 // ONE: the wavefront has a single grid, passed by value (`one`) instead of read from the table per tile: its fields are
 // then kernel constants, as in the single-map kernel before batching, and take no registers across the relaxation loop
@@ -156,24 +112,20 @@ k_df_relax(const DfField* __restrict__ fields, const DfField one, const int2* __
     // CTAs of which a few hundred have work).  No memset between launches: a tile clears its own mark when it is
     // processed, and the counter the launch after next appends to is zeroed here (three counters rotate).  The tiles of
     // all grids of a batch share the list; marks are indexed by the global tile id (tile_base + tile).
-#if DF_PDL
     // programmatic dependent launch: this grid was scheduled while the previous relaxation launch was still running;
     // nothing that launch wrote is read before it has completed, and the NEXT launch may be scheduled from here on
     // (its CTAs wait at the same point), so the ~2 us between two dependent launches overlap with the work
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
     if (blockIdx.x == 0 && threadIdx.x == 0) *count_clear = 0;
     __shared__ double sd[DF_TILE + 2][DF_TILE + 3];
     __shared__ unsigned char so[DF_TILE + 2][DF_TILE + 2];
     __shared__ int s_border_changed;
-#if DF_ROWSKIP
     __shared__ int s_rowchg[2][DF_TILE + 2];            // rows that changed in the previous / this iteration
-#endif
     const double W1 = 1.0, W2 = 1.4142135623730951;       // hypot(1, 0), hypot(1, 1) as the host's libm gives them
     const int n_cur = *count_cur;
     const int tid = threadIdx.x;
-    const int a0 = DF_ROW0(tid), b = 1 + (tid % DF_TILE);      // cell q of this thread: row DF_ROW(a0, q), column b
+    const int a0 = 1 + DF_CPT * (tid / DF_TILE), b = 1 + (tid % DF_TILE);   // cell q of this thread: row a0 + q, column b
     for (int li = blockIdx.x; li < n_cur; li += gridDim.x) {
         const int2 entry = list_cur[li];
         const DfField f = ONE ? one : fields[entry.x];
@@ -188,10 +140,8 @@ k_df_relax(const DfField* __restrict__ fields, const DfField one, const int2* __
         const int ti = tile / tiles_j, tj = tile % tiles_j;
         const int i0 = ti * DF_TILE - 1, j0 = tj * DF_TILE - 1;
         if (tid == 0) { s_border_changed = 0; mark_cur[tile_base + tile] = 0; }
-#if DF_ROWSKIP
         if (tid < DF_TILE + 2) { s_rowchg[0][tid] = 1; s_rowchg[1][tid] = 0; }      // first iteration: every row counts as changed
         int it = 0;
-#endif
         for (int k = tid; k < (DF_TILE + 2) * (DF_TILE + 2); k += DF_RELAX_THREADS) {
             const int x = k / (DF_TILE + 2), y = k % (DF_TILE + 2);
             const int i = i0 + x, j = j0 + y;
@@ -204,14 +154,13 @@ k_df_relax(const DfField* __restrict__ fields, const DfField one, const int2* __
         bool enter[DF_CPT];
 #pragma unroll
         for (int q = 0; q < DF_CPT; ++q) {
-            const int a = DF_ROW(a0, q);
+            const int a = a0 + q;
             init[q] = cur[q] = sd[a][b];
             // occupied cells are never entered (the goal cell itself is exempt: it starts closed at 0)
             enter[q] = !so[a][b] && i0 + a < W && j0 + b < H;
         }
         while (true) {
             double best[DF_CPT];
-#if DF_ROWSKIP && DF_ADJ
             // a cell can only change if a cell of rows a0 - 1 .. a0 + DF_CPT changed in the previous iteration: the warp
             // (one group of DF_CPT rows) sits the iteration out otherwise (the wave crosses a tile as a band)
             int seen = 0;
@@ -221,103 +170,53 @@ k_df_relax(const DfField* __restrict__ fields, const DfField one, const int2* __
 #pragma unroll
                 for (int q = 0; q < DF_CPT; ++q) best[q] = cur[q];
             } else {
-#endif
-#if DF_ADJ
-            // columns b - 1, b, b + 1 of rows a0 - 1 .. a0 + DF_CPT; the thread's own cells (column b) are in registers,
-            // and a cell sees the value its upper neighbour in the same thread was just given (any relaxation order
-            // reaches the same fixed point)
-            double L[DF_CPT + 2], M[DF_CPT + 2], R[DF_CPT + 2];
+                // columns b - 1, b, b + 1 of rows a0 - 1 .. a0 + DF_CPT; the thread's own cells (column b) are in
+                // registers, and a cell sees the value its upper neighbour in the same thread was just given (any
+                // relaxation order reaches the same fixed point)
+                double L[DF_CPT + 2], M[DF_CPT + 2], R[DF_CPT + 2];
 #pragma unroll
-            for (int r = 0; r < DF_CPT + 2; ++r) {
-                L[r] = sd[a0 - 1 + r][b - 1];
-                R[r] = KING ? sd[a0 - 1 + r][b + 1] : 0.0;
-            }
-            M[0] = sd[a0 - 1][b]; M[DF_CPT + 1] = sd[a0 + DF_CPT][b];
-#pragma unroll
-            for (int q = 0; q < DF_CPT; ++q) M[q + 1] = cur[q];
-#if DF_MIN_TREE
-            // fl(x + w) is monotone in x, so min(fl(x + w), fl(y + w)) == fl(min(x, y) + w) bit for bit: ONE addition per
-            // weight and cell (the minimum of the straight predecessors + 1, of the diagonal ones + sqrt 2) instead of
-            // eight, and the minimum of a row's left and right cell serves the cell between them (straight) and the two
-            // cells above / below it (diagonal).  Pawn moves only come from column b - 1.
-            double hr[DF_CPT + 2];
-#pragma unroll
-            for (int r = 0; r < DF_CPT + 2; ++r) hr[r] = KING ? df_min(L[r], R[r]) : L[r];
-#pragma unroll
-            for (int q = 0; q < DF_CPT; ++q) {
-                const int r = q + 1;
-                double v = cur[q];
-                if (enter[q]) {
-                    const double m1 = df_min(df_min(M[r - 1], M[r + 1]), hr[r]);
-                    const double m2 = df_min(hr[r - 1], hr[r + 1]);
-                    v = df_min(v, df_min(__dadd_rn(m1, W1), __dadd_rn(m2, W2)));
+                for (int r = 0; r < DF_CPT + 2; ++r) {
+                    L[r] = sd[a0 - 1 + r][b - 1];
+                    R[r] = KING ? sd[a0 - 1 + r][b + 1] : 0.0;
                 }
-                best[q] = v;
-                M[r] = v;
-            }
-#else
+                M[0] = sd[a0 - 1][b]; M[DF_CPT + 1] = sd[a0 + DF_CPT][b];
 #pragma unroll
-            for (int q = 0; q < DF_CPT; ++q) {
-                const int r = q + 1;
-                double v = cur[q];
-                if (enter[q]) {                                     // predecessor of move (di, dj) is (a - di, b - dj)
-                    v = df_min(v, __dadd_rn(M[r + 1], W1));                             // (-1,  0)
-                    v = df_min(v, __dadd_rn(L[r], W1));                                 // ( 0,  1)
-                    v = df_min2(v, __dadd_rn(L[r + 1], W2));                             // (-1,  1)
-                    v = df_min2(v, __dadd_rn(L[r - 1], W2));                             // ( 1,  1)
-                    v = df_min(v, __dadd_rn(M[r - 1], W1));                             // ( 1,  0)
-                    if (KING) {
-                        v = df_min2(v, __dadd_rn(R[r - 1], W2));                         // ( 1, -1)
-                        v = df_min(v, __dadd_rn(R[r], W1));                             // ( 0, -1)
-                        v = df_min2(v, __dadd_rn(R[r + 1], W2));                         // (-1, -1)
+                for (int q = 0; q < DF_CPT; ++q) M[q + 1] = cur[q];
+                // fl(x + w) is monotone in x, so min(fl(x + w), fl(y + w)) == fl(min(x, y) + w) bit for bit: ONE addition
+                // per weight and cell (the minimum of the straight predecessors + 1, of the diagonal ones + sqrt 2)
+                // instead of eight, and the minimum of a row's left and right cell serves the cell between them
+                // (straight) and the two cells above / below it (diagonal).  Pawn moves only come from column b - 1.
+                double hr[DF_CPT + 2];
+#pragma unroll
+                for (int r = 0; r < DF_CPT + 2; ++r) hr[r] = KING ? df_min(L[r], R[r]) : L[r];
+#pragma unroll
+                for (int q = 0; q < DF_CPT; ++q) {
+                    const int r = q + 1;
+                    double v = cur[q];
+                    if (enter[q]) {
+                        const double m1 = df_min(df_min(M[r - 1], M[r + 1]), hr[r]);
+                        const double m2 = df_min(hr[r - 1], hr[r + 1]);
+                        v = df_min(v, df_min(__dadd_rn(m1, W1), __dadd_rn(m2, W2)));
                     }
+                    best[q] = v;
+                    M[r] = v;
                 }
-                best[q] = v;
-                M[r] = v;
             }
-#endif
-#if DF_ROWSKIP
-            }
-#endif
-#else
-#pragma unroll
-            for (int q = 0; q < DF_CPT; ++q) {
-                const int a = DF_ROW(a0, q);
-                double v = cur[q];
-                if (enter[q]) {                                     // predecessor of move (di, dj) is (a - di, b - dj)
-                    v = df_min(v, __dadd_rn(sd[a + 1][b], W1));                           // (-1,  0)
-                    v = df_min(v, __dadd_rn(sd[a][b - 1], W1));                           // ( 0,  1)
-                    v = df_min(v, __dadd_rn(sd[a + 1][b - 1], W2));                       // (-1,  1)
-                    v = df_min(v, __dadd_rn(sd[a - 1][b - 1], W2));                       // ( 1,  1)
-                    v = df_min(v, __dadd_rn(sd[a - 1][b], W1));                           // ( 1,  0)
-                    if (KING) {
-                        v = df_min(v, __dadd_rn(sd[a - 1][b + 1], W2));                   // ( 1, -1)
-                        v = df_min(v, __dadd_rn(sd[a][b + 1], W1));                       // ( 0, -1)
-                        v = df_min(v, __dadd_rn(sd[a + 1][b + 1], W2));                   // (-1, -1)
-                    }
-                }
-                best[q] = v;
-            }
-#endif
             __syncthreads();
             bool ch = false;
 #pragma unroll
             for (int q = 0; q < DF_CPT; ++q)
                 if (df_less(best[q], cur[q])) {
-                    sd[DF_ROW(a0, q)][b] = best[q]; cur[q] = best[q]; ch = true;
-#if DF_ROWSKIP && DF_ADJ
-                    s_rowchg[(it + 1) & 1][DF_ROW(a0, q)] = 1;
-#endif
+                    sd[a0 + q][b] = best[q]; cur[q] = best[q]; ch = true;
+                    s_rowchg[(it + 1) & 1][a0 + q] = 1;
                 }
-#if DF_ROWSKIP && DF_ADJ
             if (tid < DF_TILE + 2) s_rowchg[it & 1][tid] = 0;      // read before the barrier above, written again in iteration it + 2
             ++it;
-#endif
             if (!__syncthreads_or(ch)) break;
         }
 #pragma unroll
         for (int q = 0; q < DF_CPT; ++q) {
-            const int a = DF_ROW(a0, q);
+            const int a = a0 + q;
             const int i = i0 + a, j = j0 + b;
             if (cur[q] < init[q] && i < W && j < H) {
                 D[(long long)i * H + j] = cur[q];
@@ -481,11 +380,7 @@ static int df_wavefront(const char* what, const std::vector<DfField>& rel, const
             cudaMemsetAsync(flags + 1, 0, DF_BATCH * sizeof(int), st);
             for (int k = 0; k < DF_BATCH; ++k) {
                 const int lc = cur & 1, ln = lc ^ 1;
-#ifdef DF_MEMSET
-                cudaMemsetAsync(mark[ln], 0, sizeof(int) * (size_t)n_tiles, st);
-#endif
                 int* c_cur = count + cur % 3; int* c_nxt = count + (cur + 1) % 3; int* c_clr = count + (cur + 2) % 3;
-#if DF_PDL
                 cudaLaunchConfig_t cfg;
                 memset(&cfg, 0, sizeof(cfg));
                 cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(DF_RELAX_THREADS); cfg.dynamicSmemBytes = 0; cfg.stream = st;
@@ -498,10 +393,6 @@ static int df_wavefront(const char* what, const std::vector<DfField>& rel, const
                 if (cudaLaunchKernelEx(&cfg, relax, d_rel, rel[0], a_lc, a_cc, list[ln], c_nxt, mark[ln], mark[lc], c_clr, a_fl) != cudaSuccess) {
                     rc = 1; break;                              // a launch that did not happen would read as "frontier empty"
                 }
-#else
-                relax<<<grid, DF_RELAX_THREADS, 0, st>>>(d_rel, rel[0], list[lc], c_cur, list[ln], c_nxt, mark[ln], mark[lc], c_clr, flags + 1 + k);
-                if (cudaGetLastError() != cudaSuccess) { rc = 1; break; }
-#endif
                 ++cur;
             }
             if (rc) { cudaStreamSynchronize(st); break; }

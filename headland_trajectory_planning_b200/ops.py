@@ -361,8 +361,7 @@ def astar_launches_per_call(envs, n_scenarios):
     larger than the resident scenario slots in two launches: first shots only, then the scenarios they left over)."""
     import os
     sm = int(_lib.load_library().hl_ctx_sm_count(envs.ctx))
-    if os.environ.get("HL_ASTAR_SINGLE_PHASE") is None and os.environ.get("HL_ASTAR_VARIANT", "spec") == "spec" \
-            and n_scenarios > 2 * sm * 5:
+    if os.environ.get("HL_ASTAR_VARIANT", "spec") == "spec" and n_scenarios > 2 * sm * 5:
         return 2
     return 1
 

@@ -1,6 +1,6 @@
 #!/bin/bash
 # build K4 variants on the GPU box (only hl_astar.cu is recompiled, ~20 s) and time each:
-#   tools/variants.sh "<flags1>" "<flags2>" ...      e.g.  tools/variants.sh "" "-DAQ_FAR=3" "-DAQ_EVERY_E=2 -DAQ_EVERY_S=2"
+#   tools/variants.sh "<flags1>" "<flags2>" ...      e.g.  tools/variants.sh "" "-DAQ_FAR=3" "-DAQ_SLOTS=4 -DAQ_GD_UNROLL=2"
 cd "$(dirname "$0")/.."
 P=headland_trajectory_planning_b200
 build() {
