@@ -76,6 +76,17 @@ class HlRasterGrid(C.Structure):
     ]
 
 
+class HlGridPack(C.Structure):
+    _fields_ = [("occ_offset", C.c_int64), ("bits_offset", C.c_int64), ("w", C.c_int32), ("h", C.c_int32)]
+
+
+class HlGridMap(C.Structure):
+    _fields_ = [
+        ("bits_offset", C.c_int64), ("w", C.c_int32), ("h", C.c_int32), ("i0", C.c_int32), ("j0", C.c_int32),
+        ("body_ext", C.c_double * 4), ("aux_first", C.c_int32), ("n_aux", C.c_int32),
+    ]
+
+
 SCENARIO_DTYPE = np.dtype([("env_id", "<i4"), ("reserved", "<i4"),
                            ("start", "<f8", (3,)), ("goal", "<f8", (3,))])
 RESULT_DTYPE = np.dtype([("status", "<i4"), ("counter", "<i4"), ("n_expanded", "<i4"),
@@ -93,6 +104,7 @@ EXPORTS = [
     "hl_ctx_set_astar_variant", "hl_env_upload", "hl_env_free", "hl_env_count", "hl_env_device", "hl_collision_check", "hl_path_reduce",
     "hl_rs_all_paths", "hl_rs_sample", "hl_hybrid_astar_batch", "hl_hybrid_astar_workspace_bytes", "hl_astar_phase_cycles",
     "hl_distance_field", "hl_distance_field_batch", "hl_grid_pack", "hl_grid_footprint_check", "hl_grid_footprint_check_at", "hl_env_rasterize",
+    "hl_grid_pack_batch", "hl_grid_footprint_check_batch",
     "hl_measure_fp32_peak", "hl_ypark_paths", "hl_arc_paths", "hl_ref_path_count", "hl_ref_path_fill",
     "hl_dubins_count", "hl_dubins_knots", "hl_dubins_fill", "hl_min_boundary_distance", "hl_corridor_hits",
 ]
@@ -174,6 +186,9 @@ def load_library():
         lib.hl_grid_pack.argtypes = [vp, vp, i32, i32, vp, vp]
         lib.hl_grid_footprint_check.argtypes = [vp, vp, i32, i32, dbl, vp, i64, C.POINTER(dbl), vp, vp]
         lib.hl_grid_footprint_check_at.argtypes = [vp, vp, i32, i32, i32, i32, dbl, vp, i64, C.POINTER(dbl), vp, vp]
+        lib.hl_grid_pack_batch.argtypes = [vp, vp, i64, C.POINTER(HlGridPack), i32, vp, i64, vp]
+        lib.hl_grid_footprint_check_batch.argtypes = [vp, vp, i64, C.POINTER(HlGridMap), i32, C.POINTER(dbl), i32, dbl, vp, vp,
+                                                      vp, i64, u32, vp, vp]
         lib.hl_env_rasterize.argtypes = [vp, vp, C.POINTER(HlRasterGrid), i32, dbl, u32, vp, i64, vp, vp]
         lib.hl_measure_fp32_peak.argtypes = [vp, C.POINTER(dbl)]
         lib.hl_ypark_paths.argtypes = [vp, vp, vp, i64, dbl, vp, vp]

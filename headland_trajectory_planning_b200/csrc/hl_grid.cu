@@ -596,24 +596,114 @@ extern "C" int hl_distance_field_batch(hl_ctx* ctx, const uint8_t* d_occ, int64_
 }
 
 // ------------------------------------------------------------------------- K7
-__global__ void k_grid_pack(const uint8_t* __restrict__ occ, long long cells, uint32_t* __restrict__ bits) {
-    long long wd = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    long long n_words = (cells + 31) / 32;
-    if (wd >= n_words) return;
-    uint32_t v = 0;
-    for (int b = 0; b < 32; ++b) {
-        long long c = wd * 32 + b;
-        if (c < cells && occ[c]) v |= 1u << b;
+// Every K7 entry point runs over a table: hl_grid_pack and hl_grid_footprint_check(_at) are batches of one whose
+// single entry is passed by value (tab / maps == NULL), so they copy nothing to the device.
+
+// one grid of a pack: its bytes, its bit slice and its first chunk (GP_WPW words) in the batch's chunk numbering
+struct GpGrid {
+    const uint8_t* occ;
+    uint32_t* bits;
+    long long cells;
+    long long chunk_base;
+};
+
+#define GP_WPW 32                         // words (of 32 cells) per warp
+static long long gp_chunks(long long cells) { return ((cells + 31) / 32 + GP_WPW - 1) / GP_WPW; }
+
+// One warp per chunk of GP_WPW consecutive words of one grid.  Round q: lane b reads cell 32 * (first word + q) + b
+// (a coalesced 32-byte load; all GP_WPW loads are issued before the first ballot) and the ballot is word q, bit b =
+// that cell, zero past the last cell; lane q keeps word q and the warp stores its words in one coalesced write.  The
+// chunks of all grids share one numbering (chunk_base): one table search per GP_WPW words.
+__global__ void __launch_bounds__(256) k_grid_pack(const GpGrid* __restrict__ tab, int n, const GpGrid one, long long chunks) {
+    const long long g = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    if (g >= chunks) return;                                  // the same for every lane of a warp
+    GpGrid e = one;
+    if (tab) {
+        int lo = 0, hi = n - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (tab[mid].chunk_base <= g) lo = mid; else hi = mid - 1;
+        }
+        e = tab[lo];
+        __builtin_assume(__isGlobal(e.occ));
+        __builtin_assume(__isGlobal(e.bits));
     }
-    bits[wd] = v;
+    const int lane = threadIdx.x & 31;
+    const long long wa = (g - e.chunk_base) * GP_WPW;         // first word of the chunk
+    const long long left = e.cells - wa * 32 - lane;          // round q reads this lane's cell iff 32 * q < left
+    const uint8_t* __restrict__ src = e.occ + wa * 32 + lane;
+    uint32_t v[GP_WPW];
+#pragma unroll
+    for (int q = 0; q < GP_WPW; ++q) v[q] = (32 * q < left) ? __ldg(src + 32 * q) : 0;
+    uint32_t mine = 0;
+#pragma unroll
+    for (int q = 0; q < GP_WPW; ++q) {
+        const uint32_t b = __ballot_sync(0xFFFFFFFFu, v[q] != 0);
+        if (lane == q) mine = b;
+    }
+    if (wa + lane < (e.cells + 31) / 32) e.bits[wa + lane] = mine;
 }
 
 extern "C" int hl_grid_pack(hl_ctx* ctx, const uint8_t* d_occ, int32_t w, int32_t h, uint32_t* d_bits, void* stream) {
     if (!ctx || !d_occ || !d_bits || w <= 0 || h <= 0) { hl_set_error("hl_grid_pack: bad arguments"); return 1; }
     if (hl_enter(ctx, nullptr, d_bits, "hl_grid_pack")) return 1;
-    long long cells = (long long)w * h, n_words = (cells + 31) / 32;
-    k_grid_pack<<<(unsigned)((n_words + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d_occ, cells, d_bits);
+    const long long cells = (long long)w * h, chunks = gp_chunks(cells);
+    const GpGrid one = {d_occ, d_bits, cells, 0};
+    k_grid_pack<<<(unsigned)((chunks + 7) / 8), 256, 0, (cudaStream_t)stream>>>(nullptr, 1, one, chunks);
     HL_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int hl_grid_pack_batch(hl_ctx* ctx, const uint8_t* d_occ, int64_t occ_bytes, const HlGridPack* h_grids,
+                                  int32_t n_grids, uint32_t* d_bits, int64_t bits_words, void* stream) {
+    const char* what = "hl_grid_pack_batch";
+    if (!ctx || n_grids < 0 || occ_bytes < 0 || bits_words < 0 || (n_grids > 0 && (!h_grids || !d_occ || !d_bits))) {
+        hl_set_error("%s: bad arguments", what); return 1;
+    }
+    std::vector<GpGrid> tab(n_grids);
+    long long chunks = 0;
+    for (int k = 0; k < n_grids; ++k) {
+        const HlGridPack& g = h_grids[k];
+        if (g.w < 1 || g.h < 1) { hl_set_error("%s: grid %d: a %dx%d grid (w and h must be at least 1)", what, k, g.w, g.h); return 1; }
+        const long long cells = (long long)g.w * g.h, nw = (cells + 31) / 32;
+        if (g.occ_offset < 0 || g.occ_offset > occ_bytes - cells) {
+            hl_set_error("%s: grid %d: grid bytes [%lld, %lld) outside the %lld bytes of d_occ", what, k,
+                         (long long)g.occ_offset, (long long)g.occ_offset + cells, (long long)occ_bytes); return 1;
+        }
+        if (g.bits_offset < 0 || g.bits_offset > bits_words - nw) {
+            hl_set_error("%s: grid %d: bit slice [%lld, %lld) outside the %lld words of d_bits", what, k,
+                         (long long)g.bits_offset, (long long)g.bits_offset + nw, (long long)bits_words); return 1;
+        }
+        tab[k] = {d_occ + g.occ_offset, d_bits + g.bits_offset, cells, chunks};
+        chunks += gp_chunks(cells);
+    }
+    // sorted by start, two slices overlap only if some pair of neighbours does
+    std::vector<int> order(n_grids);
+    for (int k = 0; k < n_grids; ++k) order[k] = k;
+    std::sort(order.begin(), order.end(), [&](int a, int b) {
+        return h_grids[a].bits_offset != h_grids[b].bits_offset ? h_grids[a].bits_offset < h_grids[b].bits_offset : a < b;
+    });
+    for (int k = 1; k < n_grids; ++k) {
+        const HlGridPack& a = h_grids[order[k - 1]];
+        if (h_grids[order[k]].bits_offset < a.bits_offset + ((long long)a.w * a.h + 31) / 32) {
+            hl_set_error("%s: grids %d and %d: bit slices overlap", what, std::min(order[k - 1], order[k]),
+                         std::max(order[k - 1], order[k]));
+            return 1;
+        }
+    }
+    if ((chunks + 7) / 8 > INT_MAX) { hl_set_error("%s: %lld chunks of %d words exceed one launch", what, chunks, GP_WPW); return 1; }
+    if (hl_enter(ctx, nullptr, n_grids ? d_bits : nullptr, what)) return 1;
+    if (n_grids == 0) return 0;
+    const cudaStream_t st = (cudaStream_t)stream;
+    GpGrid* d_tab = nullptr;
+    HL_CUDA_OK(cudaMallocAsync((void**)&d_tab, sizeof(GpGrid) * (size_t)n_grids, st));
+    cudaError_t e = cudaMemcpyAsync(d_tab, tab.data(), sizeof(GpGrid) * (size_t)n_grids, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) {
+        k_grid_pack<<<(unsigned)((chunks + 7) / 8), 256, 0, st>>>(d_tab, n_grids, tab[0], chunks);
+        e = cudaGetLastError();
+    }
+    cudaFreeAsync(d_tab, st);
+    if (e != cudaSuccess) { hl_set_error("%s: CUDA error: %s", what, cudaGetErrorString(e)); return 1; }
     return 0;
 }
 
@@ -647,16 +737,20 @@ __device__ __forceinline__ void cell_range(double vmin, double vmax, double res,
     lo = max(lo, (long long)g0); hi = min(hi, b - 1);
 }
 
-// (gi0, gj0): global index of the grid's cell (0, 0); bits are indexed by the local cell (i - gi0) * H + (j - gj0)
-__global__ void __launch_bounds__(256)
-k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, int gi0, int gj0, double res, const double* __restrict__ poses,
-                 long long n, double x0, double x1, double y0, double y1, uint8_t* __restrict__ out) {
-    long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (idx >= n) return;
-    const double px = poses[3 * idx], py = poses[3 * idx + 1], yaw = poses[3 * idx + 2];
-    // a pose that is not finite can never be certified free (fmin / fmax below would drop NaN corners)
-    if (!isfinite(px) || !isfinite(py) || !isfinite(yaw)) { out[idx] = 1; return; }
-    const double c = cos(yaw), s = sin(yaw);
+// one map of a footprint check: the grid's bit slice, its size and origin (global index of cell (0, 0)), the body
+// rectangle and the vehicle's implement rectangles [aux_first, aux_first + n_aux) of the pooled extent array
+struct GfMap {
+    const uint32_t* bits;
+    int w, h, i0, j0;
+    double ext[4];                // x0, x1, y0, y1
+    int aux_first, n_aux;
+};
+
+// does the closed rectangle [x0, x1] x [y0, y1] of the pose (px, py, c = cos yaw, s = sin yaw) meet the closed square
+// of an occupied cell?  A scanline over the grid columns the rotated rectangle spans; stops at the first hit.
+__device__ __forceinline__ bool rect_meets_grid(const uint32_t* __restrict__ bits, int W, int H, int gi0, int gj0, double res,
+                                                double px, double py, double c, double s, double x0, double x1, double y0,
+                                                double y1) {
     const double lx[4] = {x0, x0, x1, x1}, ly[4] = {y1, y0, y0, y1};
     double cx[4], cy[4];
     double xmin = INFINITY, xmax = -INFINITY;
@@ -669,8 +763,7 @@ k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, int gi0, int g
     // closed sets: a rectangle touching a cell edge meets the cells on both sides of it
     long long ia, ib;
     cell_range(xmin, xmax, res, gi0, W, ia, ib);
-    bool hit = false;
-    for (long long i = ia; i <= ib && !hit; ++i) {
+    for (long long i = ia; i <= ib; ++i) {
         const double a = (double)i * res, b = ((double)i + 1.0) * res;
         double ymin = INFINITY, ymax = -INFINITY;
 #pragma unroll
@@ -692,7 +785,37 @@ k_grid_footprint(const uint32_t* __restrict__ bits, int W, int H, int gi0, int g
         if (ymin > ymax) continue;
         long long ja, jb;
         cell_range(ymin, ymax, res, gj0, H, ja, jb);
-        if (ja <= jb) hit = row_any(bits, (i - gi0) * H, (int)(ja - gj0), (int)(jb - gj0));
+        if (ja <= jb && row_any(bits, (i - gi0) * H, (int)(ja - gj0), (int)(jb - gj0))) return true;
+    }
+    return false;
+}
+
+// One pose per thread.  Pose p uses map map_id[p] (map 0 without map_id; `one` when maps is NULL); a map id outside
+// [0, n_maps) hits.  The body rectangle always counts; with pose_idx (HL_CHECK_AUX) so do the map's implement
+// rectangles at even pose_idx[p] (car_model.py:58).  cos / sin once per pose, the first hit ends the pose.
+__global__ void __launch_bounds__(256)
+k_grid_footprint(const GfMap* __restrict__ maps, int n_maps, const GfMap one, const double* __restrict__ aux,
+                 const int32_t* __restrict__ map_id, const double* __restrict__ poses, const int32_t* __restrict__ pose_idx,
+                 long long n, double res, uint8_t* __restrict__ out) {
+    const long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (idx >= n) return;
+    const int mid = map_id ? map_id[idx] : 0;
+    if (mid < 0 || mid >= n_maps) { out[idx] = 1; return; }
+    const double px = poses[3 * idx], py = poses[3 * idx + 1], yaw = poses[3 * idx + 2];
+    // a pose that is not finite can never be certified free (fmin / fmax in the check would drop NaN corners)
+    if (!isfinite(px) || !isfinite(py) || !isfinite(yaw)) { out[idx] = 1; return; }
+    const GfMap m = maps ? maps[mid] : one;
+    __builtin_assume(__isGlobal(m.bits));
+    const double c = cos(yaw), s = sin(yaw);
+    const int n_rect = 1 + ((pose_idx && (pose_idx[idx] & 1) == 0) ? m.n_aux : 0);
+    bool hit = false;
+    for (int r = 0; r < n_rect && !hit; ++r) {
+        double x0 = m.ext[0], x1 = m.ext[1], y0 = m.ext[2], y1 = m.ext[3];
+        if (r) {
+            const double* e = aux + 4 * ((long long)m.aux_first + r - 1);
+            x0 = __ldg(e); x1 = __ldg(e + 1); y0 = __ldg(e + 2); y1 = __ldg(e + 3);
+        }
+        hit = rect_meets_grid(m.bits, m.w, m.h, m.i0, m.j0, res, px, py, c, s, x0, x1, y0, y1);
     }
     out[idx] = hit ? 1 : 0;
 }
@@ -702,12 +825,12 @@ static int grid_footprint_launch(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_
                                  void* stream, const char* what) {
     if (n == 0) return 0;
     if (hl_enter(ctx, nullptr, d_out, what)) return 1;
+    const GfMap one = {d_occ_bits, w, h, i0, j0, {body_ext[0], body_ext[1], body_ext[2], body_ext[3]}, 0, 0};
     k_grid_footprint<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        d_occ_bits, w, h, i0, j0, res, d_poses, (long long)n, body_ext[0], body_ext[1], body_ext[2], body_ext[3], d_out);
+        nullptr, 1, one, nullptr, nullptr, d_poses, nullptr, (long long)n, res, d_out);
     HL_CUDA_OK(cudaGetLastError());
     return 0;
 }
-
 extern "C" int hl_grid_footprint_check(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_t w, int32_t h,
                                        double res, const double* d_poses, int64_t n,
                                        const double body_ext[4], uint8_t* d_out, void* stream) {
@@ -732,4 +855,65 @@ extern "C" int hl_grid_footprint_check_at(hl_ctx* ctx, const uint32_t* d_occ_bit
         hl_set_error("%s: the grid's cell edges are not finite at res = %g", what, res); return 1;
     }
     return grid_footprint_launch(ctx, d_occ_bits, w, h, i0, j0, res, d_poses, n, body_ext, d_out, stream, what);
+}
+
+extern "C" int hl_grid_footprint_check_batch(hl_ctx* ctx, const uint32_t* d_bits, int64_t bits_words, const HlGridMap* h_maps,
+                                             int32_t n_maps, const double* h_aux_ext, int32_t n_aux_ext, double res,
+                                             const int32_t* d_map_id, const double* d_poses, const int32_t* d_pose_idx,
+                                             int64_t n, uint32_t flags, uint8_t* d_out, void* stream) {
+    const char* what = "hl_grid_footprint_check_batch";
+    if (!ctx || n < 0 || n_maps < 0 || n_aux_ext < 0 || bits_words < 0 || (n_maps > 0 && (!h_maps || !d_bits)) ||
+        (n_aux_ext > 0 && !h_aux_ext) || (n > 0 && (!d_poses || !d_out))) {
+        hl_set_error("%s: bad arguments", what); return 1;
+    }
+    if (flags & ~HL_CHECK_AUX) { hl_set_error("%s: flags must be 0 or HL_CHECK_AUX, got %u", what, flags); return 1; }
+    if ((flags & HL_CHECK_AUX) && !d_pose_idx) {
+        hl_set_error("%s: HL_CHECK_AUX needs d_pose_idx (implements are tested at even path indices)", what); return 1;
+    }
+    if (!(res > 0) || !isfinite(res)) { hl_set_error("%s: res must be finite and positive, got %g", what, res); return 1; }
+    if (n > 0 && n_maps == 0) { hl_set_error("%s: %lld poses and no maps", what, (long long)n); return 1; }
+    // the table and the implement extents go to the device in one copy: maps[n_maps] | aux[n_aux_ext][4]
+    const size_t tab_bytes = sizeof(GfMap) * (size_t)n_maps, bytes = tab_bytes + 4 * sizeof(double) * (size_t)n_aux_ext;
+    std::vector<char> host(bytes);
+    GfMap* tab = (GfMap*)host.data();
+    for (int k = 0; k < n_maps; ++k) {
+        const HlGridMap& g = h_maps[k];
+        if (g.w < 1 || g.h < 1) { hl_set_error("%s: map %d: a %dx%d grid (w and h must be at least 1)", what, k, g.w, g.h); return 1; }
+        if ((long long)g.i0 + g.w > INT_MAX || (long long)g.j0 + g.h > INT_MAX) {
+            hl_set_error("%s: map %d: a %dx%d grid at (%d, %d) overflows the int32 cell index", what, k, g.w, g.h, g.i0, g.j0);
+            return 1;
+        }
+        if (!isfinite((double)g.i0 * res) || !isfinite((double)(g.i0 + g.w) * res) || !isfinite((double)g.j0 * res) ||
+            !isfinite((double)(g.j0 + g.h) * res)) {
+            hl_set_error("%s: map %d: cell edges are not finite at res = %g", what, k, res); return 1;
+        }
+        const long long nw = ((long long)g.w * g.h + 31) / 32;
+        if (g.bits_offset < 0 || g.bits_offset > bits_words - nw) {
+            hl_set_error("%s: map %d: bit slice [%lld, %lld) outside the %lld words of d_bits", what, k,
+                         (long long)g.bits_offset, (long long)g.bits_offset + nw, (long long)bits_words); return 1;
+        }
+        if (g.aux_first < 0 || g.n_aux < 0 || (long long)g.aux_first + g.n_aux > n_aux_ext) {
+            hl_set_error("%s: map %d: implement rectangles [%d, %lld) outside the %d of h_aux_ext", what, k, g.aux_first,
+                         (long long)g.aux_first + g.n_aux, n_aux_ext); return 1;
+        }
+        tab[k] = {d_bits + g.bits_offset, g.w, g.h, g.i0, g.j0, {g.body_ext[0], g.body_ext[1], g.body_ext[2], g.body_ext[3]},
+                  g.aux_first, g.n_aux};
+    }
+    if (n_aux_ext > 0) memcpy(host.data() + tab_bytes, h_aux_ext, 4 * sizeof(double) * (size_t)n_aux_ext);
+    if (hl_enter(ctx, nullptr, n ? d_out : nullptr, what)) return 1;
+    if (n == 0) return 0;
+    const cudaStream_t st = (cudaStream_t)stream;
+    char* d_tab = nullptr;
+    HL_CUDA_OK(cudaMallocAsync((void**)&d_tab, bytes, st));
+    cudaError_t e = cudaMemcpyAsync(d_tab, host.data(), bytes, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) {
+        const GfMap* d_maps = (const GfMap*)d_tab;
+        k_grid_footprint<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(
+            d_maps, n_maps, tab[0], (const double*)(d_tab + tab_bytes), d_map_id, d_poses,
+            (flags & HL_CHECK_AUX) ? d_pose_idx : nullptr, (long long)n, res, d_out);
+        e = cudaGetLastError();
+    }
+    cudaFreeAsync(d_tab, st);
+    if (e != cudaSuccess) { hl_set_error("%s: CUDA error: %s", what, cudaGetErrorString(e)); return 1; }
+    return 0;
 }

@@ -471,6 +471,97 @@ def grid_footprint_check(bits, shape, res, poses, body_ext, origin=(0, 0)):
     return out
 
 
+def grid_pack_batch(grids):
+    """K7 pack of many grids in one launch (``hl_grid_pack_batch``).  ``grids``: [W, H] bool/uint8 grids, host arrays
+    or CUDA tensors.  Returns (bits: int32 CUDA tensor, word_offsets: int64 host array): grid k's slice starts at word
+    ``word_offsets[k]`` and equals ``grid_pack`` of that grid.  When every grid is a contiguous one-byte view of one CUDA
+    storage (the list ``rasterize`` returns) they are packed from that storage in place; otherwise they are uploaded
+    in one copy."""
+    torch = _torch()
+    lib = _lib.load_library()
+    grids = [g if torch.is_tensor(g) else np.asarray(g) for g in grids]
+    dev = _device(None, *grids)
+    if any(g.ndim != 2 for g in grids):
+        raise _lib.HeadlandError("grid_pack_batch: every grid must be 2-D [W, H]")
+    shapes = [(_int32(g.shape[0], f"grid_pack_batch: grid {k}: w"), _int32(g.shape[1], f"grid_pack_batch: grid {k}: h"))
+              for k, g in enumerate(grids)]
+    words = np.array([(w * h + 31) // 32 for w, h in shapes], dtype=np.int64)
+    word_offsets = np.concatenate([[0], np.cumsum(words)])[:-1].astype(np.int64)
+    bits = torch.empty(int(words.sum()), dtype=torch.int32, device=dev)
+    if not grids:
+        return bits, word_offsets
+    in_place = all(torch.is_tensor(g) and g.dtype in (torch.uint8, torch.bool) and g.is_contiguous() for g in grids) and \
+        len({g.untyped_storage().data_ptr() for g in grids}) == 1
+    if in_place:
+        storage = grids[0].untyped_storage()
+        base, occ_bytes = storage.data_ptr(), storage.nbytes()
+        occ_ptr, occ_off = C.c_void_p(base), [g.data_ptr() - base for g in grids]
+    else:
+        if any(torch.is_tensor(g) for g in grids):
+            occ = torch.cat([(g if torch.is_tensor(g) else torch.from_numpy(g.astype(np.uint8))).to(dev, torch.uint8).reshape(-1)
+                             for g in grids])
+        else:                              # host grids: one upload
+            occ = torch.from_numpy(np.concatenate([g.astype(np.uint8).reshape(-1) for g in grids])).to(dev)
+        occ_ptr, occ_bytes = _lib.ptr(occ), occ.numel()
+        occ_off = np.concatenate([[0], np.cumsum([w * h for w, h in shapes])])[:-1]
+    table = (_lib.HlGridPack * len(grids))()
+    for k, ((w, h), a, b) in enumerate(zip(shapes, occ_off, word_offsets)):
+        table[k] = _lib.HlGridPack(int(a), int(b), w, h)
+    _lib.check(lib.hl_grid_pack_batch(_lib.get_ctx(dev.index), occ_ptr, occ_bytes, table, len(grids), _lib.ptr(bits),
+                                      bits.numel(), _lib.stream_ptr()), "hl_grid_pack_batch")
+    return bits, word_offsets
+
+
+def grid_footprint_check_batch(bits, maps, res, poses, map_id=None, pose_idx=None, check_aux=False):
+    """K7 over many maps in one launch (``hl_grid_footprint_check_batch``): 1 where pose p meets an occupied cell of
+    map ``map_id[p]`` (map 0 without ``map_id``; an id outside the maps gives 1).  ``bits``: int32 CUDA tensor of
+    bit-packed grids (``grid_pack_batch``); ``maps``: sequence of (word_offset, (w, h), (i0, j0), body_ext, aux_exts)
+    -- the grid's slice, size and origin as ``grid_footprint_check`` takes them, the body rectangle and the vehicle's
+    [k, 4] implement rectangles.  With ``check_aux`` the implements count at even ``pose_idx`` (index of each pose
+    within its path), as in ``collision_check``.  Returns a uint8 CUDA tensor [N]."""
+    torch = _torch()
+    lib = _lib.load_library()
+    dev = _device(None, bits, poses, map_id, pose_idx)
+    if not torch.is_tensor(poses):
+        poses = torch.from_numpy(np.ascontiguousarray(np.asarray(poses, dtype=np.float64).reshape(-1, 3))).to(dev)
+    poses = poses.contiguous()
+    n = poses.shape[0]
+    map_id, pose_idx = [None if v is None else (v if torch.is_tensor(v) else torch.from_numpy(np.asarray(v))).to(dev, torch.int32).contiguous()
+                        for v in (map_id, pose_idx)]
+    table = (_lib.HlGridMap * max(len(maps), 1))()
+    aux, n_aux = [], 0
+    for k, (off, shape, origin, body, exts) in enumerate(maps):
+        exts = np.asarray(exts if exts is not None else np.zeros((0, 4)), dtype=np.float64).reshape(-1, 4)
+        m = table[k]
+        m.bits_offset = int(off)
+        m.w, m.h = _int32(shape[0], f"grid_footprint_check_batch: map {k}: w"), _int32(shape[1], f"grid_footprint_check_batch: map {k}: h")
+        m.i0, m.j0 = _int32(origin[0], f"grid_footprint_check_batch: map {k}: i0"), _int32(origin[1], f"grid_footprint_check_batch: map {k}: j0")
+        m.body_ext[:] = [float(v) for v in body]
+        m.aux_first, m.n_aux = n_aux, len(exts)
+        aux.append(exts)
+        n_aux += len(exts)
+    aux = np.ascontiguousarray(np.concatenate(aux) if aux else np.zeros((0, 4)))
+    out = torch.empty(n, dtype=torch.uint8, device=dev)
+    _lib.check(lib.hl_grid_footprint_check_batch(_lib.get_ctx(dev.index), _lib.ptr(bits), bits.numel(), table, len(maps),
+                                                 _lib.dptr(aux), len(aux), float(res), _lib.ptr(map_id), _lib.ptr(poses),
+                                                 _lib.ptr(pose_idx), n, CHECK_AUX if check_aux else 0, _lib.ptr(out),
+                                                 _lib.stream_ptr()), "hl_grid_footprint_check_batch")
+    return out
+
+
+def grid_check_sweep(vehicles, windows, grids, res, poses, map_id=None, pose_idx=None, check_aux=False):
+    """Pooled poses of a sweep against the grids of its environments in one pack and one check.  ``windows`` and
+    ``grids`` are what ``rasterize`` took and returned ((env_id, i0, j0, w, h) per grid, and the grids); ``vehicles``
+    holds per env_id an ``EnvRecord`` or ``CarModel`` (body rectangle and implements).  Pose p is checked against grid
+    ``map_id[p]`` with that grid's vehicle; see ``grid_footprint_check_batch``."""
+    bits, offsets = grid_pack_batch(grids)
+    maps = []
+    for (env_id, i0, j0, w, h), off in zip(windows, offsets):
+        v = vehicles[env_id]
+        maps.append((off, (w, h), (i0, j0), v.body_ext, getattr(v, "aux_exts", getattr(v, "aux", None))))
+    return grid_footprint_check_batch(bits, maps, res, poses, map_id=map_id, pose_idx=pose_idx, check_aux=check_aux)
+
+
 def _cell_range(vmin, vmax, res):
     """Cells lo..hi whose closed interval [fl(i*res), fl((i+1)*res)] meets [vmin, vmax] (K7's cell_range rule, not
     clamped to a grid): the floor() estimate stepped by the float64 edge comparisons themselves."""

@@ -46,11 +46,17 @@ def get_grid_map_features(occupancy_map, resolution, map_2d_position=(0.0, 0.0),
     return f
 
 
-def check_poses_on_grid(features, car_model, path):
+def check_poses_on_grid(features, car_model, path, aux_check=False):
     """Grid footprint check (the reference's commented-out
-    ``check_path_feasibility_with_grid_map``): uint8 CUDA tensor, 1 = body meets an occupied cell."""
-    return ops.grid_footprint_check(features.device_bits, features.obstacles_boolean.shape, features.resolution,
-                                    np.asarray(path, dtype=np.float64)[:, :3], car_model.body_ext)
+    ``check_path_feasibility_with_grid_map``): uint8 CUDA tensor, 1 = body meets an occupied cell.  With
+    ``aux_check`` the implement rectangles count too, at the even indices of ``path`` (car_model.py:58)."""
+    poses = np.asarray(path, dtype=np.float64)[:, :3]
+    if not aux_check:
+        return ops.grid_footprint_check(features.device_bits, features.obstacles_boolean.shape, features.resolution,
+                                        poses, car_model.body_ext)
+    maps = [(0, features.obstacles_boolean.shape, (0, 0), car_model.body_ext, car_model.aux_exts)]
+    return ops.grid_footprint_check_batch(features.device_bits, maps, features.resolution, poses,
+                                          pose_idx=np.arange(len(poses), dtype=np.int32), check_aux=True)
 
 
 def synthetic_grid(n, seed=1, n_rows=None, n_blocks=None):

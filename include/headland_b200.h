@@ -383,6 +383,54 @@ int hl_grid_footprint_check_at(hl_ctx* ctx, const uint32_t* d_occ_bits, int32_t 
                                double res, const double* d_poses, int64_t n, const double body_ext[4],
                                uint8_t* d_out, void* stream);
 
+/* K7 over tables: many grids packed in one launch, and many (grid, vehicle) maps checked in one launch.  The three
+ * calls above are batches of one of the same kernels. */
+
+/* One grid of a pack: [w][h] bytes of d_occ (non-zero = occupied; hl_env_rasterize's and hl_distance_field_batch's
+ * layout) into its own slice of 32-bit words of d_bits. */
+typedef struct {
+    int64_t occ_offset;   /* first byte of the grid in d_occ                                                     */
+    int64_t bits_offset;  /* first word of its bit slice in d_bits: (w*h + 31) / 32 words; slices must not overlap */
+    int32_t w, h;
+} HlGridPack;
+
+/* Packs n_grids grids in one launch.  Bit (i*h + j) of a slice is cell (i, j) and the tail bits of the last word are
+ * zero, so each slice equals hl_grid_pack of its grid.
+ *   h_grids  [n_grids] HOST array; checked before anything launches (a failure names the grid index): w or h below 1,
+ *            grid bytes outside occ_bytes, bit slices outside bits_words or overlapping.  n_grids == 0 launches nothing. */
+int hl_grid_pack_batch(hl_ctx* ctx, const uint8_t* d_occ, int64_t occ_bytes, const HlGridPack* h_grids, int32_t n_grids,
+                       uint32_t* d_bits, int64_t bits_words, void* stream);
+
+/* One map of a batched footprint check: a bit-packed grid (hl_grid_footprint_check_at's w, h and origin) and a vehicle. */
+typedef struct {
+    int64_t bits_offset;  /* first word of the grid's bit slice in d_bits (slices may be shared)          */
+    int32_t w, h;         /* cells                                                                        */
+    int32_t i0, j0;       /* global index of cell (0, 0)                                                  */
+    double body_ext[4];   /* body rectangle in base_link: x0, x1, y0, y1                                  */
+    int32_t aux_first;    /* implement rectangles h_aux_ext[aux_first .. aux_first + n_aux) (car_model.py:146-162) */
+    int32_t n_aux;
+} HlGridMap;
+
+/* The footprint check of the reference's pose-sampling sweeps, check_path_feasibility(..., aux_check=True)
+ * (orchard_geometry_environment.py:423-458 as called from safety_forward_path_plan.py:457-656, 733-790), on grids:
+ * pose p is checked against map d_map_id[p] (NULL = every pose uses map 0), many maps in one launch.
+ * d_out[p] = 1 (infeasible) when
+ *   - x, y or yaw is NaN or infinite, or d_map_id[p] is outside [0, n_maps) (nothing is read then); else
+ *   - the closed body rectangle meets the closed square of an occupied cell (hl_grid_footprint_check_at's rule:
+ *     float64 corners without fused multiply-add, cell squares [fl((i0+i)*res), fl((i0+i+1)*res)] x ..., touching counts);
+ *   - with flags = HL_CHECK_AUX: d_pose_idx[p] is even and some implement rectangle of the map's vehicle meets an
+ *     occupied cell (hl_collision_check's rule, car_model.py:58).
+ *   h_maps     [n_maps] HOST array and h_aux_ext [n_aux_ext][4] HOST extents (x0, x1, y0, y1), copied to the device by
+ *              the call.  Checked before anything launches (a failure names the map index): w or h below 1, i0 + w or
+ *              j0 + h beyond int32, grid edges that are not finite, bit slices outside bits_words, implement ranges
+ *              outside h_aux_ext.  Also rejected: res not finite or not positive, flags other than 0 or HL_CHECK_AUX,
+ *              HL_CHECK_AUX without d_pose_idx, n > 0 with no maps.  n == 0 launches nothing.
+ *   d_poses    [n][3] float64; d_pose_idx [n] int32 index of each pose within its path; d_out [n] uint8          */
+int hl_grid_footprint_check_batch(hl_ctx* ctx, const uint32_t* d_bits, int64_t bits_words, const HlGridMap* h_maps,
+                                  int32_t n_maps, const double* h_aux_ext, int32_t n_aux_ext, double res,
+                                  const int32_t* d_map_id, const double* d_poses, const int32_t* d_pose_idx, int64_t n,
+                                  uint32_t flags, uint8_t* d_out, void* stream);
+
 /* ---- K12 occupancy grids from environment geometry ------------------------------------------------
  * Rasterises the obstacle / tree-row quads and the field polygon of an environment batch into [w][h] uint8 grids
  * (byte i*h + j, 1 = occupied, 0 = free: hl_distance_field's layout; hl_grid_pack makes K7's bits), many grids of
