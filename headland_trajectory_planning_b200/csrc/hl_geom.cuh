@@ -511,7 +511,7 @@ static __device__ __forceinline__ void filt_stage1(const EnvSmem& E, float px, f
         if (a_obs) amb |= HL_CHECK_OBSTACLES;
     }
     bool inside = false, overflow = false;
-    unsigned near_mask = 0;                           // edges whose LINE the rectangle may touch (n <= 32 here)
+    unsigned near_mask = 0;                           // edges the rectangle may touch (n <= 32 here)
     if (flags & HL_CHECK_BOUNDARY) {
         const int n = E.n_field;
         const float rho_eps = sqrtf(fmaf(hx, hx, hy * hy)) + eps;
@@ -530,7 +530,14 @@ static __device__ __forceinline__ void filt_stage1(const EnvSmem& E, float px, f
             if (!(fabsf(sd) > rho_eps)) {                     // within the circumradius: use the exact support radius
                 const float nu = fmaf(r1.x, c, r1.y * s), nv = fmaf(r1.y, c, -r1.x * s);  // n.u, n.v
                 const float rn = fmaf(hx, fabsf(nu), hy * fabsf(nv));                    // support radius along n
-                if (!(fabsf(sd) > rn + eps)) { if (i < 32) near_mask |= 1u << i; else overflow = true; }
+                // A field boundary is mostly runs of collinear edges, and the line test above flags the whole run:
+                // also require the rectangle to reach the edge's extent along its direction.  This is filt_field2's
+                // first test, same expression, so the edges it drops are exactly those that filt_field2 skips.
+                const float ct = fmaf(-r1.y, Cx, r1.x * Cy);
+                const float rt = fmaf(hx, fabsf(nv), hy * fabsf(nu));
+                const float2 r2 = *reinterpret_cast<const float2*>(e + 8);          // extent along the edge
+                const bool along = !(ct - rt > fmaxf(r2.x, r2.y) + eps || ct + rt < fminf(r2.x, r2.y) - eps);
+                if (!(fabsf(sd) > rn + eps) && along) { if (i < 32) near_mask |= 1u << i; else overflow = true; }
             }
         }
     }
